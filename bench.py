@@ -6,6 +6,7 @@ Hanabi env steps/s on 1/2/4/8 B200 next to the reference's host-CPU implementati
     python bench.py --impl reference --gpus N --steps K ...  # the reference's CPU path on the host cores
     python bench.py --config {1..5}                          # BASELINE.json configs[0..4]; default 4
     python bench.py --scaling weak                           # `trees_total` of the config PER GPU instead of in total
+    python bench.py --dump-outputs DIR                       # + root visits / values of the last timed search as DIR/*.npy
 
 A "step" is one batched search: Roots.prepare + MCTS.run_multi (num_simulations-1 simulations, the
 PyTorch network included, random-init weights with re-drawn heads) + root statistics.  The default is
@@ -83,7 +84,14 @@ def parse_args():
     p.add_argument("--in-flight", type=int, default=None,
                    help="independent searches kept in flight per GPU (SearchPipeline depth); 1 = one search at a time")
     p.add_argument("--quick", action="store_true", help="search + roofline only (skip env / self-play / extras)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write the root statistics of the last timed search (the `value` path) as DIR/<name>.npy")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        p.error("--dump-outputs writes what the GPU path computes: it needs --impl ours")
+    return args
 
 
 def resolve_workload(args, world):
@@ -117,6 +125,24 @@ def b_env_step(obs_dim, A, obs_bytes):
     """Algorithmic bytes of one env step of one game (SURVEY.md §8d): state r/w + the observation in the dtype
     that is actually written + legal mask + reward/done/score."""
     return 2 * 192 + obs_bytes * obs_dim + obs_bytes * A + 12
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """Writes each array (same row count, float32/float64) as path/<name>.npy, so that two builds run with the same
+    arguments can be compared output for output.  Above DUMP_LIMIT_BYTES in all, a fixed seeded sample of the rows is
+    written (the same rows in every run) and `rows.npy` holds their indices."""
+    os.makedirs(path, exist_ok=True)
+    n = len(next(iter(arrays.values())))
+    row_bytes = sum(a.nbytes for a in arrays.values()) // max(n, 1)
+    if n * row_bytes > DUMP_LIMIT_BYTES:
+        keep = (DUMP_LIMIT_BYTES - 4096) // (row_bytes + 8)        # + the float64 row index; 4 KB for the .npy headers
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = dict({k: a[rows] for k, a in arrays.items()}, rows=rows.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
 
 
 # ======================================================================================================
@@ -482,8 +508,8 @@ class SearchBench:
     def finish_pipeline(self):
         """Drain the pipeline; returns (visits, values) of the last search and all ranks' statistics of it (or None)."""
         self.pipe.drain()
-        visits, _ = self.pipe.stats(self.pipe_ticket)
-        return visits, (self.pipe.gathered(self.pipe_ticket) if self.pipe.gather is not None else None)
+        stats = self.pipe.stats(self.pipe_ticket)
+        return stats, (self.pipe.gathered(self.pipe_ticket) if self.pipe.gather is not None else None)
 
     def search_step(self, executor=None, use_graph=None):
         """Roots.prepare + run_multi + root statistics (+ the statistics all_gather, off the compute stream).  One search
@@ -561,7 +587,8 @@ def run_ours(args):
     def time_searches(bench, steps, warm, piped=False):
         """CUDA-event time of `steps` searches of one SearchBench (barrier + synchronize on both sides, max over
         ranks); the gather of the last search is inside the timed region.  piped: through SearchPipeline with
-        `--in-flight` searches on their own streams (drained inside the timed region), else one search at a time."""
+        `--in-flight` searches on their own streams (drained inside the timed region), else one search at a time.
+        -> (ms, (visits, values) of the last search, all ranks' statistics of it or None)."""
         if piped:
             for _ in range(max(warm, 3 * args.in_flight)):    # each slot: one eager search, one capture, one replay
                 bench.pipelined_step()
@@ -571,21 +598,21 @@ def run_ours(args):
             e0.record()
             for _ in range(steps):
                 bench.pipelined_step()
-            visits, out = bench.finish_pipeline()             # host-blocking: every slot's search and gather is done
+            stats, out = bench.finish_pipeline()              # host-blocking: every slot's search and gather is done
             e1.record()
             barrier()
-            return max_over_ranks(e0.elapsed_time(e1)), visits, out
+            return max_over_ranks(e0.elapsed_time(e1)), stats, out
         for _ in range(warm):
             bench.search_step()
         bench.finish()
         barrier()
         e0.record()
         for _ in range(steps):
-            visits, values = bench.search_step()
+            stats = bench.search_step()
         out = bench.finish()
         e1.record()
         barrier()
-        return max_over_ranks(e0.elapsed_time(e1)), visits, out
+        return max_over_ranks(e0.elapsed_time(e1)), stats, out
 
     launches_before, gemm_before = _lib.launch_count(), _lib.gemm_launch_count()
     sb.search_step()                       # eager search (also the launch census)
@@ -608,22 +635,27 @@ def run_ours(args):
         time.sleep(0.3)   # let nvidia-smi attach before the timed regions
     # ---- timed region 1: device-resident search ------------------------------------------------
     piped = args.in_flight > 1
-    ms_one, visits_one, _ = time_searches(sb, K, W)                  # one search at a time (the latency figure)
+    ms_one, (visits_one, _), _ = time_searches(sb, K, W)             # one search at a time (the latency figure)
     sims_total = world * N * (S - 1) * K
     value_one = sims_total / (ms_one * 1e-3)
     if piped:
-        ms_total, visits, gathered = time_searches(sb, K, W, piped=True)
+        ms_total, (visits, values), gathered = time_searches(sb, K, W, piped=True)
         # same inputs: identical trees when the pipeline runs the same library kernels; with GEMMs sized for a share of
         # the SMs the network roundings differ in the last bits, so only the simulation count is checked then
         assert sb.pipe.gemm_sm_target != 0 or sb.pipe.executor != "library" or torch.equal(visits, visits_one), "a search in the pipeline must equal the same search run alone"
         assert int(visits.sum().item()) == N * (S - 1)
     else:
-        ms_total, visits, gathered = time_searches(sb, K, W)
+        ms_total, (visits, values), gathered = time_searches(sb, K, W)
     value = sims_total / (ms_total * 1e-3)
     assert int(visits.sum().item()) == N * (S - 1), "search did not run the expected simulations"
     if gathered is not None:
         assert gathered[0].shape[0] == world * N and torch.equal(gathered[0][rank * N:(rank + 1) * N], visits), \
             "gathered root statistics do not contain this rank's shard"
+    if args.dump_outputs and rank == 0:
+        # now, before later phases reuse the pipeline's statistics buffers; every rank's shard when there are several
+        out_visits, out_values = gathered if gathered is not None else (visits, values)
+        dump_outputs(args.dump_outputs, {"root_visits": out_visits.cpu().numpy().astype(np.float32),
+                                         "root_values": out_values.cpu().numpy().astype(np.float32)})
 
     # with more than one GPU: the same search with the config's tree count PER GPU (weak scaling), for the record
     weak = None

@@ -23,9 +23,11 @@ def _build_oracle():
     # test infrastructure only; the product library is built by __graft_entry__.build()
     subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "oracle"], check=True,
                    stdout=subprocess.DEVNULL)
-    if os.path.isdir("/root/reference/core/ctree"):
-        subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "ref"], check=True,
-                       stdout=subprocess.DEVNULL)
+    # the live comparisons with the reference: oracle/Makefile builds it where its sources are (REF, or the checkout
+    # $HANABIZERO_REFERENCE names) and does nothing without them
+    ref = os.environ.get("HANABIZERO_REFERENCE")
+    subprocess.run(["make", "-C", os.path.join(ROOT, "oracle"), "ref"] + (["REF=" + os.path.abspath(ref)] if ref else []),
+                   check=True, stdout=subprocess.DEVNULL)
 
 
 def golden(name):

@@ -105,6 +105,119 @@ def unpack_env_golden(g):
     return glob_, loc
 
 
+# ---- lock-step traces of the oracle against the reference (tests/golden/make_lockstep_traces.py stores them) ----
+LOCKSTEP_TREE_CASES = [(32, 20, 50, 11, True, "random"), (16, 11, 50, 12, True, "random"),
+                       (8, 20, 120, 13, False, "random"), (9, 20, 40, 14, True, "zero_rows"),
+                       (1, 20, 50, 15, True, "random")]
+LOCKSTEP_ENV_CASES = [(preset, mode) for mode in ("random", "noplay", "smart") for preset in (0, 1)]
+
+
+def lockstep_tree_name(N, A, S, seed, noise, mask_mode):
+    return f"lockstep_tree_n{N}_a{A}_s{S}_seed{seed}{'' if noise else '_nonoise'}_{mask_mode}.npz"
+
+
+def extreme_tree_inputs():
+    """N, A, S and inputs with NaN logits at a root (not sanitised by the reference), huge/tiny logits, NaN values."""
+    N, A, S = 6, 20, 12
+    d = tree_inputs(N, A, S, 3)
+    d["logits"][0, 3] = np.nan
+    d["logits"][1, :] = -200.0
+    d["logits"][1, 5] = 50.0
+    d["logits"][2, :] = 1e30
+    d["sim_value"][2, 3] = np.nan
+    d["sim_reward"][4, 4] = np.inf
+    d["mask"][5, :] = 1
+    return N, A, S, d
+
+
+def tree_trace(engine, d, S, noise=True):
+    """One tree engine (oracle.loader.TreeEngine API) driven through `d`: root priors, then per simulation the
+    traverse outputs and the root statistics after back-propagation, then every tree's expanded nodes."""
+    engine.prepare(CONST["frac"], d["noise"] if noise else None, d["reward"], d["logits"], d["mask"])
+    t = {"priors": engine.root_priors()}
+    steps = []
+    for s in range(S - 1):
+        out = engine.traverse(CONST["pb_c_base"], CONST["pb_c_init"], CONST["discount"])
+        engine.backprop(s + 1, CONST["discount"], d["sim_reward"][s], d["sim_value"][s], d["sim_logits"][s])
+        steps.append(tuple(out) + tuple(engine.stats()))
+    for i, k in enumerate(("ix", "iy", "la", "visits", "values", "minmax")):
+        t[k] = np.stack([st[i] for st in steps])
+    ex = [engine.expanded_stats(i, S + 1) for i in range(engine.num)]
+    t["ex_n"] = np.array([len(e[0]) for e in ex], np.int32)
+    for j, k in enumerate(("ex_reward", "ex_value_sum", "ex_visits")):
+        t[k] = np.zeros((engine.num, S + 1), ex[0][j].dtype)
+        for i, e in enumerate(ex):
+            t[k][i, :len(e[j])] = e[j]
+    return t
+
+
+def assert_same_tree_trace(a, b, per_step_stats=True, expanded=True):
+    """Bit-exact agreement of two tree_trace records (per_step_stats=False: the root statistics after the last
+    simulation only; expanded=False: without the expanded nodes)."""
+    assert bits_equal(a["priors"], b["priors"]), "root priors"
+    for k in ("ix", "iy", "la"):
+        bad = np.flatnonzero((a[k] != b[k]).any(1))
+        assert not len(bad), f"{k} differs first at simulation {bad[:1]}"
+    for k in ("visits", "values", "minmax"):
+        if per_step_stats:
+            bad = [s for s in range(len(a[k])) if not bits_equal(a[k][s], b[k][s])]
+            assert not bad, f"{k} differs first at simulation {bad[0]}"
+        else:
+            assert bits_equal(a[k][-1], b[k][-1]), k
+    if expanded:
+        for k in ("ex_n", "ex_reward", "ex_value_sum", "ex_visits"):
+            assert bits_equal(a[k], b[k]), k
+
+
+def env_trace(make, preset, mode, seeds=6, episodes=4):
+    """Episodes of one Hanabi engine (oracle.loader.HanabiGameCPU API, `make(preset, seed)`): the same game object
+    per seed over `episodes` resets (the mt19937 stream persists across resets), moves picked by env_policy from the
+    engine's own state dump.  One row per reset (kind 0) or step (kind 1); `dump` is the state before a step."""
+    rows = {k: [] for k in ("kind", "action", "glob", "loc", "legal", "rds", "dump", "dump_n")}
+
+    def add(kind, action, obs, rds, dump):
+        for k, v in zip(("kind", "action", "glob", "loc", "legal", "rds"), (kind, action) + tuple(obs) + (rds,)):
+            rows[k].append(v)
+        rows["dump_n"].append(len(dump))
+        rows["dump"].append(np.pad(dump, (0, 256 - len(dump)), constant_values=-1))
+
+    for seed in range(seeds):
+        rng = np.random.default_rng(17 * seed + preset)
+        g = make(preset, seed)
+        for _ in range(episodes):
+            a = g.reset()
+            add(0, -1, a, (0, 0, 0), np.zeros(0, np.int32))
+            done = False
+            while not done:
+                dump = g.dump()
+                act = env_policy(mode, rng, g.hand_size, a[2], playable_from_dump(dump, g.colors, g.ranks, g.hand_size))
+                a = g.step(act)
+                add(1, act, a[:3], a[3:], dump)
+                done = a[4]
+    return {k: np.asarray(v, np.int32) for k, v in rows.items()}
+
+
+def env_trace_record(t):
+    """env_trace -> what is stored and compared: the episode structure, moves, reward/done/score and dump lengths in
+    full, and per row one 64-bit digest of the global and local observations, the legal mask and the state dump."""
+    import hashlib
+    rows = np.concatenate([t[k] for k in ("glob", "loc", "legal", "dump")], axis=1).astype(np.int32)
+    digest = [np.frombuffer(hashlib.blake2b(r.tobytes(), digest_size=8).digest(), np.uint64)[0] for r in rows]
+    out = {k: t[k] for k in ("kind", "action", "rds", "dump_n")}
+    out["row_digest"] = np.array(digest, np.uint64)
+    return out
+
+
+def assert_same_env_trace(a, b):
+    """Two env_trace_record records agree row by row."""
+    n = min(len(a["kind"]), len(b["kind"]))
+    for k in ("kind", "action", "rds", "dump_n", "row_digest"):
+        bad = np.flatnonzero((a[k][:n] != b[k][:n]).reshape(n, -1).any(1))
+        assert not len(bad), f"{k} differs first at row {bad[0]}"
+    assert len(a["kind"]) == len(b["kind"]), "episode lengths"
+    assert (a["kind"] == 1).sum() > 100
+
+
 class RefGameHistory:
     """The fields of core/game.py:49-215 that self-play writes, as the reference writes them (test-side port)."""
 

@@ -1,9 +1,11 @@
 """CPU: the plain-C Hanabi oracle (oracle/hanabi_oracle.c) against golden episodes produced by the
-reference's own Python HanabiEnv, and live against the compiled reference library."""
+reference's own Python HanabiEnv, against the stored lock-step episodes of tests/golden/make_lockstep_traces.py and,
+when the reference is built, live against the compiled reference library."""
 import numpy as np
 import pytest
 
-from helpers import env_policy, golden_files, load_golden, playable_from_dump, unpack_env_golden
+from helpers import (assert_same_env_trace, env_trace, env_trace_record, golden_files, load_golden,
+                     unpack_env_golden)
 from oracle import loader as L
 
 
@@ -40,28 +42,18 @@ def test_illegal_action_rejected():
         env.step(bad)
 
 
+@pytest.mark.parametrize("preset", [0, 1])
+@pytest.mark.parametrize("mode", ["random", "noplay", "smart"])
+def test_oracle_matches_stored_reference_episodes(preset, mode):
+    """The lock-step comparison below against its stored record (tests/golden/make_lockstep_traces.py): 6 seeds x 4
+    episodes on one game object per seed, observations, legal masks, state dumps, rewards and scores row by row."""
+    assert_same_env_trace(env_trace_record(env_trace(L.oracle_hanabi, preset, mode)),
+                          load_golden(f"lockstep_env_preset{preset}_{mode}.npz"))
+
+
 @pytest.mark.skipif(not L.have_ref(), reason="oracle/_ref not built")
 @pytest.mark.parametrize("preset", [0, 1])
 @pytest.mark.parametrize("mode", ["random", "noplay", "smart"])
 def test_oracle_matches_live_reference(preset, mode):
-    steps = 0
-    for seed in range(6):
-        rng = np.random.default_rng(17 * seed + preset)
-        o, r = L.oracle_hanabi(preset, seed), L.ref_hanabi(preset, seed)
-        for ep in range(4):  # same game object: the mt19937 stream persists across resets
-            a, b = o.reset(), r.reset()
-            for x, y in zip(a, b):
-                assert (x == y).all()
-            done = False
-            while not done:
-                dump = o.dump()
-                assert (dump == r.dump()).all()
-                act = env_policy(mode, rng, o.hand_size, a[2],
-                                 playable_from_dump(dump, o.colors, o.ranks, o.hand_size))
-                a, b = o.step(act), r.step(act)
-                for x, y in zip(a[:3], b[:3]):
-                    assert (x == y).all(), (seed, ep, steps)
-                assert a[3:] == b[3:]
-                done = a[4]
-                steps += 1
-    assert steps > 100
+    assert_same_env_trace(env_trace_record(env_trace(L.oracle_hanabi, preset, mode)),
+                          env_trace_record(env_trace(L.ref_hanabi, preset, mode)))

@@ -1,10 +1,11 @@
 """CPU: the plain-C tree oracle (oracle/tree_oracle.c) against golden traces produced by the
-unmodified reference ctree (oracle/_ref, rand()==0 shim) and, when present, live against it."""
+unmodified reference ctree (oracle/_ref, rand()==0 shim), against the stored lock-step traces of
+tests/golden/make_lockstep_traces.py and, when the reference is built, live against it."""
 import numpy as np
 import pytest
 
-from helpers import (CONST, bits_equal, golden_files, golden_tree_inputs, load_golden,
-                     run_tree_lockstep, tree_inputs)
+from helpers import (CONST, LOCKSTEP_TREE_CASES, assert_same_tree_trace, bits_equal, extreme_tree_inputs, golden_files,
+                     golden_tree_inputs, load_golden, lockstep_tree_name, run_tree_lockstep, tree_inputs, tree_trace)
 from oracle import loader as L
 
 
@@ -25,55 +26,36 @@ def test_input_generator_in_sync_with_golden():
         assert bits_equal(d[k], g["in_" + k]), k
 
 
-@pytest.mark.skipif(not L.have_ref(), reason="oracle/_ref not built (no /root/reference here)")
-@pytest.mark.parametrize("N,A,S,seed,noise,mask_mode", [
-    (32, 20, 50, 11, True, "random"), (16, 11, 50, 12, True, "random"),
-    (8, 20, 120, 13, False, "random"), (9, 20, 40, 14, True, "zero_rows"), (1, 20, 50, 15, True, "random")])
+@pytest.mark.parametrize("N,A,S,seed,noise,mask_mode", LOCKSTEP_TREE_CASES)
+def test_oracle_matches_stored_reference_trace(N, A, S, seed, noise, mask_mode):
+    """The lock-step comparison below against its stored trace (tests/golden/make_lockstep_traces.py): root priors,
+    every simulation's traverse outputs and root statistics, and every expanded node, bit-exact."""
+    d = tree_inputs(N, A, S, seed, mask_mode)
+    assert_same_tree_trace(tree_trace(L.oracle_tree(N, A, S), d, S, noise),
+                           load_golden(lockstep_tree_name(N, A, S, seed, noise, mask_mode)))
+
+
+@pytest.mark.skipif(not L.have_ref(), reason="oracle/_ref not built (no reference sources at build time)")
+@pytest.mark.parametrize("N,A,S,seed,noise,mask_mode", LOCKSTEP_TREE_CASES)
 def test_oracle_matches_live_reference(N, A, S, seed, noise, mask_mode):
     d = tree_inputs(N, A, S, seed, mask_mode)
-    o, r = L.oracle_tree(N, A, S), L.ref_tree(N, A, S)
-    for e in (o, r):
-        e.prepare(CONST["frac"], d["noise"] if noise else None, d["reward"], d["logits"], d["mask"])
-    assert bits_equal(o.root_priors(), r.root_priors())
-    for s in range(S - 1):
-        a = o.traverse(CONST["pb_c_base"], CONST["pb_c_init"], CONST["discount"])
-        b = r.traverse(CONST["pb_c_base"], CONST["pb_c_init"], CONST["discount"])
-        for x, y in zip(a, b):
-            assert (x == y).all(), s
-        for e in (o, r):
-            e.backprop(s + 1, CONST["discount"], d["sim_reward"][s], d["sim_value"][s], d["sim_logits"][s])
-        for x, y in zip(o.stats(), r.stats()):
-            assert bits_equal(x, y), s
-    for i in range(N):
-        for x, y in zip(o.expanded_stats(i, S + 1), r.expanded_stats(i, S + 1)):
-            assert bits_equal(x, y)
+    assert_same_tree_trace(tree_trace(L.oracle_tree(N, A, S), d, S, noise), tree_trace(L.ref_tree(N, A, S), d, S, noise))
+
+
+def test_nan_and_extreme_inputs_match_stored_reference_trace():
+    """NaN logits at the root (not sanitised by the reference), huge/tiny logits, NaN values: traverse outputs of every
+    simulation and the final root statistics against the stored trace."""
+    N, A, S, d = extreme_tree_inputs()
+    assert_same_tree_trace(tree_trace(L.oracle_tree(N, A, S), d, S), load_golden("lockstep_tree_extreme.npz"),
+                           per_step_stats=False, expanded=False)
 
 
 @pytest.mark.skipif(not L.have_ref(), reason="oracle/_ref not built")
 def test_nan_and_extreme_inputs_match_reference():
-    """NaN logits at the root (not sanitised by the reference), huge/tiny logits, NaN values."""
-    N, A, S = 6, 20, 12
-    d = tree_inputs(N, A, S, 3)
-    d["logits"][0, 3] = np.nan
-    d["logits"][1, :] = -200.0
-    d["logits"][1, 5] = 50.0
-    d["logits"][2, :] = 1e30
-    d["sim_value"][2, 3] = np.nan
-    d["sim_reward"][4, 4] = np.inf
-    d["mask"][5, :] = 1
-    o, r = L.oracle_tree(N, A, S), L.ref_tree(N, A, S)
-    for e in (o, r):
-        e.prepare(CONST["frac"], d["noise"], d["reward"], d["logits"], d["mask"])
-    assert bits_equal(o.root_priors(), r.root_priors())
-    for s in range(S - 1):
-        a = o.traverse(CONST["pb_c_base"], CONST["pb_c_init"], CONST["discount"])
-        b = r.traverse(CONST["pb_c_base"], CONST["pb_c_init"], CONST["discount"])
-        for x, y in zip(a, b):
-            assert (x == y).all(), s
-        for e in (o, r):
-            e.backprop(s + 1, CONST["discount"], d["sim_reward"][s], d["sim_value"][s], d["sim_logits"][s])
-    for x, y in zip(o.stats(), r.stats()):
-        assert bits_equal(x, y)
+    """The same inputs live against the reference."""
+    N, A, S, d = extreme_tree_inputs()
+    assert_same_tree_trace(tree_trace(L.oracle_tree(N, A, S), d, S), tree_trace(L.ref_tree(N, A, S), d, S),
+                           per_step_stats=False, expanded=False)
 
 
 def test_random_tie_mode_is_uniform_like_the_stock_reference():

@@ -62,7 +62,7 @@ class _Cfg:
 def test_unmodified_reference_mcts_drives_the_dropin(N, A, S, seed):
     from oracle import refpy
     if not refpy.available():
-        pytest.skip("oracle/_ref/refpy not built (needs /root/reference at build time)")
+        pytest.skip("oracle/_ref/refpy not built (no reference sources at build time)")
     sys.path.insert(0, os.path.join(ROOT, "dropin"))
     try:
         for k in [k for k in sys.modules if k == "core" or k.startswith("core.")]:
