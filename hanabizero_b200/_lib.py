@@ -49,6 +49,7 @@ SIGNATURES = {
     "hz_gemm_launch_count": (_i64, []),
     "hz_gemm_plan_run": (_i, [_vp, _vp, _i, _i]),
     "hz_rowchain_create": (_i, [C.POINTER(_vp), _i, _vp, _i, _vp, _i64, _vp, _vp]),
+    "hz_rowchain_create_small": (_i, [C.POINTER(_vp), _i, _vp, _i, _vp, _i64, _vp, _vp]),
     "hz_rowchain_destroy": (_i, [_vp]),
     "hz_rowchain_set_state": (_i, [_vp, _vp]),
     "hz_rowchain_run": (_i, [_vp, _vp]),

@@ -1,10 +1,14 @@
-// Row-block resident executor of MuZeroNetFull's recurrent_inference (hanabizero_b200/plan.py; the function of
-// /root/reference/core/model.py:74-84 over config/hanabi_control/model.py:199-216,301-318 in eval mode, BatchNorm folded):
+// Row-block resident executor of recurrent_inference for both Hanabi networks (hanabizero_b200/plan.py; the function of
+// /root/reference/core/model.py:74-84 over config/hanabi_control/model.py:127-335 in eval mode, BatchNorm folded):
 // ONE launch per simulation in which every CTA owns 128 rows of the batch for the WHOLE chain
 //
+// MuZeroNetFull (Hanabi-Full, hz_rowchain_create):
 //   y1 = relu(W1 [s | onehot(a)] + b1)  ->  y2 = relu(W2 y1 + b2)  ->  s' = relu(W3 y2 + b3 + s)            (dynamics)
 //   value / reward:  relu(Wh1 s')  ->  relu(WB2 .)  ->  WB3 .   (201-wide support logits, padded to P3)
 //   policy:          h = relu(Wh1 s')  ->  a1 = relu(WB2 h)  ->  a2 = relu(Wa2 a1 + h)  ->  WB3 a2
+// MuZeroNet (Hanabi-Small, hz_rowchain_create_small; the skip joins after bn1, heads 128 wide, one layer each):
+//   y1 = relu(W1 [s | onehot(a)] + b1 + s)  ->  y2 = relu(W2 y1 + b2)  ->  s' = relu(W3 y2 + b3)
+//   h = relu(Wh1 s') = [value | reward | policy]  ->  WB3[i] h_i   (51 / 51 / 11 logits, padded to 64)
 //
 // Why this shape.  The seven library GEMMs of this chain are single waves of 128x128 tiles: every CTA pulls 256 KB of
 // operands through its SM's ~165 GB/s L2 port for 1 us of tensor work, so at 4096 rows the whole device is held for
@@ -14,23 +18,30 @@
 // columns) are drained by the epilogue warps straight back into that layout, and only the weights stream in (3.2 MB
 // per row block, L2-resident, TMA into a 3 x 32 KB ring).  A 4096-row batch occupies 32 SMs instead of 148.
 //
-//   warp 0      TMA producer: weight tiles [256 (or 208) out-columns x 64 k] in the static order of the job table
-//   warp 1      tcgen05.mma issuer (one lane), M = 128, N = 256 | 208, K = 16, fp16 x fp16 -> fp32 in TMEM
+//   warp 0      TMA producer: weight tiles [N <= 256 out-columns x 64 k] in the static order of the job table
+//   warp 1      tcgen05.mma issuer (one lane), M = 128, N = 256 | 208 (Full) | 256 | 128 | 64 (Small), K = 16,
+//               fp16 x fp16 -> fp32 in TMEM
 //   warps 2-17  epilogue: tcgen05.ld -> + bias (+ residual) -> ReLU -> fp16 -> back into the activation tile (swizzled),
 //               in place; one of its threads moves whole tiles between shared and global memory as bulk tensor copies
 //               (s in, s' out to the pool and back in for the policy branch, logits out)
 //
-// A launch runs ten phases (the job table hz_rowchain_create builds): fc1 | fc2 | fc3 + s | value, reward first layers |
-// their second layers | their logits | policy h | a1 | a2 | policy logits.  A phase = one or two jobs (one per TMEM
-// half) of MMAs, then their drains; the next phase's first MMAs start as soon as the first job is drained (ready0).
+// The kernel walks a job table built on the host.  Hanabi-Full: ten phases, fc1 | fc2 | fc3 + s | value, reward first
+// layers | their second layers | their logits | policy h | a1 | a2 | policy logits.  Hanabi-Small: six, fc1 + s | fc2 |
+// fc3 | the three first layers (N 256 + 128) | value, reward logits | policy logits (N 64).  A phase = one or two jobs
+// (one per TMEM half) of MMAs, then their drains; the next phase's first MMAs start as soon as the first job is drained
+// (ready0).  Each job's weight map has a box of exactly its N rows (the producer's expect_tx counts N rows per K-block);
+// create checks that and the table's other bounds on the host.  The kernel is instantiated per network (kSmall), so the
+// Hanabi-Full launch runs none of Hanabi-Small's code.
 //
-// The one-hot action columns of fc1 are not multiplied: row r adds column a_r of W1's action block (a 32 x 512 table,
-// W1aT) in the epilogue, which is the same sum.  fc3's residual s is copied back into the consumed tile and read from
-// shared memory.  The value/reward branch runs first on the resident s'; the policy branch re-reads s' (already stored
-// to the pool) afterwards, because three 256-wide first layers need 768 TMEM columns.
+// The one-hot action columns of fc1 are not multiplied: row r adds column a_r of W1's action block (a 32 x 512 or
+// 16 x 512 table, W1aT) in the epilogue, which is the same sum.  Full: fc3's residual s is copied back into the
+// consumed tile and read from shared memory; the value/reward branch runs first on the resident s', the policy branch
+// re-reads s' (already stored to the pool) afterwards, because three 256-wide first layers need 768 TMEM columns.
+// Small: fc1's residual s is fc1's own A operand, still in the tile when fc1 drains; its three first layers fit the
+// 384 TMEM columns at once.
 //
-// fp16 plans of the Hanabi-Full network only (F = 512, H = 256); everything else stays on the library chain.
-// Measurements, stamps and what bounds it: profiles/r02_rowchain.md.
+// fp16 plans of these two networks only (F = 512, H = 256 or 128); everything else stays on the library chain.
+// Measurements, stamps and what bounds it: profiles/r02_rowchain.md (Full), profiles/r03_rowchain_small.md (Small).
 #include <cuda.h>
 #include <cuda_fp16.h>
 
@@ -42,6 +53,7 @@
 namespace hz {
 
 constexpr int kBM = 128, kBK = 64, kF = 512, kH = 256;
+constexpr int kHSmall = 128, kP3Small = 64;        // Hanabi-Small: heads 128 wide, 51 support logits padded to 64
 constexpr int kKB = kBM * kBK * 2;                 // one K-block of the activation tile: 128 rows x 128 bytes
 constexpr int kActBytes = kBM * kF * 2;            // 128 KB: 8 K-blocks
 constexpr int kWSlot = 256 * kBK * 2;              // 32 KB: a weight tile of up to 256 output columns x 64 k
@@ -58,6 +70,7 @@ struct RowJob {
   int32_t map, n0, batch, num_k, a_kb, n, half;   // weight tile source, A K-block offset, MMA N, TMEM half
   int32_t relu, dst_kb;                           // dst_kb >= 0: write fp16 into activation K-blocks dst_kb..
   int32_t res, res_off;                           // 0 none | 1 W1aT[action] + res_off | 2 x0 hidden + res_off (global) | 3 tile K-block res_off
+                                                  // | 4 W1aT[action] + n0 and tile K-block res_off
   int32_t gout, gb;                               // 0 none | 1 TMA-store the tile to `state` | 2 TMA-store K-blocks dst_kb.. to out[gb]
   int32_t kb1;                                    // MMA: K-blocks before this one need only the previous phase's FIRST job drained
   const __half* bias;
@@ -72,8 +85,8 @@ struct alignas(64) RowParams {
   CUtensorMap maps[kMaps];
   RowPhase phase[kMaxPhases];
   int32_t n_phases, rows, row_blocks, p3;
-  const __half* x0; int64_t ld_x0;                // [rows][ld_x0]: 512 hidden | 32 one-hot
-  const __half* w1a_t;                            // [32][512]
+  const __half* x0; int64_t ld_x0;                // [rows][ld_x0]: 512 hidden | 32 (Full) or 16 (Small) one-hot columns
+  const __half* w1a_t;                            // [32 or 16][512]
   __half* state;                                  // [rows][512]
   __half* out;                                    // [3][rows][p3]
   unsigned long long* trace;                      // optional [grid][kMaxPhases][4] globaltimer stamps
@@ -187,6 +200,9 @@ __device__ __forceinline__ void stamp(const RowParams& P, int phase, int slot) {
 
 using namespace rc;
 
+// kSmall: the Hanabi-Small instantiation (16 one-hot columns, residual mode 4).  The Hanabi-Full one compiles without
+// any of it, so Hanabi-Small costs the Full launch nothing.
+template <bool kSmall>
 __global__ void __launch_bounds__(kRowThreads, 1) k_row_chain(const __grid_constant__ RowParams P) {
   extern __shared__ uint8_t smem_raw[];
   const uint32_t base = (smem_u32(smem_raw) + 1023u) & ~1023u;   // swizzle-128B tiles need 1024-byte alignment
@@ -315,7 +331,7 @@ __global__ void __launch_bounds__(kRowThreads, 1) k_row_chain(const __grid_const
 #pragma unroll
       for (int kb = 0; kb < kF / kBK; ++kb) tma_load_3d(act + kb * kKB, &P.maps[map], bar, kb * kBK, rb_ * kBM, 0);
     };
-    uint32_t rf_par = 0;
+    uint32_t rf_par = 0, ea_par = 0;
     if (et == 0) load_tile(kMapX0, blockIdx.x, a_full);
     __syncwarp();
     if (lane == 0) { mbar_arrive(ready0); mbar_arrive(ready1); }
@@ -340,11 +356,15 @@ __global__ void __launch_bounds__(kRowThreads, 1) k_row_chain(const __grid_const
         for (int j = 0; j < 2; ++j) {
           if (j >= F.njobs) continue;
           const RowJob& J = F.job[j];
-          if (J.res == 1 && live) {
+          if ((J.res == 1 || (kSmall && J.res == 4)) && live) {
+            // only the row's own one-hot columns: past them lie the next row's state columns, and any of those that
+            // is exactly 1.0 would read as an action
             const uint4* oh = reinterpret_cast<const uint4*>(P.x0 + (size_t)row * P.ld_x0 + kF);
+            constexpr int n_oh = kSmall ? 2 : 4;   // 16-byte chunks of 8 one-hot columns
             int a = -1;
 #pragma unroll
             for (int v = 0; v < 4; ++v) {
+              if (v >= n_oh) break;               // (compile-time)
               const uint4 w = oh[v];
               const uint32_t u[4] = {w.x, w.y, w.z, w.w};
 #pragma unroll
@@ -353,11 +373,11 @@ __global__ void __launch_bounds__(kRowThreads, 1) k_row_chain(const __grid_const
                 if ((u[t] >> 16) == 0x3c00u) a = v * 8 + t * 2 + 1;
               }
             }
-            if (a >= 0) crow[j] = P.w1a_t + (size_t)a * kF + J.res_off;
+            if (a >= 0) crow[j] = P.w1a_t + (size_t)a * kF + (J.res == 1 ? J.res_off : J.n0);
           } else if (J.res == 2 && live) {
             crow[j] = P.x0 + (size_t)row * P.ld_x0 + J.res_off;
           }
-          if (j == 0 && crow[0]) {
+          if (j == 0 && crow[0]) {   // (res 4: only warms L1 with the W1aT chunk; the residual read is the tile's)
             const int c0 = ((part * (J.n >> 4)) >> 2) * 16;
             ef0 = __ldg(reinterpret_cast<const uint4*>(crow[0] + c0));
             ef1 = __ldg(reinterpret_cast<const uint4*>(crow[0] + c0 + 8));
@@ -371,6 +391,12 @@ __global__ void __launch_bounds__(kRowThreads, 1) k_row_chain(const __grid_const
           a_par ^= 1u << h;
         }
         tc_fence_after();
+        if (kSmall && F.a_wait) {
+          // a residual read from the tile the TMA loaded for this phase: wait for that load here too, so the bulk
+          // copy's writes are visible to these threads (the MMAs that read it have completed, so this never blocks)
+          if (F.job[0].res == 4 || F.job[1].res == 4) mbar_wait(a_full, ea_par);
+          ea_par ^= 1u;
+        }
         if (et == 0 && first_rb) stamp(P, ph, 2);
         if (F.res_load) {
           // the tile has been consumed: the input state s comes back into it (bulk copy) and is read as the residual
@@ -393,7 +419,7 @@ __global__ void __launch_bounds__(kRowThreads, 1) k_row_chain(const __grid_const
           any_store |= J.gout != 0;
           // residual of columns [c, c + 16) of this thread's row (zero when the row has none)
           auto fetch_res = [&](int c, uint4& e0, uint4& e1) {
-            if (res == 3) {
+            if (res == 3 || (kSmall && res == 4)) {
               const int ch = res_off * 8 + (c >> 3);
               e0 = ld_shared_v4(act + act_off(rloc, ch));
               e1 = ld_shared_v4(act + act_off(rloc, ch + 1));
@@ -424,6 +450,17 @@ __global__ void __launch_bounds__(kRowThreads, 1) k_row_chain(const __grid_const
                 v[2 * t] += x0.x; v[2 * t + 1] += x0.y; v[8 + 2 * t] += x1.x; v[8 + 2 * t + 1] += x1.y;
               }
             }
+            if (kSmall && res == 4 && cr) {   // fc1's action column on top of the state residual (L1-resident table)
+              const uint4 w0 = __ldg(reinterpret_cast<const uint4*>(cr + c));
+              const uint4 w1 = __ldg(reinterpret_cast<const uint4*>(cr + c + 8));
+              const __half2* g0 = reinterpret_cast<const __half2*>(&w0);
+              const __half2* g1 = reinterpret_cast<const __half2*>(&w1);
+#pragma unroll
+              for (int t = 0; t < 4; ++t) {
+                const float2 x0 = __half22float2(g0[t]), x1 = __half22float2(g1[t]);
+                v[2 * t] += x0.x; v[2 * t + 1] += x0.y; v[8 + 2 * t] += x1.x; v[8 + 2 * t + 1] += x1.y;
+              }
+            }
             uint4 o0, o1;
             __half2* p0 = reinterpret_cast<__half2*>(&o0);
             __half2* p1 = reinterpret_cast<__half2*>(&o1);
@@ -445,7 +482,7 @@ __global__ void __launch_bounds__(kRowThreads, 1) k_row_chain(const __grid_const
           };
           uint32_t ra[16], rb2[16];
           uint4 ea0 = ef0, ea1 = ef1, eb0 = make_uint4(0, 0, 0, 0), eb1 = eb0;
-          if (j == 1 || res == 3) {
+          if (j == 1 || res == 3 || (kSmall && res == 4)) {
             ea0 = ea1 = make_uint4(0, 0, 0, 0);
             fetch_res(c_begin, ea0, ea1);
           }
@@ -552,53 +589,69 @@ static bool make_w_map(CUtensorMap* map, const void* ptr, int64_t k, int64_t n, 
             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+// The kernel trusts its job table.  The one invariant it cannot survive: the producer expects J.n * 128 bytes per
+// K-block but a TMA load moves its map's whole box, so a box of other than J.n rows leaves a wait unsatisfied and the
+// kernel traps (kSpin).  Checked on the host with the table's other bounds, so a wrong table is an argument error.
+static const char* table_error(const RowParams& P, const int* box_rows, bool small) {
+  for (int p = 0; p < P.n_phases; ++p) {
+    const RowPhase& F = P.phase[p];
+    for (int j = 0; j < F.njobs; ++j) {
+      const RowJob& J = F.job[j];
+      const int kbs = (J.n + kBK - 1) / kBK, tile_kbs = kF / kBK;
+      if (J.map < 0 || J.map >= kMapX0 || box_rows[J.map] != J.n) return "a weight map's box is not the job's N rows";
+      if (J.n < 16 || J.n > 256 || J.n % 16) return "N must be a multiple of 16 between 16 and 256";
+      if (J.half < 0 || J.half > 1 || J.half * 256 + J.n > 512) return "accumulators past the 512 TMEM columns";
+      if (J.num_k < 1 || J.a_kb < 0 || J.a_kb + J.num_k > tile_kbs) return "A operand K-blocks outside the tile";
+      if (J.dst_kb >= 0 && J.dst_kb + kbs > tile_kbs) return "destination K-blocks outside the tile";
+      if (J.res >= 3 && (J.res_off < 0 || J.res_off + kbs > tile_kbs)) return "residual K-blocks outside the tile";
+      if (J.res == 4 && (!small || !F.a_wait)) return "a tile + action residual is Hanabi-Small's, in a phase with a_wait";
+    }
+  }
+  return nullptr;
+}
+
 }  // namespace hz
 
 using namespace hz;
 
 struct hz_rowchain {
   int device = 0, grid = 0, sms = 0;
+  bool small = false;                 // which job table (and kernel instantiation): Hanabi-Small or Hanabi-Full
   RowParams params;
   unsigned long long* trace = nullptr;
 };
 
-extern "C" {
-#pragma GCC visibility push(default)
+// Job table + weight maps of either network (arguments already checked by the entry points), then the launch setup.
+static int rowchain_create(const char* who, bool small, hz_rowchain** out, int device, const hz_rowchain_weights* w,
+                           int rows, const void* x0, int64_t ld_x0, void* state, void* out_logits) {
+  const int p3 = w->logit_cols;
+  // fp16 weights [batch][n][k] with row stride ld, loaded as boxes of `box` rows x 64 k (one per job's K-block)
+  struct WMap { const void* ptr; int64_t k, n, batch, ld; int box; };
+  WMap wm[kMapX0];
+  if (!small) {
+    wm[0] = {w->w1, kF, kF, 1, w->ld_w1, 256};       // action columns are added in the epilogue
+    wm[1] = {w->w2, kF, kF, 1, kF, 256};
+    wm[2] = {w->w3, kF, kF, 1, kF, 256};
+    wm[3] = {w->wh1, kF, 3 * kH, 1, kF, 256};
+    wm[4] = {w->wb2, kH, kH, 3, kH, 256};
+    wm[5] = {w->wa2, kH, kH, 1, kH, 256};
+    wm[6] = {w->wb3, kH, p3, 3, kH, p3};
+  } else {
+    wm[0] = {w->w1, kF, kF, 1, w->ld_w1, 256};
+    wm[1] = {w->w2, kF, kF, 1, kF, 256};
+    wm[2] = {w->w3, kF, kF, 1, kF, 256};
+    wm[3] = {w->wh1, kF, 3 * kHSmall, 1, kF, 256};           // rows 0..255: value | reward
+    wm[4] = {w->wh1, kF, 3 * kHSmall, 1, kF, 128};           // rows 256..383: actor
+    wm[5] = {w->wb3, kHSmall, kP3Small, 3, kHSmall, kP3Small};
+    wm[6] = wm[5];                                           // unused; a valid descriptor for the kernel's prefetch
+  }
+  int box_rows[kMapX0];
+  for (int m = 0; m < kMapX0; ++m) box_rows[m] = wm[m].box;
 
-int hz_rowchain_create(hz_rowchain** out, int device, const hz_rowchain_weights* w, int rows, const void* x0,
-                       int64_t ld_x0, void* state, void* out_logits) {
-  if (!out || !w || rows <= 0 || !x0 || !state || !out_logits) { set_error("hz_rowchain_create: bad argument"); return HZ_ERR_ARG; }
-  if (w->state_cols != kF || w->head_cols != kH || w->onehot_cols != 32 || w->logit_cols <= 0 || w->logit_cols > 256 ||
-      w->logit_cols % 16 || ld_x0 < kF + 32 || ld_x0 % 8 || w->ld_w1 < kF + 32 || w->ld_w1 % 8) {
-    set_error("hz_rowchain_create: this executor is built for state 512 / heads 256 / one-hot 32 / logits <= 256 (multiple of 16)");
-    return HZ_ERR_ARG;
-  }
-  const void* ptrs[] = {w->w1, w->w1a_t, w->b1, w->w2, w->b2, w->w3, w->b3, w->wh1, w->bh1, w->wb2, w->bb2,
-                        w->wa2, w->ba2, w->wb3, w->bb3, x0, state, out_logits};
-  for (const void* p : ptrs) {
-    if (!p || ((uintptr_t)p & 15)) { set_error("hz_rowchain_create: null or unaligned pointer"); return HZ_ERR_ARG; }
-  }
-  DeviceGuard dg(device);
-  if (!dg.ok) { set_error("hz_rowchain_create: cannot select device %d", device); return HZ_ERR_CUDA; }
-  if (!encode_fn()) { set_error("hz_rowchain_create: cuTensorMapEncodeTiled unavailable"); return HZ_ERR_CUDA; }
   hz_rowchain* e = new hz_rowchain;
   e->device = device;
   RowParams& P = e->params;
   memset(&P, 0, sizeof(P));
-  const int p3 = w->logit_cols;
-  bool ok = make_w_map(&P.maps[0], w->w1, kF, kF, 1, w->ld_w1, 256) &&       // action columns are added in the epilogue
-            make_w_map(&P.maps[1], w->w2, kF, kF, 1, kF, 256) &&
-            make_w_map(&P.maps[2], w->w3, kF, kF, 1, kF, 256) &&
-            make_w_map(&P.maps[3], w->wh1, kF, 3 * kH, 1, kF, 256) &&
-            make_w_map(&P.maps[4], w->wb2, kH, kH, 3, kH, 256) &&
-            make_w_map(&P.maps[5], w->wa2, kH, kH, 1, kH, 256) &&
-            make_w_map(&P.maps[6], w->wb3, kH, p3, 3, kH, p3) &&
-            // activations: boxes of 128 rows x 64 columns, the K-blocks of the tile (rows past the end read as zero
-            // and are not written)
-            make_w_map(&P.maps[kMapX0], x0, kF, rows, 1, ld_x0, kBM) &&
-            make_w_map(&P.maps[kMapState], state, kF, rows, 1, kF, kBM) &&
-            make_w_map(&P.maps[kMapOut], out_logits, p3, rows, 3, p3, kBM);
-  if (!ok) { delete e; set_error("hz_rowchain_create: cuTensorMapEncodeTiled failed"); return HZ_ERR_CUDA; }
   const __half *b1 = (const __half*)w->b1, *b2 = (const __half*)w->b2, *b3 = (const __half*)w->b3,
                *bh1 = (const __half*)w->bh1, *bb2 = (const __half*)w->bb2, *ba2 = (const __half*)w->ba2,
                *bb3 = (const __half*)w->bb3;
@@ -617,23 +670,36 @@ int hz_rowchain_create(hz_rowchain** out, int device, const hz_rowchain_weights*
     if (j1) F.job[1] = *j1;
   };
   RowJob t;
-  // dynamics
-  t = job(0, 256, 0, 8, 0, 256, 1, b1 + 256, 1, 4, 1, 256);  phase(0, job(0, 0, 0, 8, 0, 256, 0, b1, 1, 0, 1, 0), &t, 1);
-  t = job(1, 256, 0, 8, 0, 256, 1, b2 + 256, 1, 4);          phase(0, job(1, 0, 0, 8, 0, 256, 0, b2, 1, 0), &t);
-  t = job(2, 256, 0, 8, 0, 256, 1, b3 + 256, 1, 4, 3, 4, 1);
-  phase(0, job(2, 0, 0, 8, 0, 256, 0, b3, 1, 0, 3, 0, 1), &t);
-  P.phase[np - 1].res_load = 1;                                      // + s, reloaded into the consumed tile
-  // value | reward branch on the resident s' (Wh1 rows: actor 0..255, value 256..511, reward 512..767)
-  t = job(3, 512, 0, 8, 0, 256, 1, bh1 + 512, 1, 4);         phase(0, job(3, 256, 0, 8, 0, 256, 0, bh1 + 256, 1, 0), &t);
-  t = job(4, 0, 2, 4, 4, 256, 1, bb2 + 512, 1, 4);           phase(0, job(4, 0, 1, 4, 0, 256, 0, bb2 + 256, 1, 0), &t);
-  // the logits are staged in the (now idle) tile, K-blocks 0..3 / 4..7, and leave as bulk stores
-  t = job(6, 0, 1, 4, 4, p3, 1, bb3 + p3, 0, 4, 0, 0, 2, 1);
-  phase(1, job(6, 0, 0, 4, 0, p3, 0, bb3, 0, 0, 0, 0, 2, 0), &t);
-  // policy branch on the reloaded s'
-  phase(0, job(3, 0, 0, 8, 0, 256, 0, bh1, 1, 0), nullptr, 1);       // h  -> K-blocks 0..3
-  phase(0, job(4, 0, 0, 4, 0, 256, 1, bb2, 1, 4));                   // a1 -> K-blocks 4..7
-  phase(0, job(5, 0, 0, 4, 4, 256, 0, ba2, 1, 0, 3, 0));             // a2 = relu(Wa2 a1 + h) -> K-blocks 0..3
-  phase(2, job(6, 0, 2, 4, 0, p3, 1, bb3 + 2 * p3, 0, 4, 0, 0, 2, 2));   // policy logits staged in K-blocks 4..7
+  if (!small) {
+    // dynamics
+    t = job(0, 256, 0, 8, 0, 256, 1, b1 + 256, 1, 4, 1, 256);  phase(0, job(0, 0, 0, 8, 0, 256, 0, b1, 1, 0, 1, 0), &t, 1);
+    t = job(1, 256, 0, 8, 0, 256, 1, b2 + 256, 1, 4);          phase(0, job(1, 0, 0, 8, 0, 256, 0, b2, 1, 0), &t);
+    t = job(2, 256, 0, 8, 0, 256, 1, b3 + 256, 1, 4, 3, 4, 1);
+    phase(0, job(2, 0, 0, 8, 0, 256, 0, b3, 1, 0, 3, 0, 1), &t);
+    P.phase[np - 1].res_load = 1;                                      // + s, reloaded into the consumed tile
+    // value | reward branch on the resident s' (Wh1 rows: actor 0..255, value 256..511, reward 512..767)
+    t = job(3, 512, 0, 8, 0, 256, 1, bh1 + 512, 1, 4);         phase(0, job(3, 256, 0, 8, 0, 256, 0, bh1 + 256, 1, 0), &t);
+    t = job(4, 0, 2, 4, 4, 256, 1, bb2 + 512, 1, 4);           phase(0, job(4, 0, 1, 4, 0, 256, 0, bb2 + 256, 1, 0), &t);
+    // the logits are staged in the (now idle) tile, K-blocks 0..3 / 4..7, and leave as bulk stores
+    t = job(6, 0, 1, 4, 4, p3, 1, bb3 + p3, 0, 4, 0, 0, 2, 1);
+    phase(1, job(6, 0, 0, 4, 0, p3, 0, bb3, 0, 0, 0, 0, 2, 0), &t);
+    // policy branch on the reloaded s'
+    phase(0, job(3, 0, 0, 8, 0, 256, 0, bh1, 1, 0), nullptr, 1);       // h  -> K-blocks 0..3
+    phase(0, job(4, 0, 0, 4, 0, 256, 1, bb2, 1, 4));                   // a1 -> K-blocks 4..7
+    phase(0, job(5, 0, 0, 4, 4, 256, 0, ba2, 1, 0, 3, 0));             // a2 = relu(Wa2 a1 + h) -> K-blocks 0..3
+    phase(2, job(6, 0, 2, 4, 0, p3, 1, bb3 + 2 * p3, 0, 4, 0, 0, 2, 2));   // policy logits staged in K-blocks 4..7
+  } else {
+    // dynamics: fc1's skip s joins after bn1; s is fc1's own A operand, still in the tile when its drain runs
+    t = job(0, 256, 0, 8, 0, 256, 1, b1 + 256, 1, 4, 4, 4);    phase(0, job(0, 0, 0, 8, 0, 256, 0, b1, 1, 0, 4, 0), &t, 1);
+    t = job(1, 256, 0, 8, 0, 256, 1, b2 + 256, 1, 4);          phase(0, job(1, 0, 0, 8, 0, 256, 0, b2, 1, 0), &t);
+    t = job(2, 256, 0, 8, 0, 256, 1, b3 + 256, 1, 4);          phase(0, job(2, 0, 0, 8, 0, 256, 0, b3, 1, 0, 0, 0, 1), &t);
+    // the three heads' first layers on the resident s' (Wh1 rows: value 0..127, reward 128..255, actor 256..383)
+    t = job(4, 256, 0, 8, 0, 128, 1, bh1 + 256, 1, 4);         phase(0, job(3, 0, 0, 8, 0, 256, 0, bh1, 1, 0), &t);
+    // logits staged in tile K-blocks the heads no longer need (value 6, reward 7, then policy 0), out as bulk stores
+    t = job(5, 0, 1, 2, 2, p3, 1, bb3 + p3, 0, 7, 0, 0, 2, 1);
+    phase(0, job(5, 0, 0, 2, 0, p3, 0, bb3, 0, 6, 0, 0, 2, 0), &t);
+    phase(2, job(5, 0, 2, 2, 4, p3, 0, bb3 + 2 * p3, 0, 0, 0, 0, 2, 2));
+  }
   // how far a phase's first job may run on the previous phase's first job alone (see ready0 / ready1 in the kernel)
   for (int p = 0; p < np; ++p) {
     RowPhase& F = P.phase[p];
@@ -649,6 +715,23 @@ int hz_rowchain_create(hz_rowchain** out, int device, const hz_rowchain_weights*
     J.kb1 = k;
   }
   P.n_phases = np;
+  if (const char* bad = table_error(P, box_rows, small)) {
+    delete e;
+    set_error("%s: job table: %s", who, bad);
+    return HZ_ERR_ARG;
+  }
+  DeviceGuard dg(device);
+  if (!dg.ok) { delete e; set_error("%s: cannot select device %d", who, device); return HZ_ERR_CUDA; }
+  if (!encode_fn()) { delete e; set_error("%s: cuTensorMapEncodeTiled unavailable", who); return HZ_ERR_CUDA; }
+  bool ok = true;
+  for (int m = 0; m < kMapX0; ++m)
+    ok = ok && make_w_map(&P.maps[m], wm[m].ptr, wm[m].k, wm[m].n, wm[m].batch, wm[m].ld, wm[m].box);
+  // activations: boxes of 128 rows x 64 columns, the K-blocks of the tile (rows past the end read as zero and are not
+  // written)
+  ok = ok && make_w_map(&P.maps[kMapX0], x0, kF, rows, 1, ld_x0, kBM) &&
+       make_w_map(&P.maps[kMapState], state, kF, rows, 1, kF, kBM) &&
+       make_w_map(&P.maps[kMapOut], out_logits, p3, rows, 3, p3, kBM);
+  if (!ok) { delete e; set_error("%s: cuTensorMapEncodeTiled failed", who); return HZ_ERR_CUDA; }
   P.rows = rows;
   P.row_blocks = (rows + kBM - 1) / kBM;
   P.p3 = p3;
@@ -657,14 +740,55 @@ int hz_rowchain_create(hz_rowchain** out, int device, const hz_rowchain_weights*
   P.w1a_t = (const __half*)w->w1a_t;
   P.state = (__half*)state;
   P.out = (__half*)out_logits;
-  cudaError_t err = cudaFuncSetAttribute(k_row_chain, cudaFuncAttributeMaxDynamicSharedMemorySize, kRowSmem);
+  e->small = small;
+  cudaError_t err = small ? cudaFuncSetAttribute(k_row_chain<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kRowSmem)
+                          : cudaFuncSetAttribute(k_row_chain<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kRowSmem);
   cudaDeviceProp prop;
   if (err == cudaSuccess) err = cudaGetDeviceProperties(&prop, device);
-  if (err != cudaSuccess) { delete e; return fail_cuda(err, "hz_rowchain_create: setup"); }
+  if (err != cudaSuccess) { delete e; return fail_cuda(err, who); }
   e->sms = prop.multiProcessorCount;
   e->grid = P.row_blocks < e->sms ? P.row_blocks : e->sms;
   *out = e;
   return HZ_OK;
+}
+
+extern "C" {
+#pragma GCC visibility push(default)
+
+int hz_rowchain_create(hz_rowchain** out, int device, const hz_rowchain_weights* w, int rows, const void* x0,
+                       int64_t ld_x0, void* state, void* out_logits) {
+  if (!out || !w || rows <= 0 || !x0 || !state || !out_logits) { set_error("hz_rowchain_create: bad argument"); return HZ_ERR_ARG; }
+  if (w->state_cols != kF || w->head_cols != kH || w->onehot_cols != 32 || w->logit_cols <= 0 || w->logit_cols > 256 ||
+      w->logit_cols % 16 || ld_x0 < kF + 32 || ld_x0 % 8 || w->ld_w1 < kF + 32 || w->ld_w1 % 8) {
+    set_error("hz_rowchain_create: this executor is built for state 512 / heads 256 / one-hot 32 / logits <= 256 (multiple of 16)");
+    return HZ_ERR_ARG;
+  }
+  const void* ptrs[] = {w->w1, w->w1a_t, w->b1, w->w2, w->b2, w->w3, w->b3, w->wh1, w->bh1, w->wb2, w->bb2,
+                        w->wa2, w->ba2, w->wb3, w->bb3, x0, state, out_logits};
+  for (const void* p : ptrs) {
+    if (!p || ((uintptr_t)p & 15)) { set_error("hz_rowchain_create: null or unaligned pointer"); return HZ_ERR_ARG; }
+  }
+  return rowchain_create("hz_rowchain_create", false, out, device, w, rows, x0, ld_x0, state, out_logits);
+}
+
+int hz_rowchain_create_small(hz_rowchain** out, int device, const hz_rowchain_weights* w, int rows, const void* x0,
+                             int64_t ld_x0, void* state, void* out_logits) {
+  if (!out || !w || rows <= 0 || !x0 || !state || !out_logits) { set_error("hz_rowchain_create_small: bad argument"); return HZ_ERR_ARG; }
+  if (w->state_cols != kF || w->head_cols != kHSmall || w->onehot_cols != 16 || w->logit_cols != kP3Small ||
+      ld_x0 < kF + 16 || ld_x0 % 8 || w->ld_w1 < kF + 16 || w->ld_w1 % 8) {
+    set_error("hz_rowchain_create_small: this executor is built for state 512 / heads 128 / one-hot 16 / logits 64");
+    return HZ_ERR_ARG;
+  }
+  if (w->wb2 || w->bb2 || w->wa2 || w->ba2) {
+    set_error("hz_rowchain_create_small: wb2 / bb2 / wa2 / ba2 belong to the Hanabi-Full heads and must be NULL");
+    return HZ_ERR_ARG;
+  }
+  const void* ptrs[] = {w->w1, w->w1a_t, w->b1, w->w2, w->b2, w->w3, w->b3, w->wh1, w->bh1, w->wb3, w->bb3,
+                        x0, state, out_logits};
+  for (const void* p : ptrs) {
+    if (!p || ((uintptr_t)p & 15)) { set_error("hz_rowchain_create_small: null or unaligned pointer"); return HZ_ERR_ARG; }
+  }
+  return rowchain_create("hz_rowchain_create_small", true, out, device, w, rows, x0, ld_x0, state, out_logits);
 }
 
 int hz_rowchain_destroy(hz_rowchain* e) {
@@ -711,7 +835,8 @@ int hz_rowchain_grid(const hz_rowchain* e) { return e ? e->grid : 0; }
 int hz_rowchain_run(hz_rowchain* e, void* stream) {
   if (!e) { set_error("hz_rowchain_run: bad argument"); return HZ_ERR_ARG; }
   DeviceGuard dg(e->device);
-  k_row_chain<<<e->grid, kRowThreads, kRowSmem, (cudaStream_t)stream>>>(e->params);
+  if (e->small) k_row_chain<true><<<e->grid, kRowThreads, kRowSmem, (cudaStream_t)stream>>>(e->params);
+  else k_row_chain<false><<<e->grid, kRowThreads, kRowSmem, (cudaStream_t)stream>>>(e->params);
   HZ_LAUNCH_CHECK("k_row_chain");
   return HZ_OK;
 }

@@ -214,7 +214,7 @@ class MCTS(object):
         that keep several searches in flight on different streams: SearchPipeline sets it); stage_limit > 0 likewise
         shrinks the tree step's shared-memory staging so that it shares SMs with other searches' GEMMs
         (hz_search_io.stage_limit).  executor="rows" runs the network as one row-block resident launch per simulation
-        (BoundChain.set_executor; fp16 Hanabi-Full plan, otherwise ignored).  None of them changes any result of the
+        (BoundChain.set_executor; fp16 plans of Hanabi-Full and Hanabi-Small, otherwise ignored).  None of them changes any result of the
         tree step; the SM target and the executor change network roundings in the last bits."""
         with torch.no_grad():
             if getattr(model, "training", True):
@@ -269,6 +269,24 @@ def gemm_sm_target_for(num_roots, in_flight, device):
     return int(max(16, min(3 * num_roots // 64, 56 * sms // 148)))
 
 
+ROWS_MIN_BLOCKS_SMALL = 48   # row blocks in flight from which Hanabi-Small gains from the row executor (B200, measured)
+
+
+def network_executor_for(model, num_roots, in_flight):
+    """The network executor executor="auto" picks for `in_flight` independent searches (SearchPipeline slots,
+    SelfPlayPool engines) of `num_roots` trees each.  One search at a time: the library chain, whose latency is lower.
+    Searches in flight: the row-block resident executor, which holds num_roots / 128 SMs per search instead of the whole
+    device.  For the Hanabi-Small network its longer chain (37 us against 15-24 us) only pays once the searches in
+    flight keep at least ROWS_MIN_BLOCKS_SMALL 128-row blocks going: measured on B200 (profiles/r03_rowchain_small.md),
+    512 trees x 8 and 1024 x 4 in flight (32 blocks) run 11-21 % faster on the library chain, 768 x 8 and 512 x 12
+    (48 blocks) 4-13 % slower.  Plans the row executor does not cover (fp32) run the library chain whatever this says."""
+    if in_flight <= 1:
+        return "library"
+    if not getattr(model, "full", True) and in_flight * -(-int(num_roots) // 128) < ROWS_MIN_BLOCKS_SMALL:
+        return "library"
+    return "rows"
+
+
 class SearchPipeline:
     """Searches kept in flight: `depth` slots, each with its own tree batch (and therefore its own captured search
     graph, network buffers and staging buffers) and its own compute stream.  Inputs are copied in on a copy stream and
@@ -291,7 +309,8 @@ class SearchPipeline:
     the module.
 
     With depth > 1 the network runs on the row-block resident executor (`executor`, hz_rowchain: one launch per
-    simulation on n/128 SMs; profiles/r02_rowchain.md) where the plan supports it.  For the library chain two settings
+    simulation on n/128 SMs; profiles/r02_rowchain.md, r03_rowchain_small.md) where the plan supports it and, for
+    Hanabi-Small, where enough row blocks are in flight for it to pay (network_executor_for).  For the library chain two settings
     make the slots share the GPU instead of queueing (profiles/r02_sm_target.md): `gemm_sm_target`
     (default gemm_sm_target_for(num_roots, depth)) sizes each search's library GEMMs for a share of the SMs, and
     `stage_limit` (default 4) keeps the tree step's shared-memory footprint small enough to sit next to a GEMM CTA.
@@ -303,10 +322,10 @@ class SearchPipeline:
         self.mcts, self.model = mcts, model
         self.depth = int(depth)
         # "rows": the network as one row-block resident launch per simulation (BoundChain.set_executor) — a quarter of
-        # the SMs per search at 4096 trees, which is what searches in flight want; "library": seven cuBLASLt launches,
-        # the lower latency for a search that runs alone.  "auto" = rows whenever searches overlap (plans the
-        # executor does not cover fall back to the library chain inside MCTS).
-        self.executor = ("rows" if self.depth > 1 else "library") if executor == "auto" else executor
+        # the SMs per search at 4096 trees, which is what searches in flight want; "library": seven (Hanabi-Full) or
+        # five (Hanabi-Small) cuBLASLt launches, the lower latency for a search that runs alone.  "auto": see
+        # network_executor_for (plans the row executor does not cover fall back to the library chain inside MCTS).
+        self.executor = network_executor_for(model, num_roots, self.depth) if executor == "auto" else executor
         self.n, self.a, self.depth = int(num_roots), int(num_actions), int(depth)
         self.device = next(model.parameters()).device if device is None else torch.device(device)
         dev, sims = self.device, int(mcts.config.num_simulations)

@@ -102,32 +102,39 @@ class BoundChain:
         self._rows, self._use_rows = C.c_void_p(), False
 
     def rows_supported(self):
-        """The row-block resident executor (hz_rowchain, include/hzb200.h) covers the fp16 Hanabi-Full plan."""
+        """The row-block resident executor (hz_rowchain, include/hzb200.h) covers the fp16 plans of both networks:
+        Hanabi-Full (F 512, H 256, one-hot 32) and Hanabi-Small (F 512, H 128, one-hot 16, 64 logit columns)."""
         p = self.plan
-        return bool(p.full and p.dtype == torch.float16 and p.F == 512 and p.H == 256 and p.OH == 32 and p.P3 <= 256)
+        if p.dtype != torch.float16 or p.F != 512:
+            return False
+        if p.full:
+            return bool(p.H == 256 and p.OH == 32 and p.P3 <= 256)
+        return bool(p.H == 128 and p.OH == 16 and p.P3 == 64)
 
     def set_executor(self, name):
-        """"library": seven cuBLASLt launches (lowest latency for one search on an idle GPU).  "rows": ONE launch in
-        which each CTA carries 128 rows through the whole chain (hz_rowchain): 1/4 of the SMs at 4096 rows, for
-        searches in flight.  Same function; roundings differ in the last fp16 bits."""
+        """"library": seven (Hanabi-Full) / five (Hanabi-Small) cuBLASLt launches (lowest latency for one search on an
+        idle GPU).  "rows": ONE launch in which each CTA carries 128 rows through the whole chain (hz_rowchain): 1/4 of
+        the SMs at 4096 rows, for searches in flight.  Same function; roundings differ in the last fp16 bits."""
         if name not in ("library", "rows"):
             raise ValueError("executor must be 'library' or 'rows'")
         if name == "rows":
             if not self.rows_supported():
-                raise RuntimeError("the row-block executor needs the fp16 Hanabi-Full plan (F=512, H=256)")
+                raise RuntimeError("the row-block executor needs an fp16 plan of Hanabi-Full (F=512, H=256) or "
+                                   "Hanabi-Small (F=512, H=128)")
             if not self._rows:
                 p, w = self.plan, self.plan._w
                 ws = _lib.RowChainWeights()
                 ws.w1, ws.ld_w1, ws.w1a_t, ws.b1 = w["W1"].data_ptr(), w["W1"].stride(0), w["W1aT"].data_ptr(), w["b1"].data_ptr()
                 ws.w2, ws.b2, ws.w3, ws.b3 = w["W2"].data_ptr(), w["b2"].data_ptr(), w["W3"].data_ptr(), w["b3"].data_ptr()
                 ws.wh1, ws.bh1 = w["Wh1"].data_ptr(), w["bh1"].data_ptr()
-                ws.wb2, ws.bb2 = w["WB2"].data_ptr(), w["bB2"].data_ptr()
-                ws.wa2, ws.ba2 = w["Wa2"].data_ptr(), w["ba2"].data_ptr()
+                if p.full:   # Hanabi-Small's heads have no second layers: those pointers stay NULL
+                    ws.wb2, ws.bb2 = w["WB2"].data_ptr(), w["bB2"].data_ptr()
+                    ws.wa2, ws.ba2 = w["Wa2"].data_ptr(), w["ba2"].data_ptr()
                 ws.wb3, ws.bb3 = w["WB3"].data_ptr(), w["bB3"].data_ptr()
                 ws.state_cols, ws.head_cols, ws.onehot_cols, ws.logit_cols = p.F, p.H, p.OH, p.P3
-                check(p.lib.hz_rowchain_create(C.byref(self._rows), p.device.index, C.byref(ws), self.n,
-                                               self.x0.data_ptr(), self.x0.stride(0), self._state_ptr,
-                                               self.out.data_ptr()))
+                create = p.lib.hz_rowchain_create if p.full else p.lib.hz_rowchain_create_small
+                check(create(C.byref(self._rows), p.device.index, C.byref(ws), self.n, self.x0.data_ptr(),
+                             self.x0.stride(0), self._state_ptr, self.out.data_ptr()))
         self._use_rows = name == "rows"
 
     def set_sm_target(self, sm_count):

@@ -251,11 +251,11 @@ class SelfPlayPool:
             raise ValueError("SelfPlayPool needs at least one engine")
         dev = self.engines[0].dev
         self.streams = [torch.cuda.Stream(dev) for _ in self.engines]
-        from .mcts import STAGE_LIMIT_IN_FLIGHT, gemm_sm_target_for
+        from .mcts import STAGE_LIMIT_IN_FLIGHT, gemm_sm_target_for, network_executor_for
         for eng in self.engines:
             eng.gemm_sm_target = gemm_sm_target_for(eng.n, len(self.engines), dev)
             eng.stage_limit = STAGE_LIMIT_IN_FLIGHT if len(self.engines) > 1 else 0
-            eng.executor = "rows" if len(self.engines) > 1 else "library"
+            eng.executor = network_executor_for(eng.model, eng.n, len(self.engines))
         cur = torch.cuda.current_stream(dev)
         for s in self.streams:
             s.wait_stream(cur)       # engine construction ran on the caller's stream

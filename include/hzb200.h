@@ -387,15 +387,17 @@ int hz_gemm_plan_set_sm_target(hz_gemm_plan* p, int sm_count);
 int64_t hz_gemm_launch_count(void);
 int hz_gemm_plan_run(hz_gemm_plan* p, void* stream, int first, int count);
 
-/* Row-block resident executor of the Hanabi-Full recurrent_inference chain (fp16): the same function as the
- * seven-step hz_gemm_plan that hanabizero_b200/plan.py builds for MuZeroNetFull
- * (/root/reference/core/model.py:74-84, config/hanabi_control/model.py:199-216,301-318, eval mode, BatchNorm folded),
+/* Row-block resident executor of the recurrent_inference chain (fp16): the same function as the hz_gemm_plan that
+ * hanabizero_b200/plan.py builds (seven steps for MuZeroNetFull, five for MuZeroNet / Hanabi-Small;
+ * /root/reference/core/model.py:74-84, config/hanabi_control/model.py:199-216,301-318, eval mode, BatchNorm folded),
  * as ONE launch in which each CTA keeps 128 rows of the batch in shared memory / TMEM through all layers and only the
  * weights stream in (TMA + tcgen05, hanabizero_b200/csrc/hz_rowchain.cu).  A 4096-row batch occupies 32 SMs, which is
- * what several searches in flight want.  All pointers dev, fp16, 16-byte aligned, captured at creation. */
+ * what several searches in flight want.  hz_rowchain_create builds the Hanabi-Full chain, hz_rowchain_create_small the
+ * Hanabi-Small one; every other hz_rowchain_* call serves both.  All pointers dev, fp16, 16-byte aligned, captured at
+ * creation. */
 typedef struct hz_rowchain_weights {
   const void* w1;  int64_t ld_w1;     /* [512][ld_w1]: fc1 (+bn1) over [state | one-hot action] */
-  const void* w1a_t;                  /* [32][512]: the action columns of w1, transposed */
+  const void* w1a_t;                  /* [onehot_cols][512]: the action columns of w1, transposed */
   const void* b1;
   const void* w2;  const void* b2;    /* [512][512] */
   const void* w3;  const void* b3;    /* [512][512]; the residual is the input state */
@@ -404,18 +406,25 @@ typedef struct hz_rowchain_weights {
   const void* wa2; const void* ba2;   /* [256][256]: policy residual block, second layer */
   const void* wb3; const void* bb3;   /* [3][logit_cols][256]: output layers value | reward | policy */
   int32_t state_cols, head_cols, onehot_cols, logit_cols;   /* 512, 256, 32, <= 256 (multiple of 16) */
-} hz_rowchain_weights;
+} hz_rowchain_weights;   /* shapes as hz_rowchain_create takes them; hz_rowchain_create_small states its own */
 typedef struct hz_rowchain hz_rowchain;
 /* x0 [rows][ld_x0] = state | one-hot(action) (what hz_trees_search_step hands over), state [rows][512] receives the
  * next hidden state, out_logits [3][rows][logit_cols] = value | reward | policy logits. */
 int hz_rowchain_create(hz_rowchain** out, int device, const hz_rowchain_weights* w, int rows, const void* x0,
                        int64_t ld_x0, void* state, void* out_logits);                                   /* sync */
+/* Hanabi-Small (MuZeroNet): fc1's skip s joins after bn1, no residual after fc3, one layer per head.  Same struct:
+ * state_cols 512, head_cols 128, onehot_cols 16, logit_cols 64; w1 [512][ld_w1 >= 528], w1a_t [16][512],
+ * wh1 [384][512] = first layers of value | reward | policy heads, wb3 [3][64][128] = their output layers (same order);
+ * wb2 / bb2 / wa2 / ba2 must be NULL.  x0 [rows][ld_x0 >= 528], out_logits [3][rows][64]. */
+int hz_rowchain_create_small(hz_rowchain** out, int device, const hz_rowchain_weights* w, int rows, const void* x0,
+                             int64_t ld_x0, void* state, void* out_logits);                             /* sync */
 int hz_rowchain_destroy(hz_rowchain* e);
 /* Re-point the next-state output (the search loop passes pool[x]); takes effect for the following runs. */
 int hz_rowchain_set_state(hz_rowchain* e, void* state);
 int hz_rowchain_run(hz_rowchain* e, void* stream);
 int hz_rowchain_grid(const hz_rowchain* e);                     /* CTAs per launch */
-/* Debug: per-CTA globaltimer stamps of the first row block, uint64[grid][10 phases][4] =
+/* Debug: per-CTA globaltimer stamps of the first row block, uint64[grid][10 phase slots][4] (Hanabi-Full runs 10
+ * phases, Hanabi-Small 6) =
  * {MMA may start, MMAs issued, accumulators complete, tile written back}. */
 int hz_rowchain_set_trace(hz_rowchain* e, int enable);
 int hz_rowchain_read_trace(hz_rowchain* e, uint64_t* host_out, int64_t count);                          /* sync */

@@ -1,22 +1,27 @@
-"""Experiment: the row-block resident network executor (hz_rowchain) against the seven-launch cuBLASLt chain.
+"""Experiment: the row-block resident network executor (hz_rowchain) against the cuBLASLt library chain (seven
+launches; five for Hanabi-Small).
   1. parity of state / value / reward / policy logits (vs the library chain and vs a float64 evaluation)
   2. per-phase stamps of CTA 0
   3. time per chain alone (CUDA graph, back to back) and with D chains on D streams (what searches in flight see)
-Env: N (rows, default 4096), D (streams, default 7)."""
+Env: N (rows, default 4096), D (streams, default 7), NET (full | small: MuZeroNetFull or the Hanabi-Small MuZeroNet,
+default full)."""
 import ctypes, os, sys, traceback
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
 import torch
 from hanabizero_b200 import _lib
-from hanabizero_b200.model import MuZeroNetFull
+from hanabizero_b200.model import MuZeroNet, MuZeroNetFull
 from hanabizero_b200.plan import BoundChain
 
 dev = torch.device("cuda")
-N = int(os.environ.get("N", "4096")); D = int(os.environ.get("D", "7"))
+N = int(os.environ.get("N", "4096")); D = int(os.environ.get("D", "7")); NET = os.environ.get("NET", "full")
+if NET not in ("full", "small"):
+    sys.exit("NET must be full or small")
 lib = _lib.load()
 torch.manual_seed(0)
-model = MuZeroNetFull(785 * 4, 20).randomize_heads().to(dev).eval()
+model = (MuZeroNetFull(785 * 4, 20) if NET == "full" else MuZeroNet(193 * 4, 11)).randomize_heads().to(dev).eval()
 plan = model.recurrent_plan(torch.float16)
+PHASES = 10 if NET == "full" else 6      # the job table's phases (hz_rowchain.cu)
 
 
 def fill(ch, seed):
@@ -33,8 +38,13 @@ def ref64(ch):
     w = {k: v.double() for k, v in plan._w.items()}
     x = ch.x0.double()
     relu = torch.relu
+    H = plan.H
+    if NET == "small":   # skip after bn1, no residual after fc3, one layer per head ([value | reward | policy])
+        y1 = relu(x @ w["W1"].T + w["b1"] + x[:, :plan.F]); y2 = relu(y1 @ w["W2"].T + w["b2"]); s = relu(y2 @ w["W3"].T + w["b3"])
+        h1 = relu(s @ w["Wh1"].T + w["bh1"])
+        return s, torch.stack([h1[:, i * H:(i + 1) * H] @ w["WB3"][i].T + w["bB3"][i] for i in range(3)])
     y1 = relu(x @ w["W1"].T + w["b1"]); y2 = relu(y1 @ w["W2"].T + w["b2"]); s = relu(y2 @ w["W3"].T + w["b3"] + x[:, :plan.F])
-    h1 = relu(s @ w["Wh1"].T + w["bh1"]); H = plan.H
+    h1 = relu(s @ w["Wh1"].T + w["bh1"])
     a1 = relu(h1[:, :H] @ w["WB2"][0].T + w["bB2"][0]); v2 = relu(h1[:, H:2 * H] @ w["WB2"][1].T + w["bB2"][1])
     r2 = relu(h1[:, 2 * H:] @ w["WB2"][2].T + w["bB2"][2]); a2 = relu(a1 @ w["Wa2"].T + w["ba2"] + h1[:, :H])
     outs = [t @ w["WB3"][i].T + w["bB3"][i] for i, t in enumerate((v2, r2, a2))]
@@ -80,12 +90,12 @@ def stamps(ch):
     check(lib.hz_rowchain_read_trace(ch._rows, buf, g * 40))
     t = np.frombuffer(buf, dtype=np.uint64).reshape(g, 10, 4).astype(np.int64)
     check(lib.hz_rowchain_set_trace(ch._rows, 0))
-    t0 = t[0, 0, 0]
+    t0, last = t[0, 0, 0], PHASES - 1
     print("  CTA 0 stamps, ns from the first phase's start: [MMA may start, MMAs issued, accumulators complete, tile written]")
-    for ph in range(10):
+    for ph in range(PHASES):
         print(f"    phase {ph}: {(t[0, ph] - t0).tolist()}")
-    print(f"  whole chain, CTA 0: {(t[0, 9, 3] - t0) / 1e3:.1f} us; over CTAs: min {((t[:, 9, 3] - t[:, 0, 0]).min()) / 1e3:.1f} "
-          f"max {((t[:, 9, 3] - t[:, 0, 0]).max()) / 1e3:.1f} us", flush=True)
+    print(f"  whole chain, CTA 0: {(t[0, last, 3] - t0) / 1e3:.1f} us; over CTAs: min {((t[:, last, 3] - t[:, 0, 0]).min()) / 1e3:.1f} "
+          f"max {((t[:, last, 3] - t[:, 0, 0]).max()) / 1e3:.1f} us", flush=True)
 
 
 def graph_of(ch, reps, stream):
