@@ -470,9 +470,10 @@ __global__ void __launch_bounds__(kRowThreads, 1) k_row_chain(const __grid_const
               p1[t] = __floats2half2_rn(v[8 + 2 * t], v[8 + 2 * t + 1]);
             }
             if (relu) {   // rounding is monotonic and keeps the sign: max(round(x), 0) == round(max(x, 0))
+              // NaN stays NaN, as in the library chain's ReLU epilogue (plain __hmax2 would return the 0)
               const __half2 z = __float2half2_rn(0.0f);
 #pragma unroll
-              for (int t = 0; t < 4; ++t) { p0[t] = __hmax2(p0[t], z); p1[t] = __hmax2(p1[t], z); }
+              for (int t = 0; t < 4; ++t) { p0[t] = __hmax2_nan(p0[t], z); p1[t] = __hmax2_nan(p1[t], z); }
             }
             if (dst_kb >= 0) {
               const int ch = dst_kb * 8 + (c >> 3);
@@ -486,7 +487,8 @@ __global__ void __launch_bounds__(kRowThreads, 1) k_row_chain(const __grid_const
             ea0 = ea1 = make_uint4(0, 0, 0, 0);
             fetch_res(c_begin, ea0, ea1);
           }
-          tc_ld16(t_addr + (uint32_t)c_begin, ra);
+          // a warp may own no columns (jobs narrower than 64): it must not issue a load it never waits for
+          if (c_begin < c_end) tc_ld16(t_addr + (uint32_t)c_begin, ra);
           for (int c = c_begin; c < c_end; c += 32) {
             tc_wait_ld();
             const bool more1 = c + 16 < c_end;

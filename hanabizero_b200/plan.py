@@ -204,7 +204,8 @@ class RecurrentPlan:
         self.n_support = net._value_support.numel()
         if net._reward_support.numel() != self.n_support:
             raise ValueError("value and reward supports must have the same size")
-        self.P3 = _round_up(self.n_support, 16)   # 32-byte aligned logit rows (vector loads in the decode)
+        # 32-byte aligned logit rows (vector loads in the decode), wide enough for the policy's A logits too
+        self.P3 = _round_up(max(self.n_support, self.A), 16)
         self.support = net._value_support.detach().float().contiguous()
         self._sig, self._w, self._chains = None, {}, {}
         self.refresh(force=True)

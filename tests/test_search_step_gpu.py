@@ -130,6 +130,10 @@ def _run(N, A, S, width, dtype, deep=False, seed=0):
     (64, 20, 130, 201, torch.float16),     # capacity > 64: 8 q registers per lane
     (33, 20, 300, 201, torch.float32),     # capacity > 256: general back-propagation routine
     (2048, 20, 200, 201, torch.float16),   # BASELINE configs[4] per-GPU shard: 16384 trees x 200 sims over 8 GPUs
+    (300, 20, 30, 21, torch.float16),      # narrow support: 3 of the decode's 32 lanes hold logits
+    (129, 11, 40, 21, torch.float32),
+    (300, 20, 30, 255, torch.float16),     # the widest odd support: every lane, the last one 7 columns
+    (129, 11, 40, 255, torch.float32),
 ])
 def test_search_step_equals_generic_calls(N, A, S, width, dtype):
     _run(N, A, S, width, dtype)
