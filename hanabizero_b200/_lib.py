@@ -89,6 +89,8 @@ SIGNATURES = {
     "hz_host_random_legal": (_i, [_vp, _i64, _i, _i, _i, C.c_uint64, C.c_uint32, _vp]),
     "hz_envs_check": (_i, [_vp, _vp, _vp]),
     "hz_envs_dump": (_i, [_vp, _vp, _vp]),
+    "hz_wave_pack": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
+    "hz_wave_unpack": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp]),
 }
 
 
@@ -125,6 +127,12 @@ class GemmStep(C.Structure):
                 ("bias", _vp), ("stride_bias", _i64), ("c", _vp), ("ldc", _i64), ("stride_c", _i64),
                 ("d", _vp), ("ldd", _i64), ("stride_d", _i64), ("m", C.c_int32), ("n", C.c_int32),
                 ("k", C.c_int32), ("batch", C.c_int32), ("relu", C.c_int32)]
+
+
+class WaveTicket(C.Structure):
+    """struct hz_wave_ticket (include/hzb200.h)."""
+    _fields_ = [("noise", _vp), ("reward", _vp), ("logits", _vp), ("legal", _vp), ("hidden", _vp),
+                ("out_visits", _vp), ("out_values", _vp)]
 
 
 _lib = None

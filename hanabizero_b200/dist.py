@@ -13,6 +13,16 @@ def shard_range(total, rank, world_size):
     return lo, lo + base + (1 if rank < rem else 0)
 
 
+def wave_rows(visits, values, world, wave, position):
+    """One ticket's rows of a gathered search wave (mcts.SearchPipeline(wave=G)): every rank contributes G * n rows,
+    ticket `position` owns rows [position * n, (position + 1) * n) of each.  visits [world * G * n, A] and values
+    [world * G * n] (AsyncStatsGather.result) -> ([world * n, A], [world * n]), ranks in order."""
+    a = visits.shape[-1]
+    n = visits.shape[0] // (world * wave)
+    return (visits.reshape(world, wave, n, a)[:, position].reshape(world * n, a),
+            values.reshape(world, wave, n)[:, position].reshape(world * n))
+
+
 def gather_root_stats(visits, values, group=None):
     """all_gather of per-rank (visits int32 [n, A], values float32 [n]) -> global ([N, A], [N]) on every
     rank, ranks in order.  Equal shard sizes use one all_gather_into_tensor on a packed buffer;

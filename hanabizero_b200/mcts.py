@@ -26,6 +26,7 @@ import torch
 
 from . import _lib, cytree
 from ._lib import check, ptr
+from .dist import wave_rows
 
 
 class SearchConfig:
@@ -91,6 +92,17 @@ class MCTS(object):
         amp = getattr(self.config, "amp_type", "none") == "torch_amp"
         return model.recurrent_plan(torch.float16 if amp else torch.float32)
 
+    def pool_dtype(self, model, feature, device):
+        """Element type of the hidden-state pool a search of `model` keeps (root hidden states are converted to it)."""
+        if self._plan(model) is not None:
+            return self._plan(model).dtype
+        if hasattr(model, "recurrent_inference_device"):
+            with torch.no_grad(), self._autocast():
+                probe = model.recurrent_inference_device(
+                    torch.zeros(2, feature, device=device), torch.zeros(2, 1, dtype=torch.int64, device=device))
+            return probe[3].dtype
+        return torch.float32
+
     def _workspace(self, roots, model, hidden_state_roots, gemm_sm_target=0, stage_limit=0, executor="library"):
         sims = int(self.config.num_simulations)
         key = (roots.handle.value, id(model), sims, getattr(self.config, "amp_type", "none"), self.use_plan,
@@ -99,17 +111,8 @@ class MCTS(object):
         if ws is not None and ws.model_ref() is not model:
             ws = None   # a different model object that happens to live at a recycled address
         if ws is None:
-            n, dev = roots.root_num, roots.device
             feature = int(hidden_state_roots.shape[-1])
-            if self._plan(model) is not None:
-                dtype = self._plan(model).dtype
-            elif hasattr(model, "recurrent_inference_device"):
-                with torch.no_grad(), self._autocast():
-                    probe = model.recurrent_inference_device(
-                        torch.zeros(2, feature, device=dev), torch.zeros(2, 1, dtype=torch.int64, device=dev))
-                dtype = probe[3].dtype
-            else:
-                dtype = torch.float32
+            dtype = self.pool_dtype(model, feature, roots.device)
             if len(self._ws) >= self.max_cached_workspaces:
                 self._ws.pop(next(iter(self._ws)))
             ws = self._ws[key] = _Workspace(roots, model, sims, feature, dtype)
@@ -287,6 +290,44 @@ def network_executor_for(model, num_roots, in_flight):
     return "rows"
 
 
+class WaveSchedule:
+    """Ticket bookkeeping of SearchPipeline(wave=G): the slot and position each submit takes, and when the wave that
+    is still taking tickets ("open") must launch.  Slots are used round robin; ticket id = slot * G + position."""
+
+    def __init__(self, wave, depth):
+        self.wave, self.depth = int(wave), int(depth)
+        self.open = None      # dict(slot, noisy, fraction, count) of the open wave
+        self._next = 0
+
+    def closes(self, noisy, fraction):
+        """True when a ticket of this kind cannot join the open wave: one wave is one Roots.prepare call, so the
+        noise-ness and (with noise) the exploration fraction must match."""
+        return self.open is not None and (self.open["noisy"], self.open["fraction"]) != (noisy, fraction)
+
+    def take(self, noisy, fraction):
+        """(slot, position) of the next ticket; opens a wave on the next slot when none is open (position 0)."""
+        if self.open is None:
+            self.open = dict(slot=self._next, noisy=noisy, fraction=fraction, count=0)
+            self._next = (self._next + 1) % self.depth
+        p = self.open["count"]
+        self.open["count"] += 1
+        return self.open["slot"], p
+
+    def full(self):
+        return self.open is not None and self.open["count"] == self.wave
+
+    def close(self):
+        """The open wave (to launch now); none is open afterwards."""
+        w, self.open = self.open, None
+        return w
+
+    def slot_of(self, ticket):
+        return ticket // self.wave
+
+    def is_open(self, slot):
+        return self.open is not None and self.open["slot"] == slot
+
+
 class SearchPipeline:
     """Searches kept in flight: `depth` slots, each with its own tree batch (and therefore its own captured search
     graph, network buffers and staging buffers) and its own compute stream.  Inputs are copied in on a copy stream and
@@ -315,48 +356,89 @@ class SearchPipeline:
     (default gemm_sm_target_for(num_roots, depth)) sizes each search's library GEMMs for a share of the SMs, and
     `stage_limit` (default 4) keeps the tree step's shared-memory footprint small enough to sit next to a GEMM CTA.
     Results per search are those of MCTS.run_multi with the same two settings (the SM target changes the rounding of
-    the network outputs in the last bits, the staging limit changes nothing)."""
+    the network outputs in the last bits, the staging limit changes nothing).
+
+    Waves (`wave` = G > 1): a slot holds G tickets of `num_roots` trees each and searches them together as ONE batch of
+    G * num_roots trees — one input pack (hz_wave_pack), one graph launch, one statistics kernel, one output scatter
+    (hz_wave_unpack) and, with `gather`, one all-gather per wave instead of one of each per ticket.  Trees never
+    interact, so each ticket gets exactly its own rows back: on the row-block executor they equal, bit for bit, a
+    stand-alone Roots(num_roots) + run_multi of that ticket alone; on the library chain, where cuBLASLt may pick other
+    kernels for G * num_roots rows, they equal one run_multi over the concatenated batch.  submit() returns the ticket
+    id slot * G + position (the slot index for G = 1).  A wave launches when its G-th ticket arrives, on flush(), or
+    when wait / stats / gathered names one of its tickets; a submit whose exploration fraction or noise-ness (noises vs
+    None) differs from the open wave's launches the open wave first.  A partial wave runs the full-size search with
+    padding roots (no legal action) in its unused positions.  Inputs that are already float32 / int32 legal mask / the
+    hidden-state pool's dtype, contiguous and on this device or in page-locked host memory are read by the pack kernel
+    in place (keep them unchanged until wait(ticket)); outputs of that kind are written in place.  Anything else is
+    converted by torch on the caller's stream first, or copied out after the scatter: the slow path.  The executor and
+    SM-target rules see the wave's G * num_roots trees.  Waves of 4096 trees need only 7-8 slots in flight, so unlike
+    depth-20 pipelines of small searches they need no CUDA_DEVICE_MAX_CONNECTIONS above its default of 8.
+
+    Waves fill only when a caller submits tickets ahead of its waits: a wait / stats / gathered on a ticket of the open
+    wave launches it with the tickets it holds so far, so submit-then-wait per ticket runs waves of one ticket.  Ticket
+    ids are reused round robin: consume a ticket before `depth` more waves open (wait with a lag below depth * G
+    tickets), or the id names the slot's newer wave: wait() then launches that wave early, and stats() / gathered()
+    return the newer wave's rows (as for G = 1, a slot's statistics are valid until it is submitted again).  The
+    pipeline is not thread-safe: callers on several threads need one lock around every call (submit, wait, stats,
+    gathered, flush, drain)."""
 
     def __init__(self, mcts, model, num_roots, num_actions, depth=8, device=None, gather=None, gemm_sm_target=None,
-                 stage_limit=None, executor="auto"):
+                 stage_limit=None, executor="auto", wave=1):
         self.mcts, self.model = mcts, model
         self.depth = int(depth)
+        self.wave = int(wave)
+        if not 1 <= self.wave <= 64:
+            raise ValueError("wave must be 1..64 tickets")
+        rows = self.wave * int(num_roots)   # trees per slot
         # "rows": the network as one row-block resident launch per simulation (BoundChain.set_executor) — a quarter of
         # the SMs per search at 4096 trees, which is what searches in flight want; "library": seven (Hanabi-Full) or
         # five (Hanabi-Small) cuBLASLt launches, the lower latency for a search that runs alone.  "auto": see
         # network_executor_for (plans the row executor does not cover fall back to the library chain inside MCTS).
-        self.executor = network_executor_for(model, num_roots, self.depth) if executor == "auto" else executor
+        self.executor = network_executor_for(model, rows, self.depth) if executor == "auto" else executor
         self.n, self.a, self.depth = int(num_roots), int(num_actions), int(depth)
-        self.device = next(model.parameters()).device if device is None else torch.device(device)
+        device = next(model.parameters()).device if device is None else device
+        # always indexed ("cuda" -> "cuda:<current>"): tensors report indexed devices, and inputs / outputs are matched
+        # against this one to be read or written in place
+        self.device = torch.device("cuda", cytree._device_index(device))
         dev, sims = self.device, int(mcts.config.num_simulations)
         if gemm_sm_target is None:
-            gemm_sm_target = gemm_sm_target_for(self.n, self.depth, dev)
+            gemm_sm_target = gemm_sm_target_for(rows, self.depth, dev)
         self.gemm_sm_target = int(gemm_sm_target)
         # searches in flight: a small staging region lets the tree step share SMs with the other slots' GEMM CTAs
         self.stage_limit = (STAGE_LIMIT_IN_FLIGHT if self.depth > 1 else 0) if stage_limit is None else int(stage_limit)
         mcts.max_cached_workspaces = max(mcts.max_cached_workspaces, self.depth + 4)   # one workspace (graph) per slot
         if gather is not None and gather.depth < self.depth:
             raise ValueError("gather.depth must be at least the pipeline depth")
+        if gather is not None and gather.n != rows:
+            raise ValueError("gather.n must be wave * num_roots (the trees of one slot)")
         self.gather = gather
         self.copy_in, self.copy_out = torch.cuda.Stream(dev), torch.cuda.Stream(dev)
         self.slots = []
         for _ in range(self.depth):
             self.slots.append(dict(
-                roots=cytree.Roots(self.n, self.a, sims, device=dev), stream=torch.cuda.Stream(dev),
-                noise=torch.empty(self.n, self.a, device=dev), reward=torch.empty(self.n, device=dev),
-                logits=torch.empty(self.n, self.a, device=dev), legal=torch.empty(self.n, self.a, dtype=torch.int32, device=dev),
+                roots=cytree.Roots(rows, self.a, sims, device=dev), stream=torch.cuda.Stream(dev),
+                noise=torch.empty(rows, self.a, device=dev), reward=torch.empty(rows, device=dev),
+                logits=torch.empty(rows, self.a, device=dev), legal=torch.empty(rows, self.a, dtype=torch.int32, device=dev),
                 hidden=None, stats=None, visits=None, values=None, ticket=None,
                 ev_in=torch.cuda.Event(), ev_done=torch.cuda.Event(), ev_out=torch.cuda.Event(), busy=False))
         for s in self.slots:
             # one int32 buffer [n * A visit counts | n value bit patterns]: the statistics kernel writes both parts in
             # place and the all-gather ships the buffer as it is (no packing kernels)
-            s["stats"] = torch.empty(self.n * (self.a + 1), dtype=torch.int32, device=dev)
-            s["visits"] = s["stats"][:self.n * self.a].view(self.n, self.a)
-            s["values"] = s["stats"][self.n * self.a:].view(torch.float32)
+            s["stats"] = torch.empty(rows * (self.a + 1), dtype=torch.int32, device=dev)
+            s["visits"] = s["stats"][:rows * self.a].view(rows, self.a)
+            s["values"] = s["stats"][rows * self.a:].view(torch.float32)
+            if self.wave > 1:
+                # the open wave: its tickets' table entries, the inputs they point at, slow-path outputs, and one
+                # caller-stream event per ticket that the slot's stream waits for at launch
+                s.update(table=[], keep=[], post=[], ev_tickets=[torch.cuda.Event() for _ in range(self.wave)])
         self._next = 0
+        self._waves = WaveSchedule(self.wave, self.depth)
+        self._hidden_shape = None    # wave > 1: (feature, pool dtype) of the root hidden states
         self.host_seconds, self.submitted = 0.0, 0
 
     def submit(self, fraction, noises, rewards, logits, legal, hidden_roots, out_visits=None, out_values=None):
+        if self.wave > 1:
+            return self._submit_to_wave(fraction, noises, rewards, logits, legal, hidden_roots, out_visits, out_values)
         i = self._next
         self._next = (i + 1) % self.depth
         s = self.slots[i]
@@ -419,21 +501,147 @@ class SearchPipeline:
         return (isinstance(x, torch.Tensor) and x.device == like.device and x.dtype == like.dtype and x.shape == like.shape
                 and x.is_contiguous())
 
+    def _submit_to_wave(self, fraction, noises, rewards, logits, legal, hidden_roots, out_visits, out_values):
+        t_host = time.perf_counter()
+        noisy = noises is not None
+        fraction = float(fraction) if noisy else 0.0
+        if self._waves.closes(noisy, fraction):
+            self._launch_wave()
+        hidden_roots = torch.as_tensor(hidden_roots)
+        if self._hidden_shape is None:
+            feature = int(hidden_roots.shape[-1])
+            hidden_shape = (feature, self.mcts.pool_dtype(self.model, feature, self.device))
+        else:
+            hidden_shape = self._hidden_shape
+        feature, hdtype = hidden_shape
+        # every input converted and every output checked BEFORE the ticket takes a position: a bad argument raises here
+        # and leaves the open wave as it was
+        n, a, held = self.n, self.a, []
+        rec = _lib.WaveTicket()
+        rec.noise = self._wave_input(noises, torch.float32, (n, a), held)
+        rec.reward = self._wave_input(rewards, torch.float32, (n,), held)
+        rec.logits = self._wave_input(logits, torch.float32, (n, a), held)
+        rec.legal = self._wave_input(legal, torch.int32, (n, a), held)
+        rec.hidden = self._wave_input(hidden_roots, hdtype, (n, feature), held)
+        in_place = [self._wave_output(x, dtype, shape) for x, dtype, shape in
+                    ((out_visits, torch.int32, (n, a)), (out_values, torch.float32, (n,)))]
+        self._hidden_shape = hidden_shape
+        i, p = self._waves.take(noisy, fraction)
+        s = self.slots[i]
+        if p == 0:
+            if s["busy"]:
+                t_wait = time.perf_counter()
+                s["ev_out"].synchronize()   # the slot's previous wave has been read out
+                t_host += time.perf_counter() - t_wait   # waiting for the GPU is not host time
+            s["busy"] = True
+            s["table"], s["keep"], s["post"] = [], [], []
+            if s["hidden"] is None:
+                s["hidden"] = torch.empty(self.wave * self.n, feature, dtype=hdtype, device=self.device)
+        s["keep"] += held                   # alive until the slot is reused
+        rows = slice(p * n, (p + 1) * n)
+        for out, ok, buf in zip((out_visits, out_values), in_place, (s["visits"], s["values"])):
+            if out is not None and not ok:
+                s["post"].append((out, buf[rows]))
+        rec.out_visits = ptr(out_visits) if in_place[0] else None
+        rec.out_values = ptr(out_values) if in_place[1] else None
+        s["table"].append(rec)
+        s["ev_tickets"][p].record(torch.cuda.current_stream(self.device))   # after whatever produced the inputs
+        if self._waves.full():
+            self._launch_wave()
+        self.host_seconds += time.perf_counter() - t_host
+        self.submitted += 1
+        return i * self.wave + p    # ticket id
+
+    def _readable_in_place(self, x, dtype, shape):
+        return (isinstance(x, torch.Tensor) and x.dtype == dtype and tuple(x.shape) == shape and x.is_contiguous()
+                and (x.device == self.device or (x.device.type == "cpu" and x.is_pinned())))
+
+    def _wave_input(self, x, dtype, shape, held):
+        """Address the pack kernel reads a ticket input from (None -> NULL); the tensor read is appended to `held`."""
+        if x is None:
+            return None
+        if not self._readable_in_place(x, dtype, shape):
+            x = cytree.as_device(x, dtype, self.device, shape)     # slow path: torch converts on the caller's stream
+        held.append(x)
+        return x.data_ptr()
+
+    def _wave_output(self, x, dtype, shape):
+        """True when the scatter kernel can write a ticket output in place; False for the slow path (a torch copy after
+        the scatter).  An output that cannot take the ticket's rows raises."""
+        if x is None:
+            return False
+        if not isinstance(x, torch.Tensor) or x.numel() != int(np.prod(shape)):
+            raise ValueError(f"outputs must be tensors of {int(np.prod(shape))} elements {shape}")
+        return self._readable_in_place(x, dtype, shape)
+
+    def _launch_wave(self):
+        """Search the open wave: pack -> prepare -> run_multi -> root statistics -> (all-gather) -> scatter, all on
+        the slot's stream after the events its tickets recorded on their callers' streams."""
+        w = self._waves.close()
+        s = self.slots[w["slot"]]
+        roots, compute, count = s["roots"], s["stream"], len(s["table"])
+        lib, dev = roots._lib, roots.device_index
+        for ev in s["ev_tickets"][:count]:
+            compute.wait_event(ev)
+        if self.gather is not None and s["ticket"] is not None and self.gather.stream is not None:
+            compute.wait_event(self.gather.slots[s["ticket"]]["done"])   # the stats buffer was its send buffer
+        table = (_lib.WaveTicket * count)(*s["table"])
+        st = compute.cuda_stream
+        with torch.cuda.stream(compute):
+            check(lib.hz_wave_pack(st, dev, table, count, self.wave, self.n, self.a,
+                                   s["hidden"].shape[1] * s["hidden"].element_size(),
+                                   ptr(s["noise"]) if w["noisy"] else None, ptr(s["reward"]), ptr(s["logits"]),
+                                   ptr(s["legal"]), ptr(s["hidden"])))
+            if w["noisy"]:
+                roots.prepare(w["fraction"], s["noise"], s["reward"], s["logits"], s["legal"])
+            else:
+                roots.prepare_no_noise(s["reward"], s["logits"], s["legal"])
+            self.mcts.run_multi(roots, self.model, s["hidden"], gemm_sm_target=self.gemm_sm_target,
+                                stage_limit=self.stage_limit, executor=self.executor)
+            check(lib.hz_trees_root_stats(roots.handle, st, ptr(s["visits"]), ptr(s["values"])))
+            s["ev_done"].record(compute)
+            if self.gather is not None:
+                s["ticket"] = self.gather.submit_flat(s["stats"])
+            check(lib.hz_wave_unpack(st, dev, table, count, self.wave, self.n, self.a, ptr(s["stats"])))
+            for out, rows in s["post"]:
+                out.copy_(rows.reshape(out.shape), non_blocking=True)
+            s["ev_out"].record(compute)
+
+    def flush(self):
+        """Launch the open wave now, with however many tickets it holds (nothing to do for wave = 1)."""
+        if self._waves.open is not None:
+            t_host = time.perf_counter()
+            self._launch_wave()
+            self.host_seconds += time.perf_counter() - t_host
+
+    def _slot_of(self, ticket):
+        """Slot of a ticket; launches the ticket's wave if it is still open."""
+        slot = self._waves.slot_of(ticket)
+        if self._waves.is_open(slot):
+            self.flush()
+        return slot
+
     def wait(self, ticket):
-        self.slots[ticket]["ev_out"].synchronize()
+        self.slots[self._slot_of(ticket)]["ev_out"].synchronize()
 
     def stats(self, ticket):
-        """Device tensors (visits int32 [n, A], values float32 [n]) of a ticket's search; valid until the slot is
-        submitted again.  The current stream waits for the search."""
-        s = self.slots[ticket]
+        """Device tensors (visits int32 [n, A], values float32 [n]) of a ticket's search (its rows of the wave's
+        buffer); valid until the slot is submitted again.  The current stream waits for the search."""
+        s = self.slots[self._slot_of(ticket)]
         torch.cuda.current_stream(self.device).wait_event(s["ev_done"])
-        return s["visits"], s["values"]
+        rows = slice(ticket % self.wave * self.n, (ticket % self.wave + 1) * self.n)
+        return s["visits"][rows], s["values"][rows]
 
     def gathered(self, ticket):
-        """All ranks' statistics of a ticket's search (needs `gather`); the current stream waits for the collective."""
-        return self.gather.result(self.slots[ticket]["ticket"])
+        """All ranks' statistics of a ticket's search (needs `gather`), [world * n, A] and [world * n], ranks in order;
+        the current stream waits for the collective."""
+        visits, values = self.gather.result(self.slots[self._slot_of(ticket)]["ticket"])
+        if self.wave == 1:
+            return visits, values
+        return wave_rows(visits, values, self.gather.world, self.wave, ticket % self.wave)
 
     def drain(self):
+        self.flush()
         for s in self.slots:
             if s["busy"]:
                 s["ev_out"].synchronize()

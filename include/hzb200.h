@@ -429,6 +429,38 @@ int hz_rowchain_grid(const hz_rowchain* e);                     /* CTAs per laun
 int hz_rowchain_set_trace(hz_rowchain* e, int enable);
 int hz_rowchain_read_trace(hz_rowchain* e, uint64_t* host_out, int64_t count);                          /* sync */
 
+/* ------------------------------------------------------------------------------------------
+ * Search waves: `count` independent root batches ("tickets") of n roots each searched as ONE batch of slots * n trees
+ * (hanabizero_b200/mcts.py SearchPipeline(wave=slots); the reference's actors each submit their own p_mcts_num roots,
+ * core/selfplay_worker.py:93-102).  Ticket k owns rows [k*n, (k+1)*n) of the wave.  Every pointer of the table and
+ * every buffer is device memory of `device` or page-locked host memory (read and written by the kernel itself under
+ * unified addressing, as hz_envs_host_step does); anything else (pageable host memory, another device's memory), a
+ * misaligned pointer (16 bytes for hidden, 4 for the rest), count outside 1..slots, slots outside 1..64, num_actions
+ * outside 1..32, n < 1, slots * n > 2^24 or hidden_row_bytes not a multiple of 16 in 16..65536 is HZ_ERR_ARG, checked
+ * before anything is launched.  The table is passed to the kernel by value: it may be reused as soon as the call
+ * returns.  Both calls are one launch and asynchronous; the ticket buffers must stay valid until the stream gets there.
+ * ------------------------------------------------------------------------------------------ */
+typedef struct hz_wave_ticket {
+  const float* noise;      /* [n][A] or NULL (= zeros) */
+  const float* reward;     /* [n] */
+  const float* logits;     /* [n][A] */
+  const int32_t* legal;    /* [n][A] */
+  const void* hidden;      /* [n][hidden_row_bytes] */
+  int32_t* out_visits;     /* [n][A] or NULL (hz_wave_unpack only) */
+  float* out_values;       /* [n] or NULL (hz_wave_unpack only) */
+} hz_wave_ticket;
+/* Fills the wave's staging buffers (slots * n rows, the inputs of hz_trees_prepare and of the search's hidden-state
+ * pool): ticket k's rows go to rows [k*n, (k+1)*n); the rows of slots count..slots-1 become padding roots with zero
+ * noise, reward, logits and hidden state and an all-zero legal mask (a root without children), so a partial wave runs
+ * the full-size search unchanged.  noise == NULL (a wave prepared without noise) leaves the noise rows unwritten. */
+int hz_wave_pack(void* stream, int device, const hz_wave_ticket* tickets, int count, int slots, int n, int num_actions,
+                 int hidden_row_bytes, float* noise, float* reward, float* logits, int32_t* legal, void* hidden);
+/* Scatters the wave's root statistics, laid out as hz_trees_root_stats writes them into one int32 buffer
+ * stats = [slots*n*A visit counts | slots*n value bit patterns], to every ticket's out_visits / out_values (NULL = not
+ * wanted).  `slots` is the wave's size, which places the value block. */
+int hz_wave_unpack(void* stream, int device, const hz_wave_ticket* tickets, int count, int slots, int n,
+                   int num_actions, const int32_t* stats);
+
 #ifdef __cplusplus
 }
 #endif
