@@ -304,6 +304,27 @@ class RecurrentPlan:
         return dec[:n], dec[n:], ch.policy_logits[:, :self.A].float().contiguous()
 
 
+class BoundInitial:
+    """InitialPlan's static buffers and GEMM chain for one (n, owner).  It owns its hz_gemm_plan (a cuBLASLt handle and
+    a 32 MB device workspace), released with the object."""
+
+    def __init__(self, lib, owner):
+        self.lib, self.handle = lib, C.c_void_p()
+        self._owner = None if owner is None else weakref.ref(owner)
+
+    def owner_collected(self):
+        return self._owner is not None and self._owner() is None
+
+    def __del__(self):
+        h = getattr(self, "handle", None)
+        if h:
+            try:
+                self.lib.hz_gemm_plan_destroy(h)
+            except Exception:
+                pass
+            self.handle = None
+
+
 class InitialPlan:
     """Execution plan for `initial_inference` in eval mode (representation + policy / value heads;
     /root/reference/core/model.py:61-72, config/hanabi_control/model.py:127-335) — the per-move counterpart of
@@ -386,10 +407,14 @@ class InitialPlan:
     def bound(self, n, owner=None):
         """Static buffers + GEMM chain for batch size n (cached per (n, owner); `x` is the input buffer hz_ring_gather
         fills).  Callers that may run at the same time on different streams (the engines of a SelfPlayPool) pass
-        themselves as `owner` and get buffers of their own."""
+        themselves as `owner` and get buffers of their own.  Every call first drops the entries of owners that have been
+        collected (a dead engine's buffers and GEMM plan go now, not when the cache evicts them); a remaining entry
+        under id(owner) therefore belongs to `owner`, since live objects have distinct ids."""
+        for k in [k for k, v in self._bound.items() if v.owner_collected()]:
+            del self._bound[k]
         key = (n, None if owner is None else id(owner))
         b = self._bound.get(key)
-        if b is not None and (owner is None or b.owner() is owner):
+        if b is not None:
             return b
         dev, dt, w = self.device, self.dtype, self._w
         F, H, P3 = self.F, self.H, self.P3
@@ -406,7 +431,7 @@ class InitialPlan:
             s.m, s.n, s.k, s.batch, s.relu = m, nn, k, batch, 1 if relu else 0
             steps.append(s)
 
-        b = type("BoundInitial", (), {})()
+        b = BoundInitial(self.lib, owner)
         b.x = z(n, self.K0)
         b.state = z(n, F)
         b.h1 = z(n, 2 * H)
@@ -435,9 +460,7 @@ class InitialPlan:
             step(b.h1, w["WB3"], w["bB3"], b.out, n, P3, H, relu=False, batch=2, sa=H, sw=P3 * H, sb=P3, sd=n * P3, lda=2 * H)
         b.n_steps = len(steps)
         arr = (GemmStep * b.n_steps)(*steps)
-        b.handle = C.c_void_p()
         check(self.lib.hz_gemm_plan_create(C.byref(b.handle), dev.index, b.x.element_size(), arr, b.n_steps))
-        b.owner = (lambda: None) if owner is None else weakref.ref(owner)
         if len(self._bound) >= 16:
             self._bound.pop(next(iter(self._bound)))   # buffers stay alive while a caller holds the object
         self._bound[key] = b
