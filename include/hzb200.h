@@ -115,7 +115,9 @@ typedef struct hz_search_io {
   int32_t state_cols;         /* state_cols * elem_bytes must be a multiple of 16 */
   void* out_batch;            /* [N][ld_batch]: state_cols of hidden state, then onehot_cols of one-hot */
   int64_t ld_batch;           /* elements; ld_batch * elem_bytes multiple of 16 */
-  int32_t onehot_cols;        /* 0..32; columns >= num_actions stay zero */
+  int32_t onehot_cols;        /* 0 (no one-hot columns are written) or num_actions..32; columns >= num_actions are
+                               * written as zero.  1..num_actions-1 is an argument error: an action without a column
+                               * would reach the network as an all-zero one-hot */
   int32_t* out_ix;            /* optional int32[N]: parent hidden-state index x */
   int32_t* out_action;        /* optional int32[N]: last action */
   /* search constants */

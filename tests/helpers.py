@@ -52,6 +52,14 @@ def bits_equal(a, b):
     return a.shape == b.shape and bool((a == b).all())
 
 
+def nan_to_zero(logits):
+    """Policy logits as the search hands them to the tree (core/mcts.py:48-49): float32 with NaN -> 0 and nothing
+    else; +-inf stay infinite (np.nan_to_num would turn them into +-FLT_MAX)."""
+    a = np.array(logits, dtype=np.float32, copy=True)
+    a[np.isnan(a)] = 0.0
+    return a
+
+
 def run_tree_lockstep(engine, g, d, check_each_sim=True):
     """Drive `engine` (oracle.loader.TreeEngine-like API) through the golden trace `g`."""
     S = int(g["S"])

@@ -4,6 +4,8 @@ import numpy as np
 import pytest
 import torch
 
+from helpers import nan_to_zero
+
 pytestmark = pytest.mark.gpu
 
 N, A, S = 96, 20, 24
@@ -64,7 +66,7 @@ def _oracle_replay(rec, cfg, noise, logits, legal, a):
     for x, (v, rw, lg, _, _, _) in enumerate(rec, start=1):
         trace.append(cpu.traverse(cfg.pb_c_base, cfg.pb_c_init, cfg.discount))
         cpu.backprop(x, cfg.discount, rw.float().cpu().numpy(), v.float().cpu().numpy(),
-                     np.nan_to_num(lg.float().cpu().numpy(), nan=0.0))
+                     nan_to_zero(lg.float().cpu().numpy()))
     return cpu, trace
 
 
