@@ -91,6 +91,7 @@ SIGNATURES = {
     "hz_envs_dump": (_i, [_vp, _vp, _vp]),
     "hz_wave_pack": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "hz_wave_unpack": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp]),
+    "hz_obs_pack": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
 }
 
 
@@ -133,6 +134,22 @@ class WaveTicket(C.Structure):
     """struct hz_wave_ticket (include/hzb200.h)."""
     _fields_ = [("noise", _vp), ("reward", _vp), ("logits", _vp), ("legal", _vp), ("hidden", _vp),
                 ("out_visits", _vp), ("out_values", _vp)]
+
+
+HZ_OBS_F32, HZ_OBS_U8, HZ_OBS_BITS = 0, 1, 2
+HZ_LEGAL_I32, HZ_LEGAL_F32, HZ_LEGAL_MASK = 0, 1, 2
+
+
+class ObsTicket(C.Structure):
+    """struct hz_obs_ticket (include/hzb200.h)."""
+    _fields_ = [("obs", _vp), ("ld_obs", _i64), ("legal", _vp), ("ld_legal", _i64), ("noise", _vp),
+                ("obs_format", C.c_int32), ("legal_format", C.c_int32)]
+
+
+class ObsLayout(C.Structure):
+    """struct hz_obs_layout (include/hzb200.h)."""
+    _fields_ = [("stack", C.c_int32), ("frame_dim", C.c_int32), ("frame_stride", C.c_int32), ("elem_bytes", C.c_int32),
+                ("frame_words", C.c_int32), ("bit_offset", C.c_int32)]
 
 
 _lib = None

@@ -49,4 +49,25 @@ struct DeviceGuard {
   int target = -1;
 };
 
+// Non-NULL `p` must be device memory of `device` or page-locked host memory, aligned to `align` bytes.
+inline int check_ptr(const char* fn, const char* what, const void* p, int device, int align) {
+  if (!p) return HZ_OK;
+  if ((uintptr_t)p % align) { set_error("%s: %s must be %d-byte aligned", fn, what, align); return HZ_ERR_ARG; }
+  cudaPointerAttributes at{};
+  const cudaError_t e = cudaPointerGetAttributes(&at, p);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    return fail_cuda(e, fn);
+  }
+  if (at.type == cudaMemoryTypeDevice && at.device == device) return HZ_OK;
+  if (at.type == cudaMemoryTypeHost && at.devicePointer == p) return HZ_OK;
+  if (at.type == cudaMemoryTypeDevice) {
+    set_error("%s: %s is memory of device %d, not of device %d", fn, what, at.device, device);
+  } else {
+    set_error("%s: %s must be device memory of device %d or page-locked host memory (torch .pin_memory(), "
+              "cudaHostAlloc)", fn, what, device);
+  }
+  return HZ_ERR_ARG;
+}
+
 }  // namespace hz

@@ -80,27 +80,6 @@ static int check_sizes(const char* fn, const hz_wave_ticket* tickets, int count,
   return HZ_OK;
 }
 
-// Non-NULL `p` must be device memory of `device` or page-locked host memory, aligned to `align` bytes.
-static int check_ptr(const char* fn, const char* what, const void* p, int device, int align) {
-  if (!p) return HZ_OK;
-  if ((uintptr_t)p % align) { set_error("%s: %s must be %d-byte aligned", fn, what, align); return HZ_ERR_ARG; }
-  cudaPointerAttributes at{};
-  const cudaError_t e = cudaPointerGetAttributes(&at, p);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    return fail_cuda(e, fn);
-  }
-  if (at.type == cudaMemoryTypeDevice && at.device == device) return HZ_OK;
-  if (at.type == cudaMemoryTypeHost && at.devicePointer == p) return HZ_OK;
-  if (at.type == cudaMemoryTypeDevice) {
-    set_error("%s: %s is memory of device %d, not of device %d", fn, what, at.device, device);
-  } else {
-    set_error("%s: %s must be device memory of device %d or page-locked host memory (torch .pin_memory(), "
-              "cudaHostAlloc)", fn, what, device);
-  }
-  return HZ_ERR_ARG;
-}
-
 }  // namespace hz
 
 using namespace hz;

@@ -197,6 +197,20 @@ class HanabiVecEnv:
         return out
 
 
+def frame_layout(hanabi_name, mdp, device=None):
+    """(frame_dim, frame_words, bit_offset) of the observation frame a network of `hanabi_name` takes for `mdp`
+    ("global" or "local"), read from the game kernels' own dimensions (hz_envs_dims): the frame is bits
+    [bit_offset, bit_offset + frame_dim) of the packed string of frame_words words that step_bits / EnvPipeline(fmt="bits")
+    hand out per game — the whole string for "global", its local suffix for "local"."""
+    if mdp not in ("global", "local"):
+        raise ValueError("mdp must be 'global' or 'local'")
+    env = HanabiVecEnv(1, hanabi_name, device=device)
+    words = (env.global_dim + 31) // 32
+    if mdp == "global":
+        return env.global_dim, words, 0
+    return env.local_dim, words, env.global_dim - env.local_dim
+
+
 class EnvPipeline:
     """Host-driven stepping, double-buffered like mcts.SearchPipeline: the games are held as several independent
     GROUPS (one HanabiVecEnv each); every group has its own stream on which a step is

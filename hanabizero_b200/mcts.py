@@ -253,6 +253,12 @@ class MCTS(object):
     search = run_multi  # upstream EfficientZero name (BASELINE.json north_star)
 
 
+def _as_tensor(x):
+    """A torch tensor of `x` (numpy, lists); uint32 words (packed bits, bit masks) as the int32 the kernels take."""
+    x = x if isinstance(x, torch.Tensor) else torch.as_tensor(np.asarray(x))
+    return x.view(torch.int32) if x.dtype == torch.uint32 else x
+
+
 def _flat(x):
     return x.reshape(-1) if isinstance(x, torch.Tensor) else np.asarray(x).reshape(-1)
 
@@ -374,6 +380,10 @@ class SearchPipeline:
     SM-target rules see the wave's G * num_roots trees.  Waves of 4096 trees need only 7-8 slots in flight, so unlike
     depth-20 pipelines of small searches they need no CUDA_DEVICE_MAX_CONNECTIONS above its default of 8.
 
+    Observation tickets (`stack` = frames per root, `mdp` = "global" or "local"): submit_observations() hands in
+    stacked observations instead of the representation network's outputs, and the slot runs the root inference itself
+    (InitialPlan, one pack launch hz_obs_pack in place of hz_wave_pack).  A wave holds one kind of ticket.
+
     Waves fill only when a caller submits tickets ahead of its waits: a wait / stats / gathered on a ticket of the open
     wave launches it with the tickets it holds so far, so submit-then-wait per ticket runs waves of one ticket.  Ticket
     ids are reused round robin: consume a ticket before `depth` more waves open (wait with a lag below depth * G
@@ -383,7 +393,7 @@ class SearchPipeline:
     gathered, flush, drain)."""
 
     def __init__(self, mcts, model, num_roots, num_actions, depth=8, device=None, gather=None, gemm_sm_target=None,
-                 stage_limit=None, executor="auto", wave=1):
+                 stage_limit=None, executor="auto", wave=1, stack=None, mdp="global"):
         self.mcts, self.model = mcts, model
         self.depth = int(depth)
         self.wave = int(wave)
@@ -427,13 +437,30 @@ class SearchPipeline:
             s["stats"] = torch.empty(rows * (self.a + 1), dtype=torch.int32, device=dev)
             s["visits"] = s["stats"][:rows * self.a].view(rows, self.a)
             s["values"] = s["stats"][rows * self.a:].view(torch.float32)
-            if self.wave > 1:
+            if self.wave > 1 or stack is not None:
                 # the open wave: its tickets' table entries, the inputs they point at, slow-path outputs, and one
                 # caller-stream event per ticket that the slot's stream waits for at launch
-                s.update(table=[], keep=[], post=[], ev_tickets=[torch.cuda.Event() for _ in range(self.wave)])
+                s.update(table=[], keep=[], post=[], ev_tickets=[torch.cuda.Event() for _ in range(self.wave)],
+                         kind="hidden", obs_table=[])
         self._next = 0
         self._waves = WaveSchedule(self.wave, self.depth)
         self._hidden_shape = None    # wave > 1: (feature, pool dtype) of the root hidden states
+        self.stack, self._iplan = None if stack is None else int(stack), None
+        if self.stack is not None:
+            # observation tickets: the frame layout of the network's input, and per slot the root inference's own
+            # buffers and cuBLASLt plan (InitialPlan.bound with the slot's tree batch as owner), sized for the wave
+            from .hanabi_env import frame_layout
+            self.frame_dim, self.frame_words, bit_offset = frame_layout(
+                "Hanabi-Full" if getattr(model, "full", True) else "Hanabi-Small", mdp, dev)
+            amp = getattr(mcts.config, "amp_type", "none") == "torch_amp"
+            self._iplan = model.initial_plan(torch.float16 if amp else torch.float32, self.frame_dim, self.stack)
+            self._layout = _lib.ObsLayout(self.stack, self.frame_dim, self._iplan.frame_stride,
+                                          self._iplan.dtype.itemsize, self.frame_words, bit_offset)
+            self._zero_reward = torch.zeros(rows, device=dev)   # the root reward of initial_inference is 0
+            for s in self.slots:
+                s["ibound"] = self._iplan.bound(rows, owner=s["roots"])
+                if self.gemm_sm_target:
+                    check(self._iplan.lib.hz_gemm_plan_set_sm_target(s["ibound"].handle, self.gemm_sm_target))
         self.host_seconds, self.submitted = 0.0, 0
 
     def submit(self, fraction, noises, rewards, logits, legal, hidden_roots, out_visits=None, out_values=None):
@@ -505,7 +532,7 @@ class SearchPipeline:
         t_host = time.perf_counter()
         noisy = noises is not None
         fraction = float(fraction) if noisy else 0.0
-        if self._waves.closes(noisy, fraction):
+        if self._waves.closes(noisy, fraction) or self._open_kind() == "obs":
             self._launch_wave()
         hidden_roots = torch.as_tensor(hidden_roots)
         if self._hidden_shape is None:
@@ -526,7 +553,20 @@ class SearchPipeline:
         in_place = [self._wave_output(x, dtype, shape) for x, dtype, shape in
                     ((out_visits, torch.int32, (n, a)), (out_values, torch.float32, (n,)))]
         self._hidden_shape = hidden_shape
+        return self._join("hidden", noisy, fraction, rec, None, held, in_place, out_visits, out_values, t_host)
+
+    def _open_kind(self):
+        """Kind of ticket ("hidden" or "obs") the open wave holds, None when no wave is open."""
+        return None if self._waves.open is None else self.slots[self._waves.open["slot"]]["kind"]
+
+    def _join(self, kind, noisy, fraction, rec, obs_rec, held, in_place, out_visits, out_values, t_host):
+        """The ticket takes the next position of the open wave (opening one if needed), launching it when full."""
+        n = self.n
+        if self.wave == 1:
+            self._waves._next = self._next      # submit() and observation tickets share the round robin over slots
         i, p = self._waves.take(noisy, fraction)
+        if self.wave == 1:
+            self._next = self._waves._next
         s = self.slots[i]
         if p == 0:
             if s["busy"]:
@@ -534,9 +574,7 @@ class SearchPipeline:
                 s["ev_out"].synchronize()   # the slot's previous wave has been read out
                 t_host += time.perf_counter() - t_wait   # waiting for the GPU is not host time
             s["busy"] = True
-            s["table"], s["keep"], s["post"] = [], [], []
-            if s["hidden"] is None:
-                s["hidden"] = torch.empty(self.wave * self.n, feature, dtype=hdtype, device=self.device)
+            s["table"], s["keep"], s["post"], s["obs_table"], s["kind"] = [], [], [], [], kind
         s["keep"] += held                   # alive until the slot is reused
         rows = slice(p * n, (p + 1) * n)
         for out, ok, buf in zip((out_visits, out_values), in_place, (s["visits"], s["values"])):
@@ -545,12 +583,89 @@ class SearchPipeline:
         rec.out_visits = ptr(out_visits) if in_place[0] else None
         rec.out_values = ptr(out_values) if in_place[1] else None
         s["table"].append(rec)
+        if obs_rec is not None:
+            s["obs_table"].append(obs_rec)
         s["ev_tickets"][p].record(torch.cuda.current_stream(self.device))   # after whatever produced the inputs
         if self._waves.full():
             self._launch_wave()
         self.host_seconds += time.perf_counter() - t_host
         self.submitted += 1
         return i * self.wave + p    # ticket id
+
+    def submit_observations(self, fraction, noises, obs, legal, out_visits=None, out_values=None):
+        """A search that starts from stacked observations (core/selfplay_worker.py:258-283: stack_obs ->
+        initial_inference -> prepare -> run_multi) instead of the representation network's outputs; needs a pipeline
+        built with `stack` (frames per root) and `mdp` ("global" or "local" observations).  The root inference runs in
+        the slot (InitialPlan of the model, fp16 for amp_type "torch_amp"), the root reward is 0, and the results are
+        those of submit() with the hidden states, logits and legal mask that inference gives.  Returns a ticket id as
+        submit() does; a ticket of the other kind (submit) launches the open wave first, as a change of noise-ness does.
+
+        obs: the frames of every root, oldest first, as float32 or uint8 0/1 values [n, stack, D] (or [n, stack * D]),
+        or as packed bits: int32 [n, stack, W] (or [n, stack * W]), each frame the W-word string that step_bits /
+        EnvPipeline(fmt="bits") hand out, of which the pack kernel takes the global observation or its local suffix
+        (hanabi_env.frame_layout).  legal: int32 or float32 [n, A], or one int32 bit mask word per root ([n]; e.g.
+        `meta[:, 0]` of EnvPipeline's meta rows).  noises: float32 [n, A] or None (prepare_no_noise).  Rows may have any
+        stride.  Inputs already in one of these forms on this device or in page-locked host memory are read by the
+        pack kernel in place: keep them unchanged until wait(ticket).  Anything else is converted by torch on the
+        caller's stream first.  Outputs as for submit().  Weights: drain() before updating the module."""
+        if self._iplan is None:
+            raise RuntimeError("submit_observations needs a pipeline built with stack= (the frame layout)")
+        t_host = time.perf_counter()
+        noisy = noises is not None
+        fraction = float(fraction) if noisy else 0.0
+        n, a, held = self.n, self.a, []
+        # every input and output checked, then converted, BEFORE the ticket takes a position
+        obs, ofmt, odtype, oshape, odense = self._obs_form(obs)
+        legal, lfmt, ldtype, lshape, ldense = self._legal_form(legal)
+        if noises is not None and _as_tensor(noises).numel() != n * a:
+            raise ValueError(f"noises must hold [{n}, {a}] values, got {tuple(_as_tensor(noises).shape)}")
+        in_place = [self._wave_output(x, dtype, shape) for x, dtype, shape in
+                    ((out_visits, torch.int32, (n, a)), (out_values, torch.float32, (n,)))]
+        orec = _lib.ObsTicket()
+        orec.obs, orec.ld_obs = self._source(obs, odtype, oshape, odense, held)
+        orec.legal, orec.ld_legal = self._source(legal, ldtype, lshape, ldense, held)
+        orec.noise = self._wave_input(noises, torch.float32, (n, a), held)
+        orec.obs_format, orec.legal_format = ofmt, lfmt
+        if self._waves.closes(noisy, fraction) or self._open_kind() == "hidden":
+            self._launch_wave()
+        return self._join("obs", noisy, fraction, _lib.WaveTicket(), orec, held, in_place, out_visits, out_values,
+                          t_host)
+
+    def _obs_form(self, x):
+        """(tensor, HZ_OBS_* format, dtype the kernel reads, shape, frames dense in the row) of a ticket's frames."""
+        n, S = self.n, self.stack
+        x = _as_tensor(x)
+        if x.dtype == torch.int32:
+            fmt, width, dtype = _lib.HZ_OBS_BITS, self.frame_words, torch.int32
+        elif x.dtype == torch.uint8:
+            fmt, width, dtype = _lib.HZ_OBS_U8, self.frame_dim, torch.uint8
+        else:
+            fmt, width, dtype = _lib.HZ_OBS_F32, self.frame_dim, torch.float32
+        if tuple(x.shape) not in ((n, S, width), (n, S * width)):
+            raise ValueError(f"obs must be [{n}, {S}, {width}] or [{n}, {S * width}] ({x.dtype}), got {tuple(x.shape)}")
+        return x, fmt, dtype, (n, S * width), x.stride(-1) == 1 and (x.dim() == 2 or x.stride(1) == width)
+
+    def _legal_form(self, x):
+        """(tensor, HZ_LEGAL_* format, dtype the kernel reads, shape, row dense) of a ticket's legal moves."""
+        n, a = self.n, self.a
+        x = _as_tensor(x)
+        if x.dim() == 1:
+            if x.shape[0] != n or x.dtype != torch.int32:
+                raise ValueError(f"a legal bit mask must be int32 [{n}], got {x.dtype} {tuple(x.shape)}")
+            return x, _lib.HZ_LEGAL_MASK, torch.int32, (n,), True      # one word per root at any row stride
+        if tuple(x.shape) != (n, a):
+            raise ValueError(f"legal must be [{n}, {a}] or an int32 bit mask [{n}], got {tuple(x.shape)}")
+        if x.dtype == torch.float32:
+            return x, _lib.HZ_LEGAL_F32, torch.float32, (n, a), x.stride(-1) == 1
+        return x, _lib.HZ_LEGAL_I32, torch.int32, (n, a), x.stride(-1) == 1
+
+    def _source(self, x, dtype, shape, dense, held):
+        """(address, row stride in elements) the pack kernel reads `x` at: in place when it has the kernel's type and
+        layout on this device or in page-locked host memory, else converted by torch on the caller's stream."""
+        if not (x.dtype == dtype and dense and (x.device == self.device or (x.device.type == "cpu" and x.is_pinned()))):
+            x = cytree.as_device(x, dtype, self.device, shape)      # slow path
+        held.append(x)
+        return x.data_ptr(), x.stride(0)
 
     def _readable_in_place(self, x, dtype, shape):
         return (isinstance(x, torch.Tensor) and x.dtype == dtype and tuple(x.shape) == shape and x.is_contiguous()
@@ -588,15 +703,30 @@ class SearchPipeline:
         table = (_lib.WaveTicket * count)(*s["table"])
         st = compute.cuda_stream
         with torch.cuda.stream(compute):
-            check(lib.hz_wave_pack(st, dev, table, count, self.wave, self.n, self.a,
-                                   s["hidden"].shape[1] * s["hidden"].element_size(),
-                                   ptr(s["noise"]) if w["noisy"] else None, ptr(s["reward"]), ptr(s["logits"]),
-                                   ptr(s["legal"]), ptr(s["hidden"])))
-            if w["noisy"]:
-                roots.prepare(w["fraction"], s["noise"], s["reward"], s["logits"], s["legal"])
+            if s["kind"] == "obs":
+                b = s["ibound"]
+                check(lib.hz_obs_pack(st, dev, (_lib.ObsTicket * count)(*s["obs_table"]), count, self.wave, self.n,
+                                      self.a, _lib.C.byref(self._layout), ptr(b.x), ptr(s["legal"]),
+                                      ptr(s["noise"]) if w["noisy"] else None))
+                recurrent = self.mcts._plan(self.model)
+                if self._iplan.refresh() | bool(recurrent is not None and recurrent.refresh()):
+                    # the weights were re-folded on this stream; the other slots' streams read them too
+                    compute.synchronize()
+                hidden, reward = self._iplan.run_bound(b, s["logits"]), self._zero_reward
             else:
-                roots.prepare_no_noise(s["reward"], s["logits"], s["legal"])
-            self.mcts.run_multi(roots, self.model, s["hidden"], gemm_sm_target=self.gemm_sm_target,
+                if s["hidden"] is None:
+                    feature, hdtype = self._hidden_shape
+                    s["hidden"] = torch.empty(self.wave * self.n, feature, dtype=hdtype, device=self.device)
+                check(lib.hz_wave_pack(st, dev, table, count, self.wave, self.n, self.a,
+                                       s["hidden"].shape[1] * s["hidden"].element_size(),
+                                       ptr(s["noise"]) if w["noisy"] else None, ptr(s["reward"]), ptr(s["logits"]),
+                                       ptr(s["legal"]), ptr(s["hidden"])))
+                hidden, reward = s["hidden"], s["reward"]
+            if w["noisy"]:
+                roots.prepare(w["fraction"], s["noise"], reward, s["logits"], s["legal"])
+            else:
+                roots.prepare_no_noise(reward, s["logits"], s["legal"])
+            self.mcts.run_multi(roots, self.model, hidden, gemm_sm_target=self.gemm_sm_target,
                                 stage_limit=self.stage_limit, executor=self.executor)
             check(lib.hz_trees_root_stats(roots.handle, st, ptr(s["visits"]), ptr(s["values"])))
             s["ev_done"].record(compute)

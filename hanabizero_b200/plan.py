@@ -479,3 +479,13 @@ class InitialPlan:
             check(self.lib.hz_support_decode(st, ptr(b.out[0]), b.out.element_size(), ptr(self.support), ptr(value), n,
                                              self.n_support, self.P3, self.net.support_delta))
         return value, b.out[1][:, :self.A].float(), b.state
+
+    @torch.no_grad()
+    def run_bound(self, b, logits):
+        """Runs the chain of `b` (an entry of bound() the caller keeps, its x already filled) on the current stream and
+        converts the policy logits into `logits` (float32 [n, A]) in place, so that a caller whose later kernels point
+        at `logits` (a search slot's prepare input, wave after wave) keeps one buffer.  Returns b.state, the hidden
+        states [n, F] in the plan's dtype."""
+        check(self.lib.hz_gemm_plan_run(b.handle, torch.cuda.current_stream(self.device).cuda_stream, 0, b.n_steps))
+        logits.copy_(b.out[1][:, :self.A])
+        return b.state

@@ -463,6 +463,49 @@ int hz_wave_pack(void* stream, int device, const hz_wave_ticket* tickets, int co
 int hz_wave_unpack(void* stream, int device, const hz_wave_ticket* tickets, int count, int slots, int n,
                    int num_actions, const int32_t* stats);
 
+/* Observation tickets (SearchPipeline.submit_observations): a wave whose tickets hand in stacked observations instead
+ * of the representation network's outputs.  hz_obs_pack fills, for ticket k, rows [k*n, (k+1)*n) of
+ *   x      [slots*n][stack * frame_stride] half (elem_bytes 2) or float (4), 16-byte aligned: the root inference's input
+ *          as hz_ring_gather writes it — frame j (oldest first) at column j * frame_stride, padding columns 0;
+ *   legal  int32 [slots*n][A], the mask hz_trees_prepare takes (int32 masks as given, the others as 0 / 1);
+ *   noise  float [slots*n][A], or NULL for a wave prepared without noise (a ticket's NULL noise gives zeros).
+ * The rows of slots count..slots-1 are padding roots: zero input and an all-zero legal mask, as in hz_wave_pack.
+ * Frame formats of a ticket's obs, row i at obs + i * ld_obs elements, frame j of the row at j * D (j * W for bits):
+ *   HZ_OBS_F32   float   [n][stack][D] values, converted to x's type
+ *   HZ_OBS_U8    uint8   [n][stack][D] values (0/1 bytes: HanabiVecEnv(obs_dtype=torch.uint8), the recorder's rows)
+ *   HZ_OBS_BITS  uint32  [n][stack][W] packed strings: the frame is bits [bit_offset, bit_offset + D), bit b in word
+ *                b / 32 at position b % 32 (hz_envs_step_observe_bits' order; bit_offset 0 = the global observation,
+ *                own_len = its local suffix)
+ * Legal formats, row i at legal + i * ld_legal elements: HZ_LEGAL_I32 int32 [n][A] and HZ_LEGAL_F32 float [n][A]
+ * (non-zero = legal), HZ_LEGAL_MASK one uint32 per root, bit a = action a legal (word 0 of the meta rows
+ * hz_envs_step_observe_bits / hz_envs_host_step write: ld_legal 4).  Pointers: device memory of `device` or
+ * page-locked host memory, which the kernel reads itself; 4-byte aligned except uint8 frames.  Sizes as hz_wave_pack,
+ * plus: stack 1..64, 1 <= D <= frame_stride, frame_stride a multiple of 16, stack * frame_stride <= 65536, and for bit
+ * frames W >= 1 with bit_offset + D <= 32 W.  Everything is checked before the launch (HZ_ERR_ARG).  One launch,
+ * asynchronous; the table and layout may be reused when the call returns, the sources must stay valid until the stream
+ * gets there.  Results go back through hz_wave_unpack with only out_visits / out_values set. */
+enum { HZ_OBS_F32 = 0, HZ_OBS_U8 = 1, HZ_OBS_BITS = 2 };
+enum { HZ_LEGAL_I32 = 0, HZ_LEGAL_F32 = 1, HZ_LEGAL_MASK = 2 };
+typedef struct hz_obs_ticket {
+  const void* obs;         /* frames, `obs_format` */
+  int64_t ld_obs;          /* row stride in elements of the format (floats, bytes, words) */
+  const void* legal;       /* legal moves, `legal_format` */
+  int64_t ld_legal;        /* row stride in elements (int32 / float / mask words) */
+  const float* noise;      /* [n][A] contiguous, or NULL (= zeros) */
+  int32_t obs_format;      /* HZ_OBS_* */
+  int32_t legal_format;    /* HZ_LEGAL_* */
+} hz_obs_ticket;
+typedef struct hz_obs_layout {
+  int32_t stack;           /* frames per root */
+  int32_t frame_dim;       /* D: values per frame */
+  int32_t frame_stride;    /* columns per frame in x */
+  int32_t elem_bytes;      /* x: 2 = half, 4 = float */
+  int32_t frame_words;     /* W: words per packed frame (HZ_OBS_BITS) */
+  int32_t bit_offset;      /* first bit of the frame in its packed string (HZ_OBS_BITS) */
+} hz_obs_layout;
+int hz_obs_pack(void* stream, int device, const hz_obs_ticket* tickets, int count, int slots, int n, int num_actions,
+                const hz_obs_layout* layout, void* x, int32_t* legal, float* noise);
+
 #ifdef __cplusplus
 }
 #endif
