@@ -71,6 +71,7 @@ SIGNATURES = {
     "hz_ring_refill": (_i, [_vp, _vp, _i, _vp, _i, _i, _i]),
     "hz_traj_begin": (_i, [_vp, _vp, _vp, _i64, _vp, _vp]),
     "hz_traj_append": (_i, [_vp, _vp, _vp, _vp, _i64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "hz_traj_record_u8": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _vp, _i64, _vp, _vp]),
     "hz_traj_pack": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
     "hz_visit_policy": (_i, [_vp, _vp, _vp, _i, _i, _vp, _vp]),
     "hz_envs_create": (_i, [C.POINTER(_vp), _i, _i, _i, _vp]),
@@ -82,6 +83,8 @@ SIGNATURES = {
     "hz_envs_step_observe": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp]),
     "hz_envs_observe_u8": (_i, [_vp, _vp, _vp, _i64, _vp, _i64, _vp]),
     "hz_envs_step_observe_u8": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp]),
+    "hz_envs_step_observe_u8_terminal": (_i, [_vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _vp, _i64, _vp, _vp, _i64,
+                                              _vp]),
     "hz_envs_step_observe_bits": (_i, [_vp, _vp, _vp, _vp, _i, _vp, _i64, _vp]),
     "hz_envs_host_step": (_i, [_vp, _vp, _vp, _i, _vp, _i64, _vp]),
     "hz_envs_host_wait": (_i, [_vp]),

@@ -507,9 +507,16 @@ struct EnvArgs {
   int32_t* policy_out;
   uint32_t* policy_ctr;
   unsigned long long policy_seed;
+  // terminal rows (hz_envs_step_observe_u8_terminal, the TERM instantiation only): the observation of a finished game's
+  // terminal state in the view of out_global8 / out_local8, and its legal mask, written before the re-deal
+  uint8_t* out_term8;
+  int64_t ld_term;
+  uint8_t* out_term_legal8;
 };
 
-template <int C, int R, int H, int MI, int ML, bool RESET, bool STEP, bool OBSERVE>
+// TERM: the recording variant of step + auto-reset + byte observe; a separate instantiation, so the others carry none
+// of its code
+template <int C, int R, int H, int MI, int ML, bool RESET, bool STEP, bool OBSERVE, bool TERM = false>
 __global__ void __launch_bounds__(kEnvWarps* HZ_WARP, 8) k_env(EnvView ev, EnvArgs a) {
   using L = ObsLayout<C, R, H, MI, ML>;
   __shared__ uint32_t s_state[kEnvWarps][kStateBytes / 4];
@@ -560,6 +567,21 @@ __global__ void __launch_bounds__(kEnvWarps* HZ_WARP, 8) k_env(EnvView ev, EnvAr
       done = is_terminal(st, g);
       dirty = true;
       if (done && a.auto_reset) {
+        if (TERM) {   // GameHistory.append takes the terminal observation (rl_env.py:426-434): encode it before the re-deal
+          uint32_t* words = s_obs[warp];
+          for (int i = lane; i < L::WORDS; i += HZ_WARP) words[i] = 0u;
+          __syncwarp();
+          obs_build<C, R, H, MI, ML>(st, (int8_t)st[O_CUR], words, lane);
+          __syncwarp();
+          if (a.out_term8) {
+            uint8_t* ot = a.out_term8 + (size_t)gi * a.ld_term;
+            if (a.out_global8) store_bits_u8(ot, words, 0, L::GLOBAL, lane);
+            else store_bits_u8(ot, words, L::OWN, L::GLOBAL - L::OWN, lane);
+          }
+          const unsigned term_legal = legal_mask(st, g, lane);   // no terminal check: non-zero here, as in the reference
+          if (a.out_term_legal8 && lane < g.A) a.out_term_legal8[(size_t)gi * g.A + lane] = (term_legal >> lane) & 1u;
+          __syncwarp();   // the OBSERVE block below clears these words again
+        }
         new_state(st, g, lane);
         while ((int8_t)st[O_CUR] == -1) deal_random<C * R>(st, g, mt, mti, win, scratch, lane, gi);
 #ifdef HZ_TRACE
@@ -703,15 +725,15 @@ struct hz_envs {
   EnvView view() const { return EnvView{state, mt, mti, err, N, g}; }
 };
 
-template <bool RESET, bool STEP, bool OBSERVE>
+template <bool RESET, bool STEP, bool OBSERVE, bool TERM = false>
 static int launch_env(hz_envs* e, cudaStream_t s, const EnvArgs& args) {
   EnvArgs a = args;
   if (OBSERVE) { a.policy_out = e->policy_out; a.policy_ctr = e->policy_ctr; a.policy_seed = e->policy_seed; }
   dim3 grid((e->N + kEnvWarps - 1) / kEnvWarps), block(kEnvWarps * HZ_WARP);
   if (e->preset == 0) {
-    k_env<5, 5, 5, 8, 3, RESET, STEP, OBSERVE><<<grid, block, 0, s>>>(e->view(), a);
+    k_env<5, 5, 5, 8, 3, RESET, STEP, OBSERVE, TERM><<<grid, block, 0, s>>>(e->view(), a);
   } else {
-    k_env<2, 5, 2, 3, 1, RESET, STEP, OBSERVE><<<grid, block, 0, s>>>(e->view(), a);
+    k_env<2, 5, 2, 3, 1, RESET, STEP, OBSERVE, TERM><<<grid, block, 0, s>>>(e->view(), a);
   }
   HZ_LAUNCH_CHECK("k_env");
   return HZ_OK;
@@ -869,6 +891,33 @@ int hz_envs_step_observe_u8(hz_envs* e, void* stream, const int32_t* actions, co
   a.out_global8 = out_global; a.ld_global = ld_global;
   a.out_local8 = out_local; a.ld_local = ld_local; a.out_legal8 = out_legal;
   return launch_env<false, true, true>(e, (cudaStream_t)stream, a);
+}
+
+int hz_envs_step_observe_u8_terminal(hz_envs* e, void* stream, const int32_t* actions, const uint8_t* active,
+                                     int32_t* out_reward, uint8_t* out_done, int32_t* out_score, uint8_t* out_global,
+                                     int64_t ld_global, uint8_t* out_local, int64_t ld_local, uint8_t* out_legal,
+                                     uint8_t* out_term, int64_t ld_term, uint8_t* out_term_legal) {
+  if (!e || !actions) { set_error("hz_envs_step_observe_u8_terminal: NULL argument"); return HZ_ERR_ARG; }
+  if (!e->started) { set_error("hz_envs_step_observe_u8_terminal: reset first"); return HZ_ERR_STATE; }
+  if (!out_global == !out_local) {
+    set_error("hz_envs_step_observe_u8_terminal: exactly one of out_global / out_local (the terminal rows' view)");
+    return HZ_ERR_ARG;
+  }
+  if (int rc = check_obs_args(e, out_global, ld_global, out_local, ld_local)) return rc;
+  const int width = out_global ? e->g.own_len + e->g.enc_len + P : e->g.enc_len + P;
+  if (out_term && ld_term < width) {
+    set_error("hz_envs_step_observe_u8_terminal: terminal row stride %lld smaller than the observation (%d)",
+              (long long)ld_term, width);
+    return HZ_ERR_ARG;
+  }
+  DeviceGuard dg(e->device);
+  EnvArgs a{};
+  a.actions = actions; a.active = active; a.auto_reset = 1;
+  a.out_reward = out_reward; a.out_done = out_done; a.out_score = out_score;
+  a.out_global8 = out_global; a.ld_global = ld_global;
+  a.out_local8 = out_local; a.ld_local = ld_local; a.out_legal8 = out_legal;
+  a.out_term8 = out_term; a.ld_term = ld_term; a.out_term_legal8 = out_term_legal;
+  return launch_env<false, true, true, true>(e, (cudaStream_t)stream, a);
 }
 
 int hz_envs_step_observe_bits(hz_envs* e, void* stream, const int32_t* actions, const uint8_t* active, int auto_reset,

@@ -7,6 +7,9 @@
 //       and handed to the host episode by episode in the replay layout (game.py:136-140, `save_file`).
 //       `banks` >= 2 banks per game, used round-robin: finished episodes wait in their banks for
 //       hz_traj_pack while the next episode of that game is recorded into the next free one.
+//   hz_traj_record_u8
+//       hz_traj_append + hz_traj_begin(mask = done) as one launch over byte rows: the recording self-play
+//       engine on the frame ring (the env kernel hands over the terminal rows of finished games apart).
 //   hz_visit_policy
 //       visit counts -> policy targets with the out-of-trajectory mask of the reanalyze caller
 //       (/root/reference/core/reanalyze_worker.py:352-367; store_search_stats, game.py:194-197).
@@ -87,6 +90,68 @@ __global__ void __launch_bounds__(kTrajWarps* HZ_WARP)
       v.bank[i] = (uint8_t)((b + 1) % v.banks);
     }
   }
+}
+
+// byte 0/1 row -> bytes, `copies` consecutive destination rows (any non-zero byte is recorded as 1, as put_obs does)
+__device__ __forceinline__ void put_obs_u8(uint8_t* dst, const uint8_t* src, int dim, int copies, int lane) {
+  for (int j = lane; j < dim; j += HZ_WARP) {
+    const uint8_t b = src[j] != 0 ? 1 : 0;
+    for (int c = 0; c < copies; ++c) dst[(size_t)c * dim + j] = b;
+  }
+}
+
+// k_traj_append followed by k_traj_begin(mask = done) in one launch, from byte rows: a finished game appends its
+// terminal row (term_*) and begins the next episode from next_*; every other game appends next_*
+__global__ void __launch_bounds__(kTrajWarps* HZ_WARP)
+    k_traj_record_u8(hz_traj_view v, const int32_t* __restrict__ actions, const int32_t* __restrict__ reward,
+                     const int32_t* __restrict__ visits, const float* __restrict__ root_values,
+                     const uint8_t* __restrict__ done, const uint8_t* __restrict__ next_obs, int64_t ld_next,
+                     const uint8_t* __restrict__ next_legal, const uint8_t* __restrict__ term_obs, int64_t ld_term,
+                     const uint8_t* __restrict__ term_legal, const uint8_t* __restrict__ active) {
+  const int lane = threadIdx.x & 31;
+  const int i = blockIdx.x * kTrajWarps + (threadIdx.x >> 5);
+  if (i >= v.num) return;
+  const TrajDims d = traj_dims(v);
+  const bool fin = done[i] != 0;
+  int b = v.bank[i];
+  if (!active || active[i]) {
+    const size_t gb = (size_t)v.banks * i + b;
+    const int t = v.len[gb];
+    if (t >= v.max_len || v.finished[gb]) {
+      if (lane == 0) atomicCAS(v.overflow, 0, i + 1);
+    } else {
+      const uint8_t* obs = fin ? term_obs + (size_t)i * ld_term : next_obs + (size_t)i * ld_next;
+      const uint8_t* legal = (fin ? term_legal : next_legal) + (size_t)i * v.actions;
+      if (lane < v.actions) {
+        v.visits[(gb * v.max_len + t) * v.actions + lane] = visits[(size_t)i * v.actions + lane];
+        v.legal[(gb * d.legal_rows + t + 1) * v.actions + lane] = legal[lane] != 0;
+      }
+      put_obs_u8(v.obs + (gb * d.obs_rows + v.stack + t) * v.obs_dim, obs, v.obs_dim, 1, lane);
+      __syncwarp();   // every lane has read len / bank / finished before lane 0 updates them
+      if (lane == 0) {
+        v.action[gb * v.max_len + t] = actions[i];
+        v.reward[gb * v.max_len + t] = reward[i];
+        v.root_value[gb * v.max_len + t] = root_values[i];
+        v.len[gb] = t + 1;
+        if (fin) {
+          v.finished[gb] = 1;
+          v.bank[i] = (uint8_t)((b + 1) % v.banks);
+        }
+      }
+      if (fin) b = (b + 1) % v.banks;
+    }
+  }
+  if (!fin) return;
+  // begin: the bank just moved to is one this launch has not written (banks >= 2), so every lane may read its flag
+  const size_t gb = (size_t)v.banks * i + b;
+  if (v.finished[gb]) {
+    if (lane == 0) atomicCAS(v.overflow, 0, i + 1);
+    return;
+  }
+  put_obs_u8(v.obs + gb * d.obs_rows * v.obs_dim, next_obs + (size_t)i * ld_next, v.obs_dim, v.stack, lane);
+  if (lane < v.actions) v.legal[gb * d.legal_rows * v.actions + lane] = next_legal[(size_t)i * v.actions + lane] != 0;
+  __syncwarp();   // every lane has read len before lane 0 rewrites it (append overflow with the bank unchanged)
+  if (lane == 0) v.len[gb] = 0;
 }
 
 // one CTA per finished episode: copy its rows into the packed staging buffers and free the bank
@@ -182,6 +247,22 @@ int hz_traj_append(void* stream, const hz_traj_view* v, const int32_t* actions, 
   k_traj_append<<<(v->num + kTrajWarps - 1) / kTrajWarps, kTrajWarps * HZ_WARP, 0, (cudaStream_t)stream>>>(
       *v, actions, obs, ld_obs, legal, reward, visits, root_values, done, active);
   HZ_LAUNCH_CHECK("k_traj_append");
+  return HZ_OK;
+}
+
+int hz_traj_record_u8(void* stream, const hz_traj_view* v, const int32_t* actions, const int32_t* reward,
+                      const int32_t* visits, const float* root_values, const uint8_t* done, const uint8_t* next_obs,
+                      int64_t ld_next, const uint8_t* next_legal, const uint8_t* term_obs, int64_t ld_term,
+                      const uint8_t* term_legal, const uint8_t* active) {
+  if (int rc = check_view(v, "hz_traj_record_u8")) return rc;
+  if (!actions || !reward || !visits || !root_values || !done || !next_obs || !next_legal || !term_obs || !term_legal ||
+      ld_next < v->obs_dim || ld_term < v->obs_dim) {
+    set_error("hz_traj_record_u8: NULL argument or row stride smaller than the observation");
+    return HZ_ERR_ARG;
+  }
+  k_traj_record_u8<<<(v->num + kTrajWarps - 1) / kTrajWarps, kTrajWarps * HZ_WARP, 0, (cudaStream_t)stream>>>(
+      *v, actions, reward, visits, root_values, done, next_obs, ld_next, next_legal, term_obs, ld_term, term_legal, active);
+  HZ_LAUNCH_CHECK("k_traj_record_u8");
   return HZ_OK;
 }
 

@@ -106,12 +106,17 @@ class HanabiVecEnv:
         raise TypeError(f"observation outputs must be all float32 or all uint8, got {sorted(map(str, kinds))}")
 
     def step_all(self, actions, active=None, auto_reset=False, observe=True, out_global=None,
-                 out_local=None, out_legal=None, want_local=True, want_global=True):
+                 out_local=None, out_legal=None, want_local=True, want_global=True, out_terminal=None,
+                 out_terminal_legal=None):
         """HanabiEnv.step for every (active) game in one launch.  actions: int32 CUDA tensor [N]
         (anything else is converted).  Returns (global_obs, local_obs, legal, reward, done, score).
         With auto_reset a finished game is re-dealt inside the same launch and the returned
         observation is the first one of its next episode (reward/done/score describe the finished
-        step).  Illegal actions leave the game untouched; call check() to surface them."""
+        step).  Illegal actions leave the game untouched; call check() to surface them.
+        out_terminal / out_terminal_legal (uint8 CUDA [N, >= dim] / [N, A]; auto_reset=True, uint8 outputs and
+        exactly one view only): a finished game's terminal observation, in that view, and its legal mask are written
+        there before the re-deal (hz_envs_step_observe_u8_terminal); rows of the other games are left as they were."""
+        terminal = out_terminal is not None or out_terminal_legal is not None
         if not (isinstance(actions, torch.Tensor) and actions.dtype == torch.int32 and actions.is_cuda):
             actions = torch.as_tensor(np.asarray(actions, np.int32) if not isinstance(actions, torch.Tensor)
                                       else actions, dtype=torch.int32).to(self.device)
@@ -119,6 +124,8 @@ class HanabiVecEnv:
         if actions.numel() != self.num_games:
             raise ValueError(f"expected {self.num_games} actions, got {actions.numel()}")
         act = None if active is None else active.to(self.device, torch.uint8).contiguous()
+        if terminal and not (auto_reset and observe):
+            raise ValueError("terminal rows need auto_reset=True and observe=True")
         if not observe:
             check(self._lib.hz_envs_step(self._h, self._stream(), ptr(actions), ptr(act),
                                          ptr(self.reward), ptr(self.done), ptr(self.score)))
@@ -126,6 +133,22 @@ class HanabiVecEnv:
         g = (self.global_obs if out_global is None else out_global) if want_global else None
         l = (self.local_obs if out_local is None else out_local) if want_local else None
         a = self.legal if out_legal is None else out_legal
+        if terminal:
+            if not self._all_u8(g, l, a, out_terminal, out_terminal_legal):
+                raise TypeError("terminal rows need uint8 observation, legal and terminal outputs")
+            if (g is None) == (l is None):
+                raise ValueError("terminal rows need exactly one observation view (want_global or want_local)")
+            if out_terminal_legal is not None and (out_terminal_legal.shape != (self.num_games, self.num_actions)
+                                                   or not out_terminal_legal.is_contiguous()):
+                raise ValueError("out_terminal_legal must be a contiguous [num_games, num_actions] tensor")
+            if out_terminal is not None and (out_terminal.dim() != 2 or out_terminal.shape[0] != self.num_games
+                                             or out_terminal.stride(1) != 1):
+                raise ValueError("out_terminal must be [num_games, >= dim] with unit column stride")
+            check(self._lib.hz_envs_step_observe_u8_terminal(
+                self._h, self._stream(), ptr(actions), ptr(act), ptr(self.reward), ptr(self.done), ptr(self.score),
+                ptr(g), self._ld(g), ptr(l), self._ld(l), ptr(a), ptr(out_terminal), self._ld(out_terminal),
+                ptr(out_terminal_legal)))
+            return g, l, a, self.reward, self.done, self.score
         fn = self._lib.hz_envs_step_observe_u8 if self._all_u8(g, l, a) else self._lib.hz_envs_step_observe
         check(fn(self._h, self._stream(), ptr(actions), ptr(act), 1 if auto_reset else 0, ptr(self.reward),
                  ptr(self.done), ptr(self.score), ptr(g), self._ld(g), ptr(l), self._ld(l), ptr(a)))

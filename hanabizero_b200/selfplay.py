@@ -88,9 +88,17 @@ class SelfPlayEngine:
     def __init__(self, num_games, hanabi_name, model, config, seeds=None, mdp="global", stack=4, device=None,
                  record=False, max_episode_len=128, record_banks=2, noise_seed=0, game_offset=0):
         """record: keep every game's trajectory on the device (hanabizero_b200.trajectory, SURVEY §8f N3);
-        finished episodes are fetched with `self.recorder.flush()`.  noise_seed / game_offset key the root
+        finished episodes are fetched with `self.recorder.flush()`.  record=True records on the float frame stack with
+        the module's root inference; record="ring" records on the same fast path as an unrecorded engine (byte frame
+        ring, InitialPlan root inference, auto-reset in the env launch; the model must have `initial_plan`) with one
+        more launch per move.  Both play the moves an unrecorded engine plays.  noise_seed / game_offset key the root
         exploration noise (dirichlet_noise: move m of game i draws stream (noise_seed, m, game_offset + i)), so the
         noise of any move can be regenerated on the host with dirichlet_noise_host."""
+        ring = isinstance(record, str)
+        if ring and record != "ring":
+            raise ValueError(f"record must be False, True or 'ring', got {record!r}")
+        if ring and not hasattr(model, "initial_plan"):
+            raise ValueError("record='ring' needs a model with initial_plan (the byte frame ring's root inference)")
         self.env = HanabiVecEnv(num_games, hanabi_name, seeds, device=device)
         self.dev, self.n, self.stack, self.mdp = self.env.device, num_games, int(stack), mdp
         self.model, self.config, self.mcts = model, config, MCTS(config)
@@ -100,16 +108,19 @@ class SelfPlayEngine:
         self.lib = _lib.load()
         self._obs = torch.zeros(num_games, self.obs_dim, device=self.dev)
         self._all_done = torch.ones(num_games, dtype=torch.uint8, device=self.dev)
-        # fast path (no recording): the frame stack is a ring of 0/1 bytes the env kernel writes into, and the root
-        # inference runs as a folded GEMM plan (hanabizero_b200/plan.py InitialPlan) instead of ~70 module kernels
+        # fast path (record=False or "ring"): the frame stack is a ring of 0/1 bytes the env kernel writes into, and the
+        # root inference runs as a folded GEMM plan (hanabizero_b200/plan.py InitialPlan) instead of ~70 module kernels
         self.iplan = None
-        if not record and hasattr(model, "initial_plan"):
+        if (ring or not record) and hasattr(model, "initial_plan"):
             amp = getattr(config, "amp_type", "none") == "torch_amp"
             self.iplan = model.initial_plan(torch.float16 if amp else torch.float32, self.obs_dim, self.stack)
             self.Dp = self.iplan.frame_stride
             self.ring = torch.zeros(num_games, self.stack, self.Dp, dtype=torch.uint8, device=self.dev)
             self.legal8 = torch.zeros(num_games, self.env.num_actions, dtype=torch.uint8, device=self.dev)
             self.head = 0          # ring slot holding the OLDEST frame (the next one to be overwritten)
+            if ring:               # terminal rows of the games a move finishes (hz_envs_step_observe_u8_terminal)
+                self.term = torch.zeros(num_games, self.Dp, dtype=torch.uint8, device=self.dev)
+                self.term_legal = torch.zeros(num_games, self.env.num_actions, dtype=torch.uint8, device=self.dev)
         self.alpha = float(getattr(config, "root_dirichlet_alpha", 0.3))
         self.noise_seed, self.game_offset, self.moves = int(noise_seed), int(game_offset), 0
         self.recorder = None
@@ -155,6 +166,8 @@ class SelfPlayEngine:
             check(self.lib.hz_ring_refill(self._stream(), ptr(self.ring), 0, None, self.n, self.stack, self.Dp))
             self.head = 0
             self.legal.copy_(self.legal8)
+            if self.recorder is not None:
+                self.recorder.begin(self.ring[:, 0, :self.obs_dim].float(), self.legal)
             return self.frames_tensor(), self.legal
         self._observe()
         self._push(self._all_done)
@@ -208,9 +221,18 @@ class SelfPlayEngine:
             # the new observation replaces the oldest frame in place; finished games get their stack refilled
             slot = self.head
             g, l = self._ring_slot(slot)
-            _, _, _, reward, done, score = self.env.step_all(actions, auto_reset=True, out_global=g, out_local=l,
-                                                             out_legal=self.legal8, want_global=g is not None,
-                                                             want_local=l is not None)
+            if self.recorder is None:
+                _, _, _, reward, done, score = self.env.step_all(actions, auto_reset=True, out_global=g, out_local=l,
+                                                                 out_legal=self.legal8, want_global=g is not None,
+                                                                 want_local=l is not None)
+            else:
+                # record="ring": the step also writes finished games' terminal rows (GameHistory.append, game.py:143)
+                # before their re-deal, and one launch appends the move and begins the next episodes from the slot
+                _, _, _, reward, done, score = self.env.step_all(
+                    actions, auto_reset=True, out_global=g, out_local=l, out_legal=self.legal8, want_global=g is not None,
+                    want_local=l is not None, out_terminal=self.term[:, :self.obs_dim], out_terminal_legal=self.term_legal)
+                self.recorder.record_u8(actions, reward, visits, values, done, self.ring[:, slot], self.legal8, self.term,
+                                        self.term_legal)
             check(self.lib.hz_ring_refill(self._stream(), ptr(self.ring), slot, ptr(done), n, self.stack, self.Dp))
             self.head = (slot + 1) % self.stack
             self.legal.copy_(self.legal8)
@@ -279,6 +301,22 @@ class SelfPlayPool:
     def synchronize(self):
         for s in self.streams:
             s.synchronize()
+
+    def flush(self):
+        """The finished episodes of every recording engine: one list per engine (TrajectoryRecorder.flush; [] for an
+        engine that does not record).  Each engine's flush runs on that engine's stream, after its appends."""
+        out = []
+        for eng, s in zip(self.engines, self.streams):
+            with torch.cuda.stream(s):
+                out.append([] if eng.recorder is None else eng.recorder.flush())
+        return out
+
+    def check(self):
+        """TrajectoryRecorder.check of every recording engine, on the engine's stream (synchronises it)."""
+        for eng, s in zip(self.engines, self.streams):
+            if eng.recorder is not None:
+                with torch.cuda.stream(s):
+                    eng.recorder.check()
 
 
 @torch.no_grad()

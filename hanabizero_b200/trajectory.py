@@ -70,6 +70,22 @@ class TrajectoryRecorder:
         check(self._lib.hz_traj_append(self._stream(), self._ref, ptr(actions), ptr(obs), obs.stride(0), ptr(legal),
                                        ptr(reward), ptr(visits), ptr(root_values), ptr(done), ptr(active)))
 
+    def record_u8(self, actions, reward, visits, root_values, done, next_obs, next_legal, term_obs, term_legal,
+                  active=None):
+        """append + begin(mask=done) for one move of every game in one launch (hz_traj_record_u8), from uint8 rows:
+        a finished game appends term_obs / term_legal (its terminal rows) and begins its next episode from next_obs /
+        next_legal; the others append next_obs / next_legal.  Observation rows [N, >= obs_dim] (row stride free),
+        legal rows [N, A]; CUDA."""
+        for t in (next_obs, next_legal, term_obs, term_legal):
+            if t.dtype != torch.uint8 or not t.is_cuda or t.stride(-1) != 1:
+                raise TypeError("record_u8 takes uint8 CUDA rows with unit column stride")
+        for t in (next_legal, term_legal):
+            if t.stride(0) != self.actions:
+                raise ValueError("legal rows must be [N, num_actions] contiguous")
+        check(self._lib.hz_traj_record_u8(self._stream(), self._ref, ptr(actions), ptr(reward), ptr(visits),
+                                          ptr(root_values), ptr(done), ptr(next_obs), next_obs.stride(0), ptr(next_legal),
+                                          ptr(term_obs), term_obs.stride(0), ptr(term_legal), ptr(active)))
+
     def check(self):
         """Synchronises; raises if a game ran out of room since the last check."""
         bad = int(self.overflow.item())

@@ -219,6 +219,17 @@ int hz_envs_step_observe_u8(hz_envs* e, void* stream, const int32_t* actions, co
                             int auto_reset, int32_t* out_reward, uint8_t* out_done, int32_t* out_score,
                             uint8_t* out_global, int64_t ld_global, uint8_t* out_local, int64_t ld_local,
                             uint8_t* out_legal);
+/* hz_envs_step_observe_u8 with auto-reset, for a caller that records trajectories: a finished game's TERMINAL
+ * observation (what auto_reset = 0 would have written, the row GameHistory.append takes, rl_env.py:426-434) goes to
+ * out_term (uint8[N][ld_term]) and its legal mask to out_term_legal (uint8[N][actions]; non-zero at terminal states:
+ * the reference has no terminal check), then the game is re-dealt and the first observation of its next episode goes
+ * to the usual output row.  Rows of games that did not finish are left as they were.  Exactly one of out_global /
+ * out_local is given, and the terminal rows are in that view (ld_term >= its width); out_term / out_term_legal may be
+ * NULL like the other outputs. */
+int hz_envs_step_observe_u8_terminal(hz_envs* e, void* stream, const int32_t* actions, const uint8_t* active,
+                                     int32_t* out_reward, uint8_t* out_done, int32_t* out_score, uint8_t* out_global,
+                                     int64_t ld_global, uint8_t* out_local, int64_t ld_local, uint8_t* out_legal,
+                                     uint8_t* out_term, int64_t ld_term, uint8_t* out_term_legal);
 
 /* The host-facing form of the same launch: ONE bit-packed row of uint32 words per game (dev, row stride ld_words >=
  * W + 4 with W = ceil(global_dim / 32): 25 for Hanabi-Full, 7 for Hanabi-Small):
@@ -345,6 +356,16 @@ int hz_traj_begin(void* stream, const hz_traj_view* v, const float* obs, int64_t
 int hz_traj_append(void* stream, const hz_traj_view* v, const int32_t* actions, const float* obs, int64_t ld_obs,
                    const float* legal, const int32_t* reward, const int32_t* visits, const float* root_values,
                    const uint8_t* done, const uint8_t* active);
+/* One launch per move for the recording engine on the byte frame ring: per game exactly hz_traj_append followed by
+ * hz_traj_begin(mask = done), from uint8 rows (non-zero = 1).  The appended observation and legal row are term_obs /
+ * term_legal where done[i] != 0 (hz_envs_step_observe_u8_terminal's terminal rows) and next_obs / next_legal
+ * elsewhere; a finished game then begins its next bank with `stack` copies of next_obs and legal row 0 = next_legal.
+ * Row strides ld_next / ld_term in bytes (>= obs_dim), legal rows [N][actions].  done is required; active as in
+ * hz_traj_append (the begin of a finished game does not look at it, as hz_traj_begin does not).  All pointers dev. */
+int hz_traj_record_u8(void* stream, const hz_traj_view* v, const int32_t* actions, const int32_t* reward,
+                      const int32_t* visits, const float* root_values, const uint8_t* done, const uint8_t* next_obs,
+                      int64_t ld_next, const uint8_t* next_legal, const uint8_t* term_obs, int64_t ld_term,
+                      const uint8_t* term_legal, const uint8_t* active);
 /* Hand over finished episodes: episode e = (ep_game[e], ep_bank[e]) (dev int32) with T_e moves is copied to
  * rows [step_off[e], step_off[e] + T_e) of out_action/out_reward/out_root/out_visits, to rows
  * [step_off[e] + e*stack, +stack + T_e) of out_obs and [step_off[e] + e, +T_e + 1) of out_legal (dev
