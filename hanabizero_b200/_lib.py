@@ -95,6 +95,8 @@ SIGNATURES = {
     "hz_wave_pack": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i, _vp, _vp, _vp, _vp, _vp]),
     "hz_wave_unpack": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp]),
     "hz_obs_pack": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
+    "hz_obs_pack_windows": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _i, _vp, _vp, _vp]),
+    "hz_wave_policy": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp]),
 }
 
 
@@ -137,6 +139,11 @@ class WaveTicket(C.Structure):
     """struct hz_wave_ticket (include/hzb200.h)."""
     _fields_ = [("noise", _vp), ("reward", _vp), ("logits", _vp), ("legal", _vp), ("hidden", _vp),
                 ("out_visits", _vp), ("out_values", _vp)]
+
+
+class PolicyTicket(C.Structure):
+    """struct hz_policy_ticket (include/hzb200.h)."""
+    _fields_ = [("mask", _vp), ("out", _vp)]
 
 
 HZ_OBS_F32, HZ_OBS_U8, HZ_OBS_BITS = 0, 1, 2

@@ -3,6 +3,10 @@
 //   hz_obs_pack  every ticket's frames -> rows [k*n, (k+1)*n) of InitialPlan's input x (half or float, frame j at
 //                column j * frame_stride, padding columns 0), its legal moves -> the int32 legal staging, its noise ->
 //                the noise staging; the rows of unused slots zero (padding roots, as in hz_wave_pack)
+//   hz_obs_pack_windows  the same with every obs row a window of stack + positions - 1 consecutive frames: root
+//                i * positions + p takes window frames p .. p + stack - 1 (the reanalyze batch, whose consecutive
+//                positions share frames, is handed in as one window per sample instead of one stack per position;
+//                each root still reads its own stack, so a shared frame is read once per stack that holds it)
 // One launch per wave.  The ticket table travels by value in the kernel parameters, as in hz_wave.cu.  Sources are
 // device memory or page-locked host memory, read by the kernel itself under unified addressing: for host sources
 // the launch is spread over enough CTAs to keep many reads in flight over the host link.
@@ -95,11 +99,12 @@ __device__ __forceinline__ void store_chunk(float* dst, const float* v) {
 
 // grid (blocks per slot, slots): blockIdx.y = slot; slots >= count are padding.  Items of a slot: n * chunks_per_row
 // 16-column chunks of x (row-major, so neighbouring threads read neighbouring source bytes), then one per row for its
-// legal mask and noise.
-template <typename OutT>
+// legal mask and noise.  WIN: root r reads obs row r / positions from frame r % positions on (a compile-time variant,
+// so the stack form keeps its own instructions and registers).
+template <typename OutT, bool WIN>
 __global__ void __launch_bounds__(kObsThreads) k_obs_pack(ObsTable tab, int count, int n, int num_actions, ObsDims d,
-                                                          OutT* __restrict__ x, int32_t* __restrict__ legal,
-                                                          float* __restrict__ noise) {
+                                                          int positions, OutT* __restrict__ x,
+                                                          int32_t* __restrict__ legal, float* __restrict__ noise) {
   const int k = blockIdx.y;
   const bool real = k < count;
   // fields read one by one from the parameter space (taking the entry's address would copy the table to local memory)
@@ -116,13 +121,19 @@ __global__ void __launch_bounds__(kObsThreads) k_obs_pack(ObsTable tab, int coun
       const int j = rem / d.chunks_per_frame;
       const int c0 = (rem - j * d.chunks_per_frame) * kObsChunk;
       const int valid = min(kObsChunk, d.frame_dim - c0);    // <= 0 for a chunk of padding columns only
+      int64_t row = r;      // obs row and frame of the source
+      int f = j;
+      if (WIN) {
+        row = r / positions;
+        f = j + (int)(r - row * positions);
+      }
       float v[kObsChunk];
       if (fmt == HZ_OBS_F32) {
-        load_f32((const float*)obs + r * ld_obs + (int64_t)j * d.frame_dim + c0, valid, v);
+        load_f32((const float*)obs + row * ld_obs + (int64_t)f * d.frame_dim + c0, valid, v);
       } else if (fmt == HZ_OBS_U8) {
-        load_u8((const uint8_t*)obs + r * ld_obs + (int64_t)j * d.frame_dim + c0, valid, v);
+        load_u8((const uint8_t*)obs + row * ld_obs + (int64_t)f * d.frame_dim + c0, valid, v);
       } else if (fmt == HZ_OBS_BITS) {
-        load_bits((const uint32_t*)obs + r * ld_obs + (int64_t)j * d.frame_words, d.bit_offset + c0, valid, v);
+        load_bits((const uint32_t*)obs + row * ld_obs + (int64_t)f * d.frame_words, d.bit_offset + c0, valid, v);
       } else {
 #pragma unroll
         for (int c = 0; c < kObsChunk; ++c) v[c] = 0.f;
@@ -155,16 +166,10 @@ __global__ void __launch_bounds__(kObsThreads) k_obs_pack(ObsTable tab, int coun
   }
 }
 
-}  // namespace hz
-
-using namespace hz;
-
-extern "C" {
-#pragma GCC visibility push(default)
-
-int hz_obs_pack(void* stream, int device, const hz_obs_ticket* tickets, int count, int slots, int n, int num_actions,
-                const hz_obs_layout* layout, void* x, int32_t* legal, float* noise) {
-  const char* fn = "hz_obs_pack";
+// Argument checks and the launch of both entry points; positions == 1 without windows is hz_obs_pack.
+static int obs_pack(const char* fn, bool windows, void* stream, int device, const hz_obs_ticket* tickets, int count,
+                    int slots, int n, int num_actions, const hz_obs_layout* layout, int positions, void* x,
+                    int32_t* legal, float* noise) {
   if (!tickets) { set_error("%s: NULL ticket table", fn); return HZ_ERR_ARG; }
   if (!layout) { set_error("%s: NULL layout", fn); return HZ_ERR_ARG; }
   if (slots < 1 || slots > kObsMaxSlots) { set_error("%s: slots = %d, must be 1..%d", fn, slots, kObsMaxSlots); return HZ_ERR_ARG; }
@@ -173,6 +178,8 @@ int hz_obs_pack(void* stream, int device, const hz_obs_ticket* tickets, int coun
     set_error("%s: n = %d, must be >= 1 with slots * n <= %lld", fn, n, (long long)kObsMaxRows);
     return HZ_ERR_ARG;
   }
+  if (positions < 1 || positions > n) { set_error("%s: positions = %d, must be 1..n (%d)", fn, positions, n); return HZ_ERR_ARG; }
+  if (n % positions) { set_error("%s: n = %d is not a multiple of positions = %d", fn, n, positions); return HZ_ERR_ARG; }
   if (num_actions < 1 || num_actions > 32) { set_error("%s: num_actions = %d, must be 1..32", fn, num_actions); return HZ_ERR_ARG; }
   const hz_obs_layout L = *layout;
   if (L.stack < 1 || L.stack > kObsMaxStack) { set_error("%s: stack = %d, must be 1..%d", fn, L.stack, kObsMaxStack); return HZ_ERR_ARG; }
@@ -186,6 +193,7 @@ int hz_obs_pack(void* stream, int device, const hz_obs_ticket* tickets, int coun
   }
   if (L.elem_bytes != 2 && L.elem_bytes != 4) { set_error("%s: elem_bytes = %d, must be 2 or 4", fn, L.elem_bytes); return HZ_ERR_ARG; }
   if (!x || !legal) { set_error("%s: NULL staging buffer", fn); return HZ_ERR_ARG; }
+  const int64_t frames = (int64_t)L.stack + positions - 1;     // per obs row: a stack, or a window
   for (int k = 0; k < count; ++k) {
     const hz_obs_ticket& t = tickets[k];
     if (!t.obs || !t.legal) { set_error("%s: ticket %d has a NULL input", fn, k); return HZ_ERR_ARG; }
@@ -200,9 +208,10 @@ int hz_obs_pack(void* stream, int device, const hz_obs_ticket* tickets, int coun
       set_error("%s: ticket %d: obs_format = %d is not a HZ_OBS_* code", fn, k, t.obs_format);
       return HZ_ERR_ARG;
     }
-    const int64_t row = (int64_t)L.stack * (t.obs_format == HZ_OBS_BITS ? L.frame_words : L.frame_dim);
+    const int64_t row = frames * (t.obs_format == HZ_OBS_BITS ? L.frame_words : L.frame_dim);
     if (t.ld_obs < row) {
-      set_error("%s: ticket %d: ld_obs = %lld, must be >= the %lld elements of a row", fn, k, (long long)t.ld_obs, (long long)row);
+      set_error("%s: ticket %d: ld_obs = %lld, must be >= the %lld elements of a %s", fn, k, (long long)t.ld_obs,
+                (long long)row, windows ? "window" : "row");
       return HZ_ERR_ARG;
     }
     if (t.legal_format != HZ_LEGAL_I32 && t.legal_format != HZ_LEGAL_F32 && t.legal_format != HZ_LEGAL_MASK) {
@@ -236,13 +245,42 @@ int hz_obs_pack(void* stream, int device, const hz_obs_ticket* tickets, int coun
   const int64_t per_block = (int64_t)kObsThreads * kObsItemsPerThread;
   const int blocks = (int)std::min<int64_t>((items + per_block - 1) / per_block, kObsMaxBlocksPerSlot);
   const dim3 grid(blocks, slots);
-  if (L.elem_bytes == 2) {
-    k_obs_pack<__half><<<grid, kObsThreads, 0, (cudaStream_t)stream>>>(tab, count, n, num_actions, d, (__half*)x, legal, noise);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (windows) {
+    if (L.elem_bytes == 2) {
+      k_obs_pack<__half, true><<<grid, kObsThreads, 0, st>>>(tab, count, n, num_actions, d, positions, (__half*)x, legal, noise);
+    } else {
+      k_obs_pack<float, true><<<grid, kObsThreads, 0, st>>>(tab, count, n, num_actions, d, positions, (float*)x, legal, noise);
+    }
+    HZ_LAUNCH_CHECK("k_obs_pack<windows>");
   } else {
-    k_obs_pack<float><<<grid, kObsThreads, 0, (cudaStream_t)stream>>>(tab, count, n, num_actions, d, (float*)x, legal, noise);
+    if (L.elem_bytes == 2) {
+      k_obs_pack<__half, false><<<grid, kObsThreads, 0, st>>>(tab, count, n, num_actions, d, 1, (__half*)x, legal, noise);
+    } else {
+      k_obs_pack<float, false><<<grid, kObsThreads, 0, st>>>(tab, count, n, num_actions, d, 1, (float*)x, legal, noise);
+    }
+    HZ_LAUNCH_CHECK("k_obs_pack");
   }
-  HZ_LAUNCH_CHECK("k_obs_pack");
   return HZ_OK;
+}
+
+}  // namespace hz
+
+using namespace hz;
+
+extern "C" {
+#pragma GCC visibility push(default)
+
+int hz_obs_pack(void* stream, int device, const hz_obs_ticket* tickets, int count, int slots, int n, int num_actions,
+                const hz_obs_layout* layout, void* x, int32_t* legal, float* noise) {
+  return obs_pack("hz_obs_pack", false, stream, device, tickets, count, slots, n, num_actions, layout, 1, x, legal, noise);
+}
+
+int hz_obs_pack_windows(void* stream, int device, const hz_obs_ticket* tickets, int count, int slots, int n,
+                        int num_actions, const hz_obs_layout* layout, int positions, void* x, int32_t* legal,
+                        float* noise) {
+  return obs_pack("hz_obs_pack_windows", true, stream, device, tickets, count, slots, n, num_actions, layout, positions,
+                  x, legal, noise);
 }
 
 #pragma GCC visibility pop

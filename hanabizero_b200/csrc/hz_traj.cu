@@ -196,17 +196,8 @@ __global__ void k_visit_policy(const int32_t* __restrict__ visits, const uint8_t
                                double* __restrict__ out64, float* __restrict__ out32) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= num) return;
-  const int32_t* vc = visits + (size_t)i * A;
-  long long sum = 0;
-  for (int a = 0; a < A; ++a) sum += vc[a];
-  const bool keep = !mask || mask[i];
-  for (int a = 0; a < A; ++a) {
-    // Python: visit_count / sum_visits on ints = correctly rounded double quotient (0/0 raises there;
-    // the callers never produce it: every root has num_simulations - 1 >= 1 visits)
-    const double p = keep ? __ddiv_rn((double)vc[a], (double)sum) : 0.0;
-    if (out64) out64[(size_t)i * A + a] = p;
-    if (out32) out32[(size_t)i * A + a] = (float)p;
-  }
+  visit_policy_row(visits + (size_t)i * A, !mask || mask[i], A, out64 ? out64 + (size_t)i * A : nullptr,
+                   out32 ? out32 + (size_t)i * A : nullptr);
 }
 
 static int check_view(const hz_traj_view* v, const char* who) {

@@ -4,6 +4,8 @@
 //   hz_wave_pack    every ticket's prepare inputs and root hidden states -> rows [k*n, (k+1)*n) of the staging
 //                   buffers, the rows of unused slots zero-filled (all-zero legal mask: a root without children)
 //   hz_wave_unpack  rows [k*n, (k+1)*n) of the wave's statistics buffer -> ticket k's outputs
+//   hz_wave_policy  the visit counts of the same rows -> ticket k's float64 policy targets (hz_visit_policy's
+//                   arithmetic, per ticket mask)
 // One launch each, in place of 5*G + 2*G cudaMemcpyAsync calls.  The ticket table travels by value in the kernel
 // parameters (64 x 56 B), so no descriptor buffer has to be updated in stream order.  Sources and destinations are
 // device memory or page-locked host memory, which the kernel reads and writes itself under unified addressing (as
@@ -22,6 +24,12 @@ struct WaveTable {
   hz_wave_ticket t[kWaveMaxSlots];
 };
 static_assert(sizeof(WaveTable) <= 4096, "the ticket table must fit the kernel parameter space");
+
+struct PolicyTable {
+  hz_policy_ticket t[kWaveMaxSlots];
+};
+static_assert(sizeof(PolicyTable) == 64 * 16, "the policy table is 64 x 16 B of kernel parameters");
+constexpr int kPolicyThreads = 128;
 
 // dst[0, words) = src[0, words), or zeros when src == NULL; 16-byte vectors when both ends allow, 4-byte words
 // otherwise.  The calling slot's blocks split the range.
@@ -66,6 +74,17 @@ __global__ void __launch_bounds__(kWaveThreads) k_wave_unpack(WaveTable tab, int
   const int64_t na = (int64_t)n * num_actions;
   if (tab.t[k].out_visits) copy_words((uint32_t*)tab.t[k].out_visits, stats + k * na, na);
   if (tab.t[k].out_values) copy_words((uint32_t*)tab.t[k].out_values, stats + slots * na + (int64_t)k * n, n);
+}
+
+// grid (ceil(n / kPolicyThreads), count): one thread per root of ticket blockIdx.y
+__global__ void __launch_bounds__(kPolicyThreads) k_wave_policy(PolicyTable tab, int n, int num_actions,
+                                                                const int32_t* __restrict__ stats) {
+  const int k = blockIdx.y;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const uint8_t* mask = tab.t[k].mask;
+  visit_policy_row(stats + ((int64_t)k * n + i) * num_actions, !mask || mask[i], num_actions,
+                   tab.t[k].out + (int64_t)i * num_actions, nullptr);
 }
 
 static int check_sizes(const char* fn, const hz_wave_ticket* tickets, int count, int slots, int n, int num_actions) {
@@ -144,6 +163,36 @@ int hz_wave_unpack(void* stream, int device, const hz_wave_ticket* tickets, int 
   k_wave_unpack<<<dim3(kWaveBlocksPerSlot, count), kWaveThreads, 0, (cudaStream_t)stream>>>(
       tab, slots, n, num_actions, (const uint32_t*)stats);
   HZ_LAUNCH_CHECK("k_wave_unpack");
+  return HZ_OK;
+}
+
+int hz_wave_policy(void* stream, int device, const hz_policy_ticket* tickets, int count, int slots, int n,
+                   int num_actions, const int32_t* stats) {
+  const char* fn = "hz_wave_policy";
+  if (!tickets) { set_error("%s: NULL ticket table", fn); return HZ_ERR_ARG; }
+  if (slots < 1 || slots > kWaveMaxSlots) { set_error("%s: slots = %d, must be 1..%d", fn, slots, kWaveMaxSlots); return HZ_ERR_ARG; }
+  if (count < 1 || count > slots) { set_error("%s: count = %d, must be 1..slots (%d)", fn, count, slots); return HZ_ERR_ARG; }
+  if (n < 1 || (int64_t)slots * n > kWaveMaxRows) {
+    set_error("%s: n = %d, must be >= 1 with slots * n <= %lld", fn, n, (long long)kWaveMaxRows);
+    return HZ_ERR_ARG;
+  }
+  if (num_actions < 1 || num_actions > 32) { set_error("%s: num_actions = %d, must be 1..32", fn, num_actions); return HZ_ERR_ARG; }
+  if (!stats) { set_error("%s: NULL statistics buffer", fn); return HZ_ERR_ARG; }
+  for (int k = 0; k < count; ++k) {
+    if (!tickets[k].out) { set_error("%s: ticket %d has a NULL output", fn, k); return HZ_ERR_ARG; }
+  }
+  DeviceGuard dg(device);
+  if (!dg.ok) return fail_cuda(cudaGetLastError(), fn);
+  if (int rc = check_ptr(fn, "statistics buffer", stats, device, 4)) return rc;
+  for (int k = 0; k < count; ++k) {
+    if (int rc = check_ptr(fn, "ticket mask", tickets[k].mask, device, 1)) return rc;
+    if (int rc = check_ptr(fn, "ticket out", tickets[k].out, device, 8)) return rc;
+  }
+  PolicyTable tab{};
+  for (int k = 0; k < count; ++k) tab.t[k] = tickets[k];
+  k_wave_policy<<<dim3((n + kPolicyThreads - 1) / kPolicyThreads, count), kPolicyThreads, 0, (cudaStream_t)stream>>>(
+      tab, n, num_actions, stats);
+  HZ_LAUNCH_CHECK("k_wave_policy");
   return HZ_OK;
 }
 

@@ -382,7 +382,9 @@ class SearchPipeline:
 
     Observation tickets (`stack` = frames per root, `mdp` = "global" or "local"): submit_observations() hands in
     stacked observations instead of the representation network's outputs, and the slot runs the root inference itself
-    (InitialPlan, one pack launch hz_obs_pack in place of hz_wave_pack).  A wave holds one kind of ticket.
+    (InitialPlan, one pack launch hz_obs_pack in place of hz_wave_pack).  A wave holds one kind of ticket.  Observation
+    tickets may hand in frame windows of consecutive positions (`positions`) and ask for policy targets (`out_policy`):
+    the reanalyze pipeline (reanalyze.ReanalyzePipeline).
 
     Waves fill only when a caller submits tickets ahead of its waits: a wait / stats / gathered on a ticket of the open
     wave launches it with the tickets it holds so far, so submit-then-wait per ticket runs waves of one ticket.  Ticket
@@ -441,7 +443,7 @@ class SearchPipeline:
                 # the open wave: its tickets' table entries, the inputs they point at, slow-path outputs, and one
                 # caller-stream event per ticket that the slot's stream waits for at launch
                 s.update(table=[], keep=[], post=[], ev_tickets=[torch.cuda.Event() for _ in range(self.wave)],
-                         kind="hidden", obs_table=[])
+                         kind="hidden", obs_table=[], positions=1, policy_table=[], policy=None)
         self._next = 0
         self._waves = WaveSchedule(self.wave, self.depth)
         self._hidden_shape = None    # wave > 1: (feature, pool dtype) of the root hidden states
@@ -559,8 +561,10 @@ class SearchPipeline:
         """Kind of ticket ("hidden" or "obs") the open wave holds, None when no wave is open."""
         return None if self._waves.open is None else self.slots[self._waves.open["slot"]]["kind"]
 
-    def _join(self, kind, noisy, fraction, rec, obs_rec, held, in_place, out_visits, out_values, t_host):
-        """The ticket takes the next position of the open wave (opening one if needed), launching it when full."""
+    def _join(self, kind, noisy, fraction, rec, obs_rec, held, in_place, out_visits, out_values, t_host, positions=1,
+              policy=None):
+        """The ticket takes the next position of the open wave (opening one if needed), launching it when full.
+        policy: (policy_mask address, out_policy) of an observation ticket that asked for policy targets."""
         n = self.n
         if self.wave == 1:
             self._waves._next = self._next      # submit() and observation tickets share the round robin over slots
@@ -575,11 +579,22 @@ class SearchPipeline:
                 t_host += time.perf_counter() - t_wait   # waiting for the GPU is not host time
             s["busy"] = True
             s["table"], s["keep"], s["post"], s["obs_table"], s["kind"] = [], [], [], [], kind
+            s["positions"], s["policy_table"] = positions, []
         s["keep"] += held                   # alive until the slot is reused
         rows = slice(p * n, (p + 1) * n)
         for out, ok, buf in zip((out_visits, out_values), in_place, (s["visits"], s["values"])):
             if out is not None and not ok:
                 s["post"].append((out, buf[rows]))
+        if obs_rec is not None:
+            prec = None
+            if policy is not None:
+                mask, out_policy = policy
+                if self._writable_policy(out_policy):
+                    prec = _lib.PolicyTicket(mask=mask, out=ptr(out_policy))
+                else:      # slow path: the slot's own rows, copied out after the policy launch
+                    prec = _lib.PolicyTicket(mask=mask, out=ptr(self._policy_rows(s)[rows]))
+                    s["post"].append((out_policy, s["policy"][rows]))
+            s["policy_table"].append(prec)
         rec.out_visits = ptr(out_visits) if in_place[0] else None
         rec.out_values = ptr(out_values) if in_place[1] else None
         s["table"].append(rec)
@@ -592,7 +607,8 @@ class SearchPipeline:
         self.submitted += 1
         return i * self.wave + p    # ticket id
 
-    def submit_observations(self, fraction, noises, obs, legal, out_visits=None, out_values=None):
+    def submit_observations(self, fraction, noises, obs, legal, out_visits=None, out_values=None, positions=1,
+                            policy_mask=None, out_policy=None):
         """A search that starts from stacked observations (core/selfplay_worker.py:258-283: stack_obs ->
         initial_inference -> prepare -> run_multi) instead of the representation network's outputs; needs a pipeline
         built with `stack` (frames per root) and `mdp` ("global" or "local" observations).  The root inference runs in
@@ -607,33 +623,73 @@ class SearchPipeline:
         `meta[:, 0]` of EnvPipeline's meta rows).  noises: float32 [n, A] or None (prepare_no_noise).  Rows may have any
         stride.  Inputs already in one of these forms on this device or in page-locked host memory are read by the
         pack kernel in place: keep them unchanged until wait(ticket).  Anything else is converted by torch on the
-        caller's stream first.  Outputs as for submit().  Weights: drain() before updating the module."""
+        caller's stream first.  Outputs as for submit().  Weights: drain() before updating the module.
+
+        Frame windows (`positions` = P > 1, the reanalyze batch, whose consecutive positions share frames): obs holds
+        n / P windows of S + P - 1 frames, [n / P, S + P - 1, D] (or [n / P, (S + P - 1) * D]; bits likewise with W),
+        and root i * P + p takes frames p .. p + S - 1 of window i; legal moves and noises stay per root.  The pack
+        kernel expands the windows on the device (hz_obs_pack_windows), so the caller hands in one window per sample
+        instead of P stacks (it still reads a frame once for every stack that holds it).  A wave holds tickets of one
+        P: a different P launches the open wave first.
+        Policy targets (`out_policy`, float64 of n * A elements): the visit counts turned into hz_visit_policy's
+        correctly rounded quotients, all-zero rows where `policy_mask` (uint8 [n], None keeps every row) is 0, by one
+        launch per wave after the statistics scatter (hz_wave_policy).  out_policy is written in place when it is
+        contiguous on this device or in page-locked host memory, else copied after the wave; the mask is read in place
+        under the same rule, else converted."""
         if self._iplan is None:
             raise RuntimeError("submit_observations needs a pipeline built with stack= (the frame layout)")
         t_host = time.perf_counter()
         noisy = noises is not None
         fraction = float(fraction) if noisy else 0.0
         n, a, held = self.n, self.a, []
+        positions = int(positions)
+        if positions < 1 or n % positions:
+            raise ValueError(f"positions = {positions} must be >= 1 and divide the {n} roots of a ticket")
         # every input and output checked, then converted, BEFORE the ticket takes a position
-        obs, ofmt, odtype, oshape, odense = self._obs_form(obs)
+        obs, ofmt, odtype, oshape, odense = self._obs_form(obs, positions)
         legal, lfmt, ldtype, lshape, ldense = self._legal_form(legal)
         if noises is not None and _as_tensor(noises).numel() != n * a:
             raise ValueError(f"noises must hold [{n}, {a}] values, got {tuple(_as_tensor(noises).shape)}")
         in_place = [self._wave_output(x, dtype, shape) for x, dtype, shape in
                     ((out_visits, torch.int32, (n, a)), (out_values, torch.float32, (n,)))]
+        if out_policy is None and policy_mask is not None:
+            raise ValueError("policy_mask without out_policy")
+        if out_policy is not None:
+            self._wave_output(out_policy, torch.float64, (n, a))       # raises unless it can take n * A values
+            if out_policy.dtype != torch.float64:
+                raise ValueError(f"out_policy must be float64, got {out_policy.dtype}")
+            if policy_mask is not None:
+                policy_mask = _as_tensor(policy_mask)
+                if policy_mask.numel() != n:
+                    raise ValueError(f"policy_mask must hold {n} values, got {tuple(policy_mask.shape)}")
+                policy_mask = policy_mask.reshape(n)
         orec = _lib.ObsTicket()
         orec.obs, orec.ld_obs = self._source(obs, odtype, oshape, odense, held)
         orec.legal, orec.ld_legal = self._source(legal, ldtype, lshape, ldense, held)
         orec.noise = self._wave_input(noises, torch.float32, (n, a), held)
         orec.obs_format, orec.legal_format = ofmt, lfmt
-        if self._waves.closes(noisy, fraction) or self._open_kind() == "hidden":
+        policy = None if out_policy is None else (self._wave_input(policy_mask, torch.uint8, (n,), held), out_policy)
+        if (self._waves.closes(noisy, fraction) or self._open_kind() == "hidden"
+                or (self._open_kind() == "obs" and self.slots[self._waves.open["slot"]]["positions"] != positions)):
             self._launch_wave()
         return self._join("obs", noisy, fraction, _lib.WaveTicket(), orec, held, in_place, out_visits, out_values,
-                          t_host)
+                          t_host, positions, policy)
 
-    def _obs_form(self, x):
-        """(tensor, HZ_OBS_* format, dtype the kernel reads, shape, frames dense in the row) of a ticket's frames."""
-        n, S = self.n, self.stack
+    def _writable_policy(self, x):
+        """True when hz_wave_policy can write `out_policy` itself (contiguous float64 here or in page-locked memory)."""
+        return x.dtype == torch.float64 and x.is_contiguous() and (
+            x.device == self.device or (x.device.type == "cpu" and x.is_pinned()))
+
+    def _policy_rows(self, s):
+        """The slot's float64 [wave * n, A] policy buffer: slow-path outputs and the rows of tickets without targets."""
+        if s["policy"] is None:
+            s["policy"] = torch.empty(self.wave * self.n, self.a, dtype=torch.float64, device=self.device)
+        return s["policy"]
+
+    def _obs_form(self, x, positions=1):
+        """(tensor, HZ_OBS_* format, dtype the kernel reads, shape, frames dense in the row) of a ticket's frames:
+        n / positions rows of stack + positions - 1 frames."""
+        n, S = self.n // positions, self.stack + positions - 1
         x = _as_tensor(x)
         if x.dtype == torch.int32:
             fmt, width, dtype = _lib.HZ_OBS_BITS, self.frame_words, torch.int32
@@ -705,9 +761,15 @@ class SearchPipeline:
         with torch.cuda.stream(compute):
             if s["kind"] == "obs":
                 b = s["ibound"]
-                check(lib.hz_obs_pack(st, dev, (_lib.ObsTicket * count)(*s["obs_table"]), count, self.wave, self.n,
-                                      self.a, _lib.C.byref(self._layout), ptr(b.x), ptr(s["legal"]),
-                                      ptr(s["noise"]) if w["noisy"] else None))
+                otab = (_lib.ObsTicket * count)(*s["obs_table"])
+                noise = ptr(s["noise"]) if w["noisy"] else None
+                if s["positions"] > 1:
+                    check(lib.hz_obs_pack_windows(st, dev, otab, count, self.wave, self.n, self.a,
+                                                  _lib.C.byref(self._layout), s["positions"], ptr(b.x), ptr(s["legal"]),
+                                                  noise))
+                else:
+                    check(lib.hz_obs_pack(st, dev, otab, count, self.wave, self.n, self.a, _lib.C.byref(self._layout),
+                                          ptr(b.x), ptr(s["legal"]), noise))
                 recurrent = self.mcts._plan(self.model)
                 if self._iplan.refresh() | bool(recurrent is not None and recurrent.refresh()):
                     # the weights were re-folded on this stream; the other slots' streams read them too
@@ -733,6 +795,13 @@ class SearchPipeline:
             if self.gather is not None:
                 s["ticket"] = self.gather.submit_flat(s["stats"])
             check(lib.hz_wave_unpack(st, dev, table, count, self.wave, self.n, self.a, ptr(s["stats"])))
+            if s["kind"] == "obs" and any(r is not None for r in s["policy_table"]):
+                # tickets without policy targets write theirs into the slot's own rows (the kernel takes no NULL output)
+                prows = [r if r is not None else
+                         _lib.PolicyTicket(mask=None, out=ptr(self._policy_rows(s)[k * self.n:(k + 1) * self.n]))
+                         for k, r in enumerate(s["policy_table"])]
+                check(lib.hz_wave_policy(st, dev, (_lib.PolicyTicket * count)(*prows), count, self.wave, self.n,
+                                         self.a, ptr(s["stats"])))
             for out, rows in s["post"]:
                 out.copy_(rows.reshape(out.shape), non_blocking=True)
             s["ev_out"].record(compute)

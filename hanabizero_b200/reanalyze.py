@@ -5,13 +5,17 @@
 `batch * (num_unroll_steps + 1)` stored positions with the current target model and turns the root visit
 counts into policy targets, all-zero for positions past the end of their trajectory.  Same engine as
 self-play (roots with all-zero legal masks included), nothing leaves the device until the targets do.
+
+`ReanalyzePipeline` is its asynchronous form over a SearchPipeline: the caller hands in one window of stored frames
+per sampled trajectory (the learner's K + 1 consecutive positions share all but K of their frames), the windows are
+expanded into stacks on the device, searches stay in flight, and the policy targets are written by one launch per wave.
 """
 import numpy as np
 import torch
 
 from . import _lib, cytree
 from ._lib import check, ptr
-from .mcts import MCTS
+from .mcts import MCTS, SearchPipeline, _as_tensor
 from .selfplay import dirichlet_noise
 
 
@@ -49,3 +53,73 @@ def reanalyze_policies(config, model, obs, legal_actions, policy_mask, num_unrol
     check(lib.hz_visit_policy(torch.cuda.current_stream(dev).cuda_stream, ptr(visits), ptr(mask), B, A, ptr(out), None))
     out = out.view(B // per, per, A)
     return out if as_tensor else out.cpu().numpy()
+
+
+class ReanalyzePipeline:
+    """reanalyze_policies with searches in flight: `batch` trajectory windows of `num_unroll_steps` + 1 positions per
+    ticket, one SearchPipeline of batch * (num_unroll_steps + 1) roots (`depth` slots, `wave` tickets per search).
+
+        rp = ReanalyzePipeline(config, model, batch, K, stack)
+        t = rp.submit(obs_windows, legal_actions, policy_mask, noise_seed=s, noise_step=i)    # returns at once
+        ...
+        targets = rp.result(t)           # float64 [batch, K + 1, A]
+
+    obs_windows: [batch, K + stack, D] float32 or uint8 0/1 frames, oldest first (a slice of the recorder's flushed
+    'o' rows), or packed bit strings int32 [batch, K + stack, W] / [batch, (K + stack) * W]; position p of a sample
+    searches frames p .. p + stack - 1.  legal_actions: [batch, K + 1, A] 0/1, or int32 bit-mask words [batch, K + 1].
+    policy_mask: [batch, K + 1] (0 = position past the end of its trajectory: an all-zero target row).  Inputs may be
+    device or page-locked host tensors, read in place: keep them unchanged until result(ticket).  Frames of masked
+    positions past the end of an episode may hold anything; with all-zero legal rows there, the targets do not depend
+    on them.  Without `noises` ([batch * (K + 1), A]) the Dirichlet draw is
+    dirichlet_noise(batch * (K + 1), A, alpha, seed=noise_seed, step=noise_step) on the caller's stream, the draw
+    reanalyze_policies makes; either way it is multiplied by the legal mask, as there.  The exploration fraction is
+    config.root_exploration_fraction and the root reward 0.  `out` (float64, batch * (K + 1) * A elements) receives
+    the targets; by default a new device tensor.  Results equal a submit_observations of the expanded stacks followed
+    by hz_visit_policy; against reanalyze_policies they differ only by the plan's rounding of the root inference.
+    Weights: drain() before updating the module.  Not thread-safe, as SearchPipeline."""
+
+    def __init__(self, config, model, batch, num_unroll_steps, stack, mdp="global", depth=8, wave=1, device=None):
+        self.config, self.model = config, model
+        self.batch, self.per, self.stack = int(batch), int(num_unroll_steps) + 1, int(stack)
+        self.a = int(config.action_space_size)
+        self.roots = self.batch * self.per
+        model.eval()
+        self.pipe = SearchPipeline(MCTS(config), model, self.roots, self.a, depth=depth, device=device, wave=wave,
+                                   stack=self.stack, mdp=mdp)
+        self.device = self.pipe.device
+        self._out = {}
+
+    def submit(self, obs_windows, legal_actions, policy_mask, noises=None, noise_seed=0, noise_step=0, out=None):
+        B, per, a, dev = self.batch, self.per, self.a, self.device
+        legal = _as_tensor(legal_actions)
+        if tuple(legal.shape) not in ((B, per, a), (B, per)) or (legal.dim() == 2 and legal.dtype != torch.int32):
+            raise ValueError(f"legal_actions must be [{B}, {per}, {a}] or int32 bit masks [{B}, {per}], "
+                             f"got {legal.dtype} {tuple(legal.shape)}")
+        mask = _as_tensor(policy_mask)
+        if tuple(mask.shape) != (B, per):
+            raise ValueError(f"policy_mask must be [{B}, {per}], got {tuple(mask.shape)}")
+        self.pipe._obs_form(obs_windows, per)          # raises on a wrong window shape before any device work
+        if out is None:
+            out = torch.empty(B, per, a, dtype=torch.float64, device=dev)
+        legal = legal.reshape(self.roots, -1) if legal.dim() == 3 else legal.reshape(self.roots)
+        if legal.dim() == 2:
+            legal_f = legal.to(device=dev, dtype=torch.float32, non_blocking=True)
+        else:       # bit-mask words -> 0/1 rows for the noise mask
+            words = legal.to(device=dev, non_blocking=True)
+            legal_f = ((words.unsqueeze(1) >> torch.arange(a, device=dev, dtype=torch.int32)) & 1).float()
+        if noises is None:
+            noises = dirichlet_noise(self.roots, a, getattr(self.config, "root_dirichlet_alpha", 0.3), dev, noise_seed,
+                                     noise_step)
+        noises = cytree.as_device(noises, torch.float32, dev, (self.roots, a)) * legal_f           # :343
+        t = self.pipe.submit_observations(self.config.root_exploration_fraction, noises, obs_windows, legal,
+                                          positions=per, policy_mask=mask.reshape(self.roots), out_policy=out)
+        self._out[t] = out
+        return t
+
+    def result(self, ticket):
+        """The targets of a ticket, float64 [batch, K + 1, A] (its `out`), once its search is done."""
+        self.pipe.wait(ticket)
+        return self._out[ticket].view(self.batch, self.per, self.a)
+
+    def drain(self):
+        self.pipe.drain()

@@ -483,6 +483,18 @@ int hz_wave_pack(void* stream, int device, const hz_wave_ticket* tickets, int co
  * wanted).  `slots` is the wave's size, which places the value block. */
 int hz_wave_unpack(void* stream, int device, const hz_wave_ticket* tickets, int count, int slots, int n,
                    int num_actions, const int32_t* stats);
+/* Policy targets straight from a wave's statistics (the reanalyze caller, SearchPipeline.submit_observations with
+ * out_policy): for ticket k, out[i][a] = visits[k*n + i][a] / sum_a visits[k*n + i] as hz_visit_policy computes it
+ * (correctly rounded double quotient; all zero where mask[i] == 0, mask == NULL keeps every row), visits being the first
+ * slots*n*A words of `stats` (laid out as for hz_wave_unpack).  mask uint8 [n] and out double [n][A] (8-byte aligned,
+ * never NULL) are device memory of `device` or page-locked host memory, read and written by the kernel itself.  Sizes
+ * and pointers are checked before the launch as in hz_wave_unpack; one launch, the table travels by value. */
+typedef struct hz_policy_ticket {
+  const uint8_t* mask;     /* [n] or NULL */
+  double* out;             /* [n][A] */
+} hz_policy_ticket;
+int hz_wave_policy(void* stream, int device, const hz_policy_ticket* tickets, int count, int slots, int n,
+                   int num_actions, const int32_t* stats);
 
 /* Observation tickets (SearchPipeline.submit_observations): a wave whose tickets hand in stacked observations instead
  * of the representation network's outputs.  hz_obs_pack fills, for ticket k, rows [k*n, (k+1)*n) of
@@ -526,6 +538,14 @@ typedef struct hz_obs_layout {
 } hz_obs_layout;
 int hz_obs_pack(void* stream, int device, const hz_obs_ticket* tickets, int count, int slots, int n, int num_actions,
                 const hz_obs_layout* layout, void* x, int32_t* legal, float* noise);
+/* hz_obs_pack over frame WINDOWS (the reanalyze batch: consecutive positions of one trajectory share frames): row i of
+ * a ticket's obs holds stack + positions - 1 consecutive frames in any of the three formats (ld_obs = the window row
+ * stride, at least the window's elements), and root r = i * positions + p takes window frames p .. p + stack - 1,
+ * oldest first, landing in x exactly where hz_obs_pack puts root r of the expanded stacks.  Legal rows and noise stay
+ * per root (n rows).  positions is 1..n and divides n.  Everything else as hz_obs_pack, checked before the launch. */
+int hz_obs_pack_windows(void* stream, int device, const hz_obs_ticket* tickets, int count, int slots, int n,
+                        int num_actions, const hz_obs_layout* layout, int positions, void* x, int32_t* legal,
+                        float* noise);
 
 #ifdef __cplusplus
 }
