@@ -11,8 +11,10 @@
 //
 // and — the point of this file — the SAME function runs on the host (hz_host_dirichlet_noise): every floating-point
 // operation is an IEEE float64 +, -, *, /, sqrt or fma, and log / exp are fixed polynomials built from those, so the
-// host twin returns the device's noise bit for bit (tests/test_selfplay_gpu.py).  A search can therefore be replayed
-// on the CPU — through the reference's own cytree — with exactly the noise the device used.
+// host twin returns the device's noise bit for bit (tests/test_noise_gpu.py).  A search can therefore be replayed on
+// the CPU — through the reference's own cytree — with exactly the noise the device used.  The twin itself is checked
+// against an independent float64 port, Random123's known answers and the float32-rounded Beta law
+// (tests/test_noise_reference_cpu.py).
 #include <math.h>
 
 #include "hz_common.cuh"
@@ -137,8 +139,11 @@ HZ_HD double det_exp(double x) {   // x <= 0
   return bits_d(d_bits(p) + ((unsigned long long)(long long)k << 52));
 }
 
-// Gamma(alpha, 1) of stream (seed, step, root, action).  Every attempt consumes two Philox blocks.
-HZ_HD double gamma_draw(double alpha, unsigned long long seed, uint32_t step, uint32_t root, uint32_t action) {
+// Gamma(alpha, 1) of stream (seed, step, root, action).  Every attempt consumes two Philox blocks.  For alpha < 1 the
+// draw is d*v * U^(1/alpha), which det_exp cuts to 0 once log U / alpha < -700; *lg receives its logarithm
+// log(d*v) + log U / alpha as well, so that a row whose gammas all underflow can be rescaled (dirichlet_row_scale).
+HZ_HD double gamma_draw(double alpha, unsigned long long seed, uint32_t step, uint32_t root, uint32_t action,
+                        double* lg) {
   const uint32_t k0 = (uint32_t)seed, k1 = (uint32_t)(seed >> 32);
   const bool boost = alpha < 1.0;
   const double a = boost ? d_add(alpha, 1.0) : alpha;
@@ -160,20 +165,39 @@ HZ_HD double gamma_draw(double alpha, unsigned long long seed, uint32_t step, ui
                         det_log(u) < d_fma(0.5, x2, d_mul(d, d_add(d_add(1.0, -v), det_log(v))));
     if (!accept) continue;
     double g = d_mul(d, v);
-    if (boost) g = d_mul(g, det_exp(d_div(det_log(uniform53(b1.v[2], b1.v[3])), alpha)));   // * U^(1/alpha)
+    if (boost) {   // * U^(1/alpha)
+      const double e = d_div(det_log(uniform53(b1.v[2], b1.v[3])), alpha);
+      *lg = d_add(det_log(g), e);
+      g = d_mul(g, det_exp(e));
+    }
     return g;
   }
 }
 
+// Row maximum m of the log-gammas (alpha < 1 only).  While m >= -580 the gammas are used as drawn: any of them that
+// det_exp cut to 0 (log U / alpha < -700, so lg < -695) is below e^-116 < 2^-150 times the largest and rounds to 0 in
+// float32 anyway.  Below, the row is rescaled to exp(lg - m), so its largest gamma is 1 and the sum cannot underflow
+// to 0 (a 0/0 row).
+HZ_HD double dirichlet_row_scale(double g, double lg, double m) { return m < -580.0 ? det_exp(d_add(lg, -m)) : g; }
+
 // one warp per root on the device
-__global__ void __launch_bounds__(128) k_dirichlet(float* __restrict__ out, const uint8_t* __restrict__ legal_u8,
-                                                   const float* __restrict__ legal_f32, int N, int A, double alpha,
-                                                   unsigned long long seed, uint32_t step, uint32_t root_offset) {
+__global__ void __launch_bounds__(128) k_dirichlet(float* __restrict__ out, const float* __restrict__ legal_f32, int N,
+                                                   int A, double alpha, unsigned long long seed, uint32_t step,
+                                                   uint32_t root_offset) {
   const int lane = threadIdx.x & 31;
   const int n = blockIdx.x * 4 + (threadIdx.x >> 5);
   if (n >= N) return;
-  double g = 0.0;
-  if (lane < A) g = gamma_draw(alpha, seed, step, root_offset + (uint32_t)n, (uint32_t)lane);
+  double g = 0.0, lg = -HUGE_VAL;
+  if (lane < A) g = gamma_draw(alpha, seed, step, root_offset + (uint32_t)n, (uint32_t)lane, &lg);
+  if (alpha < 1.0) {
+    double m = lg;
+    for (int o = 16; o > 0; o >>= 1) {
+      const double mo = __hiloint2double(__shfl_xor_sync(HZ_FULL, __double2hiint(m), o),
+                                         __shfl_xor_sync(HZ_FULL, __double2loint(m), o));
+      m = mo > m ? mo : m;
+    }
+    if (lane < A) g = dirichlet_row_scale(g, lg, m);
+  }
   double sum = 0.0;
   for (int a = 0; a < A; ++a) {   // ascending, like numpy's pairwise-free small sums
     const double ga = __hiloint2double(__shfl_sync(HZ_FULL, __double2hiint(g), a), __shfl_sync(HZ_FULL, __double2loint(g), a));
@@ -182,7 +206,6 @@ __global__ void __launch_bounds__(128) k_dirichlet(float* __restrict__ out, cons
   if (lane < A) {
     float v = (float)d_div(g, sum);
     // reanalyze multiplies the draw by the legal mask (reanalyze_worker.py:343)
-    if (legal_u8 && legal_u8[(size_t)n * A + lane] == 0) v = 0.0f;
     if (legal_f32 && legal_f32[(size_t)n * A + lane] == 0.0f) v = 0.0f;
     out[(size_t)n * A + lane] = v;
   }
@@ -192,30 +215,42 @@ __global__ void __launch_bounds__(128) k_dirichlet(float* __restrict__ out, cons
 
 using namespace hz;
 
+// Finite alpha only, within [1e-300, 1e300]: below, log U / alpha can overflow to -inf for every gamma of a row; above,
+// the sum of 32 gammas can overflow to inf.  Both would give NaN rows.
+static bool alpha_ok(double alpha) { return alpha >= 1e-300 && alpha <= 1e300; }
+
 extern "C" {
 #pragma GCC visibility push(default)
 
 int hz_dirichlet_noise(void* stream, float* out, int num_roots, int num_actions, double alpha, uint64_t seed,
                        uint32_t step, uint32_t root_offset, const float* legal_mask) {
-  if (!out || num_roots <= 0 || num_actions <= 0 || num_actions > 32 || !(alpha > 0.0)) {
+  if (!out || num_roots <= 0 || num_actions <= 0 || num_actions > 32 || !alpha_ok(alpha)) {
     set_error("hz_dirichlet_noise: bad argument");
     return HZ_ERR_ARG;
   }
-  k_dirichlet<<<(num_roots + 3) / 4, 128, 0, (cudaStream_t)stream>>>(out, nullptr, legal_mask, num_roots, num_actions,
-                                                                       alpha, seed, step, root_offset);
+  k_dirichlet<<<(num_roots + 3) / 4, 128, 0, (cudaStream_t)stream>>>(out, legal_mask, num_roots, num_actions, alpha,
+                                                                       seed, step, root_offset);
   HZ_LAUNCH_CHECK("k_dirichlet");
   return HZ_OK;
 }
 
 int hz_host_dirichlet_noise(float* out, int num_roots, int num_actions, double alpha, uint64_t seed, uint32_t step,
                             uint32_t root_offset, const float* legal_mask) {
-  if (!out || num_roots <= 0 || num_actions <= 0 || num_actions > 32 || !(alpha > 0.0)) {
+  if (!out || num_roots <= 0 || num_actions <= 0 || num_actions > 32 || !alpha_ok(alpha)) {
     set_error("hz_host_dirichlet_noise: bad argument");
     return HZ_ERR_ARG;
   }
   for (int n = 0; n < num_roots; ++n) {
-    double g[32], sum = 0.0;
-    for (int a = 0; a < num_actions; ++a) g[a] = gamma_draw(alpha, seed, step, root_offset + (uint32_t)n, (uint32_t)a);
+    double g[32], lg[32], sum = 0.0;
+    for (int a = 0; a < num_actions; ++a) {
+      lg[a] = -HUGE_VAL;
+      g[a] = gamma_draw(alpha, seed, step, root_offset + (uint32_t)n, (uint32_t)a, &lg[a]);
+    }
+    if (alpha < 1.0) {
+      double m = lg[0];
+      for (int a = 1; a < num_actions; ++a) m = lg[a] > m ? lg[a] : m;
+      for (int a = 0; a < num_actions; ++a) g[a] = dirichlet_row_scale(g[a], lg[a], m);
+    }
     for (int a = 0; a < num_actions; ++a) sum = sum + g[a];
     for (int a = 0; a < num_actions; ++a) {
       float v = (float)(g[a] / sum);

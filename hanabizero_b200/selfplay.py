@@ -20,8 +20,9 @@ from .mcts import MCTS
 def dirichlet_noise(num, actions, alpha, device, seed=0, step=0, root_offset=0, legal=None):
     """np.random.dirichlet([alpha] * A) per root (selfplay_worker.py:279, reanalyze_worker.py:343), drawn on the
     device from counter-based streams keyed by (seed, step, root_offset + root, action): float32 CUDA [num, actions].
-    `legal` (float [num, actions]) zeroes the entries of illegal actions after normalisation (the reanalyze caller's
-    `noise * legal`).  `dirichlet_noise_host` returns the same numbers, bit for bit, without a GPU."""
+    `legal` (float [num, actions]) zeroes, after normalisation, the entries whose mask value == 0 (-0 included); any
+    other value, 0.5 or NaN included, leaves the entry as drawn.  alpha must lie in [1e-300, 1e300].
+    `dirichlet_noise_host` returns the same numbers, bit for bit, without a GPU."""
     lib = _lib.load()
     dev = torch.device(device)
     out = torch.empty(num, actions, dtype=torch.float32, device=dev)

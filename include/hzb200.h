@@ -290,10 +290,13 @@ int hz_support_decode(void* stream, const void* logits, int elem_bytes, const fl
 /* Root exploration noise (np.random.dirichlet([alpha] * A) per root, /root/reference/core/selfplay_worker.py:279,
  * reanalyze_worker.py:343-344) from counter-based streams: Philox4x32-10 keyed by `seed`, counter (block, action,
  * root_offset + root, step); Gamma(alpha) by Marsaglia-Tsang, normalised in ascending order, rounded to float32.
- * out float[N][A] (dev).  legal_mask (optional, float[N][A]): entries with mask 0 are zeroed AFTER normalisation, as
- * the reanalyze caller does.  hz_host_dirichlet_noise is the host twin (host pointers, no device work): the same
- * arithmetic built from IEEE float64 operations only, bit-identical output — a search can be replayed on the CPU
- * (e.g. through the reference's own cytree) with exactly the noise the device drew. */
+ * alpha must lie in [1e-300, 1e300] (NaN and inf are rejected with HZ_ERR_ARG); 1 <= A <= 32.  For alpha < 1 a row
+ * whose gammas would all underflow is rescaled by its largest one, so every row is finite and sums to 1 within
+ * float32 rounding.  out float[N][A] (dev).  legal_mask (optional, float[N][A]): an entry is zeroed AFTER
+ * normalisation when its mask value == 0.0f (-0.0f included); any other value, 0.5 or NaN included, leaves the entry
+ * as drawn — this is not noise * legal.  hz_host_dirichlet_noise is the host twin (host pointers, no device work):
+ * the same arithmetic built from IEEE float64 operations only, bit-identical output — a search can be replayed on the
+ * CPU (e.g. through the reference's own cytree) with exactly the noise the device drew. */
 int hz_dirichlet_noise(void* stream, float* out, int num_roots, int num_actions, double alpha, uint64_t seed,
                        uint32_t step, uint32_t root_offset, const float* legal_mask);
 int hz_host_dirichlet_noise(float* out, int num_roots, int num_actions, double alpha, uint64_t seed, uint32_t step,

@@ -299,3 +299,22 @@ def unpack_traj_golden(g):
                         r=g["out_r"][s:s + n], o=out_o[so:so + stack + n], la=g["out_la"][sl:sl + n + 1]))
         s, so, sl = s + n, so + stack + n, sl + n + 1
     return obs, eps
+
+
+def rounded_beta_ks(x, a, b):
+    """KS p-value of float32 samples x against fl32(Beta(a, b)): P(fl32(X) <= v) = F(midpoint of v and the next
+    float32 above v), a discrete law, so the supremum is taken at each observed value and just below it.  The
+    continuous-law p-value is conservative for a discrete law."""
+    from scipy import special, stats
+    x = np.sort(np.asarray(x, np.float32))
+    n = x.size
+    v, counts = np.unique(x, return_counts=True)
+    up = np.nextafter(v, np.float32(np.inf)).astype(np.float64)
+    dn = np.nextafter(v, np.float32(-np.inf)).astype(np.float64)
+    vd = v.astype(np.float64)
+    cdf_at = np.where(v >= 1.0, 1.0, special.betainc(a, b, np.minimum((vd + up) / 2, 1.0)))
+    cdf_below = np.where(v <= 0.0, 0.0, special.betainc(a, b, np.maximum((vd + dn) / 2, 0.0)))
+    emp_at = np.cumsum(counts) / n
+    emp_below = emp_at - counts / n
+    d = max(np.abs(emp_at - cdf_at).max(), np.abs(emp_below - cdf_below).max())
+    return stats.kstwo.sf(d, n)

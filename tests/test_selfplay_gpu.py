@@ -132,23 +132,6 @@ def test_evaluate_equals_a_reference_style_host_loop():
     assert all(m >= 1 for m in moves)
 
 
-@pytest.mark.parametrize("alpha,A,N", [(0.3, 20, 4096), (0.3, 11, 37), (1.5, 32, 5)])
-def test_device_dirichlet_equals_its_host_twin_bit_for_bit(alpha, A, N):
-    """hz_dirichlet_noise (device) == hz_host_dirichlet_noise (host): same Philox streams, same IEEE float64
-    arithmetic, so a device search can be replayed on the CPU with exactly its noise (SURVEY §8f N1)."""
-    from hanabizero_b200.selfplay import dirichlet_noise, dirichlet_noise_host
-    dev = torch.device("cuda")
-    legal = (torch.rand(N, A, device=dev) < 0.6).float()
-    for step, off, lg in ((0, 0, None), (7, 1000, None), (3, 5, legal)):
-        d = dirichlet_noise(N, A, alpha, dev, seed=1234567890123, step=step, root_offset=off, legal=lg).cpu().numpy()
-        h = dirichlet_noise_host(N, A, alpha, seed=1234567890123, step=step, root_offset=off,
-                                 legal=None if lg is None else lg.cpu().numpy())
-        assert (d.view(np.uint32) == h.view(np.uint32)).all(), (step, off)
-        assert np.isfinite(d).all() and (d >= 0).all()
-        if lg is None:
-            np.testing.assert_allclose(d.astype(np.float64).sum(1), 1.0, atol=2e-6)
-
-
 def test_selfplay_engine_noise_is_reproducible_on_the_host():
     """SelfPlayEngine draws move m's root noise from stream (noise_seed, m, game): regenerating it on the host and
     searching the same roots through the generic calls gives the engine's visit counts."""
