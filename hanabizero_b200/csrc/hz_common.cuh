@@ -72,12 +72,12 @@ inline int check_ptr(const char* fn, const char* what, const void* p, int device
 
 // One root's policy target from its visit counts vc[0, A) (hz_visit_policy, hz_wave_policy): out[a] = vc[a] / sum as a
 // correctly rounded double quotient (Python's int / int), all zero when !keep.  out64 / out32 may be NULL.
+// A kept row with sum 0 is all NaN (0 / 0, where Python raises); searches leave num_simulations - 1 >= 1 visits.
 __device__ __forceinline__ void visit_policy_row(const int32_t* vc, bool keep, int A, double* out64, float* out32) {
-  long long sum = 0;
+  long long sum = 0;   // 32 counts up to 2^31 - 1: past 2^32, exact in 64 bits and in the double it becomes
   for (int a = 0; a < A; ++a) sum += vc[a];
   for (int a = 0; a < A; ++a) {
-    // Python: visit_count / sum_visits on ints = correctly rounded double quotient (0/0 raises there;
-    // the callers never produce it: every root has num_simulations - 1 >= 1 visits)
+    // Python: visit_count / sum_visits on ints = correctly rounded double quotient
     const double p = keep ? __ddiv_rn((double)vc[a], (double)sum) : 0.0;
     if (out64) out64[a] = p;
     if (out32) out32[a] = (float)p;

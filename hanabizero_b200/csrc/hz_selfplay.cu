@@ -13,13 +13,13 @@
 namespace hz {
 
 __global__ void k_select_action(int32_t* __restrict__ visits, const float* __restrict__ legal,
-                                const float* __restrict__ temperature, const double* __restrict__ uniforms,
+                                const double* __restrict__ temperature, const double* __restrict__ uniforms,
                                 int N, int A, int32_t* __restrict__ out_action, float* __restrict__ out_entropy) {
   const int i = blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= N) return;
   int32_t* v = visits + (size_t)i * A;
   const float* lg = legal + (size_t)i * A;
-  const double inv_t = 1.0 / (double)(temperature ? temperature[i] : 1.0f);
+  const double inv_t = temperature ? 1.0 / temperature[i] : 1.0;   // Python's 1 / temperature, in double
   double p[32];
   double total = 0.0;
   int best = 0, best_v = -2147483647 - 1;
@@ -28,7 +28,14 @@ __global__ void k_select_action(int32_t* __restrict__ visits, const float* __res
     if (lg[a] == 0.0f && c >= 1) { c = 0; v[a] = 0; }          // utils.py:282-284 (mutates the counts)
     if (c > best_v) { best_v = c; best = a; }                   // np.argmax: first maximum
     p[a] = (inv_t == 1.0) ? (double)c : pow((double)c, inv_t);  // visit_count ** (1 / temperature)
-    total += p[a];
+    total += p[a];                                              // ascending order (not Python >= 3.12's compensated sum)
+  }
+  if (!(total > 0.0 && isfinite(total))) {
+    // no visits left after the zeroing (the reference's ZeroDivisionError), or c^(1/T) or its sum out of range (its
+    // OverflowError): no move is defined.  -1 is never legal, so the env kernel raises its sticky illegal-move error.
+    out_action[i] = -1;
+    if (out_entropy) out_entropy[i] = __int_as_float(0x7fc00000);
+    return;
   }
   double ent = 0.0, cum = 0.0;
   for (int a = 0; a < A; ++a) {
@@ -129,7 +136,7 @@ using namespace hz;
 extern "C" {
 #pragma GCC visibility push(default)
 
-int hz_select_action(void* stream, int32_t* visits, const float* legal, const float* temperature,
+int hz_select_action(void* stream, int32_t* visits, const float* legal, const double* temperature,
                      const double* uniforms, int num, int num_actions, int32_t* out_action, float* out_entropy) {
   if (!visits || !legal || !out_action || num <= 0 || num_actions <= 0 || num_actions > 32) {
     set_error("hz_select_action: bad argument");

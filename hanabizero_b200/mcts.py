@@ -36,6 +36,10 @@ class SearchConfig:
     def __init__(self, num_simulations=50, discount=0.999, value_delta_max=0.006, pb_c_base=19652,
                  pb_c_init=1.25, amp_type="none", root_dirichlet_alpha=0.3,
                  root_exploration_fraction=0.25):
+        if int(num_simulations) < 2:
+            # the last simulation is skipped (core/mcts.py:25-26): one simulation leaves the root without visits, and
+            # neither a move nor a policy target is defined from zero counts
+            raise ValueError(f"num_simulations = {num_simulations}: a search needs at least 2")
         self.num_simulations = num_simulations
         self.discount = discount
         self.value_delta_max = value_delta_max

@@ -46,14 +46,16 @@ def select_action_batch(visit_counts, legal_actions, temperature=1.0, determinis
     """Batched select_action on the device.  visit_counts int32 [N, A] CUDA (illegal entries are zeroed
     in place, as the reference mutates its argument), legal_actions float [N, A].  Non-deterministic
     sampling consumes `uniforms` (float64 [N] in [0, 1); drawn with torch if omitted) through
-    numpy.random.choice's inverse-CDF rule.  Returns (actions int32 [N], entropies float32 [N])."""
+    numpy.random.choice's inverse-CDF rule.  `temperature` (a number or [N] per row) reaches the kernel as float64, so
+    the exponent is Python's 1 / temperature.  Returns (actions int32 [N], entropies float32 [N]); a row left without
+    a distribution (no visits on a legal move, or c^(1/T) overflowing) gets action -1 and NaN entropy."""
     n, a = visit_counts.shape
     dev = visit_counts.device
     lib = _lib.load()
     legal = legal_actions.to(device=dev, dtype=torch.float32).contiguous()
     temp = None
     if not (isinstance(temperature, (int, float)) and float(temperature) == 1.0):
-        temp = torch.as_tensor(temperature, dtype=torch.float32, device=dev).expand(n).contiguous()
+        temp = torch.as_tensor(temperature, dtype=torch.float64, device=dev).expand(n).contiguous()
     if deterministic:
         uni = None
     else:

@@ -303,11 +303,14 @@ int hz_host_dirichlet_noise(float* out, int num_roots, int num_actions, double a
                             uint32_t root_offset, const float* legal_mask);
 
 /* select_action (/root/reference/core/utils.py:280-295): visits int32[N][A] (dev; counts of illegal
- * actions are zeroed in place like the reference does), legal float[N][A], temperature float[N] or
- * NULL (= 1), uniforms double[N] in [0,1) or NULL (deterministic: first arg-max).  Sampling follows
- * numpy.random.choice (cdf = cumsum(p)/sum, searchsorted side='right') for the given uniform.
- * out_action int32[N], out_entropy float[N] or NULL (base-2 entropy of the visit distribution). */
-int hz_select_action(void* stream, int32_t* visits, const float* legal, const float* temperature,
+ * actions are zeroed in place like the reference does), legal float[N][A], temperature double[N] or
+ * NULL (= 1), uniforms double[N] in [0,1) or NULL (deterministic: first arg-max).  p[a] = pow(c[a], 1 / T)
+ * in double, summed in ascending order.  Sampling follows numpy.random.choice (cdf = cumsum(p)/sum,
+ * searchsorted side='right') for the given uniform.  out_action int32[N], out_entropy float[N] or NULL
+ * (base-2 entropy of the visit distribution).  A row whose sum of p is 0 (no visits left on a legal move) or not
+ * finite (c^(1/T) overflows: a tiny or zero temperature) has no distribution: its action is -1, which the env
+ * kernels reject as an illegal move, and its entropy NaN. */
+int hz_select_action(void* stream, int32_t* visits, const float* legal, const double* temperature,
                      const double* uniforms, int num, int num_actions, int32_t* out_action, float* out_entropy);
 /* Frame stack on the device (core/game.py:169-174): stack float[N][depth][dim] shifts left by one
  * frame and appends obs[i] (row stride ld_obs); where done[i] != 0 every slot is filled with obs[i]
@@ -378,8 +381,10 @@ int hz_traj_pack(void* stream, const hz_traj_view* v, int num_episodes, const in
                  int32_t* out_reward, int32_t* out_visits, float* out_root);
 /* Policy targets from visit counts (store_search_stats, game.py:194-197; the reanalyze caller,
  * /root/reference/core/reanalyze_worker.py:352-367, SURVEY.md §8f N4): out[i][a] = visits[i][a] / sum_a visits[i]
- * as a correctly rounded double quotient (Python's int / int), rows with mask[i] == 0 (dev uint8[N], NULL = keep
- * all) all zero.  out64 double[N][A] and/or out32 float[N][A] (dev). */
+ * as a correctly rounded double quotient (Python's int / int, the sum taken in 64 bits), rows with mask[i] == 0
+ * (dev uint8[N], NULL = keep all) all zero.  A kept row whose counts sum to 0 is all NaN (0 / 0: Python raises
+ * ZeroDivisionError there); SearchConfig rejects num_simulations < 2, so no search leaves such a root.
+ * out64 double[N][A] and/or out32 float[N][A] (dev). */
 int hz_visit_policy(void* stream, const int32_t* visits, const uint8_t* mask, int num, int num_actions, double* out64,
                     float* out32);
 

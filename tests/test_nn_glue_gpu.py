@@ -30,10 +30,11 @@ DECODE_CASES = [(torch.float32, 201, 201), (torch.float16, 201, 208), (torch.flo
 
 @pytest.mark.parametrize("dtype,width,ld", DECODE_CASES)
 def test_support_decode_matches_float64_reference(dtype, width, ld):
-    """Accurate float32 arithmetic only (libdevice expf, IEEE division and square root): within the path's 1e-5
-    relative bar of a float64 evaluation of the reference's formula, plus 2e-5 absolute per 100 of the support's
-    half-width (at least 2e-5) — two ulp of expf times the half-width, which is what float32 softmax sums over the
-    support can cancel to — and closer to float64 than the reference's own float32 evaluation, whose textbook form
+    """float32 arithmetic with one approximate step (exp as ex2.approx.ftz, 2 ulp; IEEE division and square root):
+    within the path's 1e-5 relative bar of a float64 evaluation of the reference's formula, plus 2e-5 absolute per 100
+    of the support's half-width (at least 2e-5) — two ulp of the exponential times the half-width, which is what float32
+    softmax sums over the support can cancel to (tests/test_selfplay_glue_gpu.py holds the decode to a bound derived
+    term by term) — and closer to float64 than the reference's own float32 evaluation, whose textbook form
     cancels twice near zero (where that form loses anything at all).  The same rows read from a base one element past
     a 16-byte boundary (the scalar load path) decode to the same bits."""
     from hanabizero_b200 import _lib

@@ -93,8 +93,9 @@ def test_full_entry_still_rejects_small_shapes():
     lib = _lib.load()
     h = ctypes.c_void_p()
     w = _weights()
+    launches = lib.hz_launch_count()          # (GPU tests earlier in the same process have launched kernels)
     assert lib.hz_rowchain_create(ctypes.byref(h), 0, ctypes.byref(w), 128, BUF, 528, BUF, BUF) == _lib.HZ_ERR_ARG
-    assert lib.hz_launch_count() == 0
+    assert lib.hz_launch_count() == launches
 
 
 def test_auto_executor_follows_the_measured_crossover():
