@@ -97,6 +97,7 @@ SIGNATURES = {
     "hz_obs_pack": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _vp, _vp, _vp]),
     "hz_obs_pack_windows": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _i, _vp, _vp, _vp]),
     "hz_wave_policy": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp]),
+    "hz_obs_pack_episodes": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _vp, _i, _vp, _vp, _vp]),
 }
 
 
@@ -154,6 +155,11 @@ class ObsTicket(C.Structure):
     """struct hz_obs_ticket (include/hzb200.h)."""
     _fields_ = [("obs", _vp), ("ld_obs", _i64), ("legal", _vp), ("ld_legal", _i64), ("noise", _vp),
                 ("obs_format", C.c_int32), ("legal_format", C.c_int32)]
+
+
+class EpisodeTicket(C.Structure):
+    """struct hz_obs_episode_ticket (include/hzb200.h)."""
+    _fields_ = [("frames", _vp), ("ld_frames", _i64), ("legal", _vp), ("samples", _vp), ("noise", _vp), ("mask", _vp)]
 
 
 class ObsLayout(C.Structure):

@@ -7,6 +7,9 @@
 //                i * positions + p takes window frames p .. p + stack - 1 (the reanalyze batch, whose consecutive
 //                positions share frames, is handed in as one window per sample instead of one stack per position;
 //                each root still reads its own stack, so a shared frame is read once per stack that holds it)
+//   hz_obs_pack_episodes  the windows read from an episode store's byte arenas (trajectory.EpisodeStore) by
+//                (first frame row, last frame row, first legal row, positions with targets) per sample: frames past the
+//                episode's end clamped to its last row, legal rows and noise zero and the policy mask 0 past it
 // One launch per wave.  The ticket table travels by value in the kernel parameters, as in hz_wave.cu.  Sources are
 // device memory or page-locked host memory, read by the kernel itself under unified addressing: for host sources
 // the launch is spread over enough CTAs to keep many reads in flight over the host link.
@@ -264,6 +267,138 @@ static int obs_pack(const char* fn, bool windows, void* stream, int device, cons
   return HZ_OK;
 }
 
+// ---- episode tickets: windows read straight from an episode store's arenas ------------------------------------------
+
+struct EpisodeTable {
+  hz_obs_episode_ticket t[kObsMaxSlots];
+};
+static_assert(sizeof(EpisodeTable) <= 4096, "the ticket table must fit the kernel parameter space");
+
+// grid and items as k_obs_pack<OutT, true>.  Root r = i * positions + p of a ticket reads its frames j = 0..stack-1 from
+// arena row min(first + p + j, last) of sample i, and its legal row, noise and mask from the sample's target count.
+template <typename OutT>
+__global__ void __launch_bounds__(kObsThreads) k_obs_pack_episodes(EpisodeTable tab, int count, int n, int num_actions,
+                                                                   ObsDims d, int positions, OutT* __restrict__ x,
+                                                                   int32_t* __restrict__ legal,
+                                                                   float* __restrict__ noise) {
+  const int k = blockIdx.y;
+  const bool real = k < count;
+  const uint8_t* frames = real ? tab.t[k].frames : nullptr;
+  const int64_t ld = real ? tab.t[k].ld_frames : 0;
+  const int32_t* samples = real ? tab.t[k].samples : nullptr;
+  const int64_t obs_items = (int64_t)n * d.chunks_per_row;
+  const int64_t row_cols = (int64_t)d.stack * d.frame_stride;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < obs_items + n; i += stride) {
+    if (i < obs_items) {
+      const int64_t r = i / d.chunks_per_row;
+      const int rem = (int)(i - r * d.chunks_per_row);
+      const int j = rem / d.chunks_per_frame;
+      const int c0 = (rem - j * d.chunks_per_frame) * kObsChunk;
+      const int valid = min(kObsChunk, d.frame_dim - c0);
+      float v[kObsChunk];
+      if (real) {
+        const int64_t s = r / positions;
+        const int p = (int)(r - s * positions);
+        const int4 smp = reinterpret_cast<const int4*>(samples)[s];
+        const int64_t row = min(smp.x + p + j, smp.y);
+        load_u8(frames + row * ld + c0, valid, v);
+      } else {
+#pragma unroll
+        for (int c = 0; c < kObsChunk; ++c) v[c] = 0.f;
+      }
+      store_chunk(x + ((int64_t)k * n + r) * row_cols + (int64_t)j * d.frame_stride + c0, v);
+    } else {
+      const int64_t r = i - obs_items;
+      int32_t* out = legal + ((int64_t)k * n + r) * num_actions;
+      float* o = noise ? noise + ((int64_t)k * n + r) * num_actions : nullptr;
+      const uint8_t* src = nullptr;
+      if (real) {
+        const int64_t s = r / positions;
+        const int p = (int)(r - s * positions);
+        const int4 smp = reinterpret_cast<const int4*>(samples)[s];
+        const bool keep = p < smp.w;
+        if (keep) src = tab.t[k].legal + (int64_t)(smp.z + p) * num_actions;
+        tab.t[k].mask[r] = keep ? 1 : 0;
+      }
+      const float* nz = real ? tab.t[k].noise : nullptr;
+      for (int a = 0; a < num_actions; ++a) {
+        const bool on = src && src[a] != 0;
+        out[a] = on ? 1 : 0;
+        if (o) o[a] = on && nz ? nz[r * num_actions + a] : 0.f;
+      }
+    }
+  }
+}
+
+static int obs_pack_episodes(const char* fn, void* stream, int device, const hz_obs_episode_ticket* tickets, int count,
+                             int slots, int n, int num_actions, const hz_obs_layout* layout, int positions, void* x,
+                             int32_t* legal, float* noise) {
+  if (!tickets) { set_error("%s: NULL ticket table", fn); return HZ_ERR_ARG; }
+  if (!layout) { set_error("%s: NULL layout", fn); return HZ_ERR_ARG; }
+  if (slots < 1 || slots > kObsMaxSlots) { set_error("%s: slots = %d, must be 1..%d", fn, slots, kObsMaxSlots); return HZ_ERR_ARG; }
+  if (count < 1 || count > slots) { set_error("%s: count = %d, must be 1..slots (%d)", fn, count, slots); return HZ_ERR_ARG; }
+  if (n < 1 || (int64_t)slots * n > kObsMaxRows) {
+    set_error("%s: n = %d, must be >= 1 with slots * n <= %lld", fn, n, (long long)kObsMaxRows);
+    return HZ_ERR_ARG;
+  }
+  if (positions < 1 || positions > n) { set_error("%s: positions = %d, must be 1..n (%d)", fn, positions, n); return HZ_ERR_ARG; }
+  if (n % positions) { set_error("%s: n = %d is not a multiple of positions = %d", fn, n, positions); return HZ_ERR_ARG; }
+  if (num_actions < 1 || num_actions > 32) { set_error("%s: num_actions = %d, must be 1..32", fn, num_actions); return HZ_ERR_ARG; }
+  const hz_obs_layout L = *layout;
+  if (L.stack < 1 || L.stack > kObsMaxStack) { set_error("%s: stack = %d, must be 1..%d", fn, L.stack, kObsMaxStack); return HZ_ERR_ARG; }
+  if (L.frame_stride < 16 || L.frame_stride % 16 || (int64_t)L.stack * L.frame_stride > kObsMaxCols) {
+    set_error("%s: frame_stride = %d, must be a multiple of 16 with stack * frame_stride <= %d", fn, L.frame_stride, kObsMaxCols);
+    return HZ_ERR_ARG;
+  }
+  if (L.frame_dim < 1 || L.frame_dim > L.frame_stride) {
+    set_error("%s: frame_dim = %d, must be 1..frame_stride (%d)", fn, L.frame_dim, L.frame_stride);
+    return HZ_ERR_ARG;
+  }
+  if (L.elem_bytes != 2 && L.elem_bytes != 4) { set_error("%s: elem_bytes = %d, must be 2 or 4", fn, L.elem_bytes); return HZ_ERR_ARG; }
+  if (!x || !legal) { set_error("%s: NULL staging buffer", fn); return HZ_ERR_ARG; }
+  for (int k = 0; k < count; ++k) {
+    const hz_obs_episode_ticket& t = tickets[k];
+    if (!t.frames || !t.legal || !t.samples) { set_error("%s: ticket %d has a NULL input", fn, k); return HZ_ERR_ARG; }
+    if (!t.mask) { set_error("%s: ticket %d has a NULL mask output", fn, k); return HZ_ERR_ARG; }
+    if (t.ld_frames < L.frame_dim) {
+      set_error("%s: ticket %d: ld_frames = %lld, must be >= frame_dim (%d)", fn, k, (long long)t.ld_frames, L.frame_dim);
+      return HZ_ERR_ARG;
+    }
+  }
+  DeviceGuard dg(device);
+  if (!dg.ok) return fail_cuda(cudaGetLastError(), fn);
+  if (int rc = check_ptr(fn, "staging x", x, device, 16)) return rc;
+  if (int rc = check_ptr(fn, "staging legal", legal, device, 4)) return rc;
+  if (int rc = check_ptr(fn, "staging noise", noise, device, 4)) return rc;
+  for (int k = 0; k < count; ++k) {
+    const hz_obs_episode_ticket& t = tickets[k];
+    if (int rc = check_ptr(fn, "ticket frames", t.frames, device, 1)) return rc;
+    if (int rc = check_ptr(fn, "ticket legal", t.legal, device, 1)) return rc;
+    if (int rc = check_ptr(fn, "ticket samples", t.samples, device, 16)) return rc;
+    if (int rc = check_ptr(fn, "ticket noise", t.noise, device, 4)) return rc;
+    if (int rc = check_ptr(fn, "ticket mask", t.mask, device, 1)) return rc;
+  }
+  EpisodeTable tab{};
+  for (int k = 0; k < count; ++k) tab.t[k] = tickets[k];
+  ObsDims d;
+  d.stack = L.stack, d.frame_dim = L.frame_dim, d.frame_stride = L.frame_stride, d.frame_words = L.frame_words;
+  d.bit_offset = L.bit_offset, d.chunks_per_frame = L.frame_stride / kObsChunk;
+  d.chunks_per_row = L.stack * d.chunks_per_frame;
+  const int64_t items = (int64_t)n * (d.chunks_per_row + 1);
+  const int64_t per_block = (int64_t)kObsThreads * kObsItemsPerThread;
+  const int blocks = (int)std::min<int64_t>((items + per_block - 1) / per_block, kObsMaxBlocksPerSlot);
+  const dim3 grid(blocks, slots);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (L.elem_bytes == 2) {
+    k_obs_pack_episodes<__half><<<grid, kObsThreads, 0, st>>>(tab, count, n, num_actions, d, positions, (__half*)x, legal, noise);
+  } else {
+    k_obs_pack_episodes<float><<<grid, kObsThreads, 0, st>>>(tab, count, n, num_actions, d, positions, (float*)x, legal, noise);
+  }
+  HZ_LAUNCH_CHECK("k_obs_pack_episodes");
+  return HZ_OK;
+}
+
 }  // namespace hz
 
 using namespace hz;
@@ -281,6 +416,13 @@ int hz_obs_pack_windows(void* stream, int device, const hz_obs_ticket* tickets, 
                         float* noise) {
   return obs_pack("hz_obs_pack_windows", true, stream, device, tickets, count, slots, n, num_actions, layout, positions,
                   x, legal, noise);
+}
+
+int hz_obs_pack_episodes(void* stream, int device, const hz_obs_episode_ticket* tickets, int count, int slots, int n,
+                         int num_actions, const hz_obs_layout* layout, int positions, void* x, int32_t* legal,
+                         float* noise) {
+  return obs_pack_episodes("hz_obs_pack_episodes", stream, device, tickets, count, slots, n, num_actions, layout,
+                           positions, x, legal, noise);
 }
 
 #pragma GCC visibility pop

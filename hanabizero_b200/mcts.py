@@ -388,7 +388,8 @@ class SearchPipeline:
     stacked observations instead of the representation network's outputs, and the slot runs the root inference itself
     (InitialPlan, one pack launch hz_obs_pack in place of hz_wave_pack).  A wave holds one kind of ticket.  Observation
     tickets may hand in frame windows of consecutive positions (`positions`) and ask for policy targets (`out_policy`):
-    the reanalyze pipeline (reanalyze.ReanalyzePipeline).
+    the reanalyze pipeline (reanalyze.ReanalyzePipeline).  A third kind, episode tickets, reads those windows from an
+    EpisodeStore in device memory (hz_obs_pack_episodes; ReanalyzePipeline.submit_episodes).
 
     Waves fill only when a caller submits tickets ahead of its waits: a wait / stats / gathered on a ticket of the open
     wave launches it with the tickets it holds so far, so submit-then-wait per ticket runs waves of one ticket.  Ticket
@@ -447,7 +448,7 @@ class SearchPipeline:
                 # the open wave: its tickets' table entries, the inputs they point at, slow-path outputs, and one
                 # caller-stream event per ticket that the slot's stream waits for at launch
                 s.update(table=[], keep=[], post=[], ev_tickets=[torch.cuda.Event() for _ in range(self.wave)],
-                         kind="hidden", obs_table=[], positions=1, policy_table=[], policy=None)
+                         kind="hidden", obs_table=[], positions=1, policy_table=[], policy=None, stores=[])
         self._next = 0
         self._waves = WaveSchedule(self.wave, self.depth)
         self._hidden_shape = None    # wave > 1: (feature, pool dtype) of the root hidden states
@@ -538,7 +539,7 @@ class SearchPipeline:
         t_host = time.perf_counter()
         noisy = noises is not None
         fraction = float(fraction) if noisy else 0.0
-        if self._waves.closes(noisy, fraction) or self._open_kind() == "obs":
+        if self._waves.closes(noisy, fraction) or self._open_kind() not in (None, "hidden"):
             self._launch_wave()
         hidden_roots = torch.as_tensor(hidden_roots)
         if self._hidden_shape is None:
@@ -562,13 +563,19 @@ class SearchPipeline:
         return self._join("hidden", noisy, fraction, rec, None, held, in_place, out_visits, out_values, t_host)
 
     def _open_kind(self):
-        """Kind of ticket ("hidden" or "obs") the open wave holds, None when no wave is open."""
+        """Kind of ticket ("hidden", "obs" or "episodes") the open wave holds, None when no wave is open."""
         return None if self._waves.open is None else self.slots[self._waves.open["slot"]]["kind"]
 
+    def _open_reads(self, store):
+        """True when the open wave holds a ticket that reads `store` (an EpisodeStore)."""
+        return self._open_kind() == "episodes" and any(
+            st is store for st, _, _ in self.slots[self._waves.open["slot"]]["stores"])
+
     def _join(self, kind, noisy, fraction, rec, obs_rec, held, in_place, out_visits, out_values, t_host, positions=1,
-              policy=None):
+              policy=None, store=None):
         """The ticket takes the next position of the open wave (opening one if needed), launching it when full.
-        policy: (policy_mask address, out_policy) of an observation ticket that asked for policy targets."""
+        policy: (policy_mask address, out_policy) of an observation ticket that asked for policy targets.
+        store: (EpisodeStore, lowest id read, the store's newest add event or None) of an episode ticket."""
         n = self.n
         if self.wave == 1:
             self._waves._next = self._next      # submit() and observation tickets share the round robin over slots
@@ -583,7 +590,9 @@ class SearchPipeline:
                 t_host += time.perf_counter() - t_wait   # waiting for the GPU is not host time
             s["busy"] = True
             s["table"], s["keep"], s["post"], s["obs_table"], s["kind"] = [], [], [], [], kind
-            s["positions"], s["policy_table"] = positions, []
+            s["positions"], s["policy_table"], s["stores"] = positions, [], []
+        if store is not None:
+            s["stores"].append(store)
         s["keep"] += held                   # alive until the slot is reused
         rows = slice(p * n, (p + 1) * n)
         for out, ok, buf in zip((out_visits, out_values), in_place, (s["visits"], s["values"])):
@@ -673,11 +682,41 @@ class SearchPipeline:
         orec.noise = self._wave_input(noises, torch.float32, (n, a), held)
         orec.obs_format, orec.legal_format = ofmt, lfmt
         policy = None if out_policy is None else (self._wave_input(policy_mask, torch.uint8, (n,), held), out_policy)
-        if (self._waves.closes(noisy, fraction) or self._open_kind() == "hidden"
+        if (self._waves.closes(noisy, fraction) or self._open_kind() not in (None, "obs")
                 or (self._open_kind() == "obs" and self.slots[self._waves.open["slot"]]["positions"] != positions)):
             self._launch_wave()
         return self._join("obs", noisy, fraction, _lib.WaveTicket(), orec, held, in_place, out_visits, out_values,
                           t_host, positions, policy)
+
+    def _submit_episodes(self, fraction, noises, store, samples, low_id, out_policy):
+        """An observation ticket of frame windows read from an EpisodeStore (reanalyze.ReanalyzePipeline
+        .submit_episodes): `samples` is hz_obs_pack_episodes' int32 [n / P, 4] on this device (P = positions), low_id
+        the lowest episode id it names, noises float32 [n, A] on this device (masked by the legal rows in the pack) or
+        None, out_policy float64 of n * A elements (its targets; rows past an episode's end zero).  The checks against
+        the store are the caller's; the pack waits for the store's adds made so far, and the store is told about the
+        pack (reader event) and about this pipeline (an evicting add launches the open wave first).  A wave holds
+        tickets of one kind and one P."""
+        if self._iplan is None:
+            raise RuntimeError("episode tickets need a pipeline built with stack= (the frame layout)")
+        t_host = time.perf_counter()
+        noisy = noises is not None
+        fraction = float(fraction) if noisy else 0.0
+        n, a, held = self.n, self.a, [samples]
+        positions = n // samples.shape[0]
+        self._wave_output(out_policy, torch.float64, (n, a))       # raises unless it can take n * A values
+        if out_policy.dtype != torch.float64:
+            raise ValueError(f"out_policy must be float64, got {out_policy.dtype}")
+        mask = torch.empty(n, dtype=torch.uint8, device=self.device)   # written by the pack, read by hz_wave_policy
+        held.append(mask)
+        rec = _lib.EpisodeTicket(frames=ptr(store.frames), ld_frames=store.frames.stride(0), legal=ptr(store.legal),
+                                 samples=ptr(samples), noise=self._wave_input(noises, torch.float32, (n, a), held),
+                                 mask=ptr(mask))
+        if (self._waves.closes(noisy, fraction) or self._open_kind() not in (None, "episodes")
+                or (self._open_kind() == "episodes" and self.slots[self._waves.open["slot"]]["positions"] != positions)):
+            self._launch_wave()
+        store._watch(self)
+        return self._join("episodes", noisy, fraction, _lib.WaveTicket(), rec, held, [False, False], None, None, t_host,
+                          positions, (ptr(mask), out_policy), store=(store, int(low_id), store._last_add))
 
     def _writable_policy(self, x):
         """True when hz_wave_policy can write `out_policy` itself (contiguous float64 here or in page-locked memory)."""
@@ -758,16 +797,27 @@ class SearchPipeline:
         lib, dev = roots._lib, roots.device_index
         for ev in s["ev_tickets"][:count]:
             compute.wait_event(ev)
+        for _, _, ev in s["stores"]:
+            if ev is not None:
+                compute.wait_event(ev)       # the episode store's adds made before the ticket was submitted
         if self.gather is not None and s["ticket"] is not None and self.gather.stream is not None:
             compute.wait_event(self.gather.slots[s["ticket"]]["done"])   # the stats buffer was its send buffer
         table = (_lib.WaveTicket * count)(*s["table"])
         st = compute.cuda_stream
         with torch.cuda.stream(compute):
-            if s["kind"] == "obs":
+            if s["kind"] != "hidden":
                 b = s["ibound"]
-                otab = (_lib.ObsTicket * count)(*s["obs_table"])
                 noise = ptr(s["noise"]) if w["noisy"] else None
-                if s["positions"] > 1:
+                otab = ((_lib.ObsTicket if s["kind"] == "obs" else _lib.EpisodeTicket) * count)(*s["obs_table"])
+                if s["kind"] == "episodes":
+                    check(lib.hz_obs_pack_episodes(st, dev, otab, count, self.wave, self.n, self.a,
+                                                   _lib.C.byref(self._layout), s["positions"], ptr(b.x),
+                                                   ptr(s["legal"]), noise))
+                    read = torch.cuda.Event()
+                    read.record(compute)         # an add that evicts what this pack read waits for it
+                    for store, low, _ in s["stores"]:
+                        store._read(read, low)
+                elif s["positions"] > 1:
                     check(lib.hz_obs_pack_windows(st, dev, otab, count, self.wave, self.n, self.a,
                                                   _lib.C.byref(self._layout), s["positions"], ptr(b.x), ptr(s["legal"]),
                                                   noise))
@@ -799,7 +849,7 @@ class SearchPipeline:
             if self.gather is not None:
                 s["ticket"] = self.gather.submit_flat(s["stats"])
             check(lib.hz_wave_unpack(st, dev, table, count, self.wave, self.n, self.a, ptr(s["stats"])))
-            if s["kind"] == "obs" and any(r is not None for r in s["policy_table"]):
+            if s["kind"] != "hidden" and any(r is not None for r in s["policy_table"]):
                 # tickets without policy targets write theirs into the slot's own rows (the kernel takes no NULL output)
                 prows = [r if r is not None else
                          _lib.PolicyTicket(mask=None, out=ptr(self._policy_rows(s)[k * self.n:(k + 1) * self.n]))

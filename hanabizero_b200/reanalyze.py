@@ -9,6 +9,8 @@ self-play (roots with all-zero legal masks included), nothing leaves the device 
 `ReanalyzePipeline` is its asynchronous form over a SearchPipeline: the caller hands in one window of stored frames
 per sampled trajectory (the learner's K + 1 consecutive positions share all but K of their frames), the windows are
 expanded into stacks on the device, searches stay in flight, and the policy targets are written by one launch per wave.
+With an EpisodeStore (trajectory.py) on the same GPU, `submit_episodes` names each sample as (episode id, start) and the
+pack reads the windows from the store's arenas: the frames never cross the host link.
 """
 import numpy as np
 import torch
@@ -113,6 +115,40 @@ class ReanalyzePipeline:
         noises = cytree.as_device(noises, torch.float32, dev, (self.roots, a)) * legal_f           # :343
         t = self.pipe.submit_observations(self.config.root_exploration_fraction, noises, obs_windows, legal,
                                           positions=per, policy_mask=mask.reshape(self.roots), out_policy=out)
+        self._out[t] = out
+        return t
+
+    def submit_episodes(self, store, ids, starts, noises=None, noise_seed=0, noise_step=0, out=None):
+        """submit() with the windows read from an EpisodeStore on this device: sample b searches positions
+        starts[b] .. starts[b] + K of episode ids[b] (int [batch] each).  Frames are the episode's rows from frame
+        starts[b] on, the last frame repeated past its end; positions past the end (start + p >= T) get all-zero legal
+        rows and a zero target row.  Only the sample rows (16 bytes a sample) cross from the host.  Targets equal
+        submit() of the same windows, legal rows and masks cut from the flushed episodes.  Raises before taking a ticket
+        on an evicted or unknown id, a start outside 0..T - 1, or a store whose device, obs_dim, num_actions or stack
+        is not the pipeline's.  Noise, `out` and the result as submit()."""
+        B, per, a, dev = self.batch, self.per, self.a, self.device
+        if (store.device, store.obs_dim, store.num_actions, store.stack) != (dev, self.pipe.frame_dim, a, self.stack):
+            raise ValueError(f"store ({store.device}, obs_dim {store.obs_dim}, num_actions {store.num_actions}, stack "
+                             f"{store.stack}) does not fit the pipeline ({dev}, obs_dim {self.pipe.frame_dim}, "
+                             f"num_actions {a}, stack {self.stack})")
+        ids = np.asarray(ids, np.int64).reshape(-1)
+        starts = np.asarray(starts, np.int64).reshape(-1)
+        if ids.size != B or starts.size != B:
+            raise ValueError(f"ids and starts must hold {B} values each, got {ids.size} and {starts.size}")
+        samples = store.samples(ids, starts, per)        # raises on evicted ids and bad starts
+        if noises is not None and _as_tensor(noises).numel() != self.roots * a:
+            raise ValueError(f"noises must hold [{self.roots}, {a}] values, got {tuple(_as_tensor(noises).shape)}")
+        if out is None:
+            out = torch.empty(B, per, a, dtype=torch.float64, device=dev)
+        self.pipe._wave_output(out, torch.float64, (self.roots, a))      # raises before anything is enqueued
+        if out.dtype != torch.float64:
+            raise ValueError(f"out must be float64, got {out.dtype}")
+        if noises is None:
+            noises = dirichlet_noise(self.roots, a, getattr(self.config, "root_dirichlet_alpha", 0.3), dev, noise_seed,
+                                     noise_step)
+        noises = cytree.as_device(noises, torch.float32, dev, (self.roots, a))     # legal-masked in the pack (:343)
+        samples = torch.from_numpy(samples).pin_memory().to(dev, non_blocking=True)
+        t = self.pipe._submit_episodes(self.config.root_exploration_fraction, noises, store, samples, int(ids.min()), out)
         self._out[t] = out
         return t
 

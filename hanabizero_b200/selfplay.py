@@ -305,13 +305,15 @@ class SelfPlayPool:
         for s in self.streams:
             s.synchronize()
 
-    def flush(self):
+    def flush(self, store=None):
         """The finished episodes of every recording engine: one list per engine (TrajectoryRecorder.flush; [] for an
-        engine that does not record).  Each engine's flush runs on that engine's stream, after its appends."""
+        engine that does not record).  Each engine's flush runs on that engine's stream, after its appends.  With
+        `store` (trajectory.EpisodeStore) the frames and legal rows go into the store on those streams and the dicts
+        carry store ids instead of frames (TrajectoryRecorder.flush(store=...))."""
         out = []
         for eng, s in zip(self.engines, self.streams):
             with torch.cuda.stream(s):
-                out.append([] if eng.recorder is None else eng.recorder.flush())
+                out.append([] if eng.recorder is None else eng.recorder.flush(store=store))
         return out
 
     def check(self):

@@ -554,6 +554,28 @@ int hz_obs_pack(void* stream, int device, const hz_obs_ticket* tickets, int coun
 int hz_obs_pack_windows(void* stream, int device, const hz_obs_ticket* tickets, int count, int slots, int n,
                         int num_actions, const hz_obs_layout* layout, int positions, void* x, int32_t* legal,
                         float* noise);
+/* hz_obs_pack_windows with the windows read from an episode store (hanabizero_b200/trajectory.py EpisodeStore): byte
+ * frame rows of D = frame_dim values in `frames` (row stride ld_frames bytes) and legal rows of num_actions 0/1 bytes in
+ * `legal`, as hz_traj_pack writes them.  Sample i of a ticket (roots i * positions .. i * positions + positions - 1) is
+ * four int32 in samples[i]: {first frame row of its window, last frame row of its episode, legal row of its first
+ * position, number of positions with targets c (0..positions)}.  Root r = i * positions + p takes frame rows
+ * min(first + p + j, last) for j = 0..stack-1, legal row first_legal + p and its noise where p < c (noise entries whose
+ * legal byte is 0 become 0), an all-zero legal row and noise where p >= c, and mask[r] = p < c — the mask that
+ * hz_wave_policy takes for the ticket's targets.  frames, legal, samples (16-byte aligned), noise and mask: device
+ * memory of `device` or page-locked host memory, read and written by the kernel itself; only mask may not be NULL among
+ * the outputs, noise may (zeros).  The rows the samples name are not checked: they must lie in the arenas.  Everything
+ * else as hz_obs_pack_windows, checked before the launch; one launch, the table (48 bytes a ticket) travels by value. */
+typedef struct hz_obs_episode_ticket {
+  const uint8_t* frames;   /* frame arena */
+  int64_t ld_frames;       /* bytes per frame row (>= frame_dim) */
+  const uint8_t* legal;    /* legal arena [rows][num_actions] */
+  const int32_t* samples;  /* [n / positions][4] */
+  const float* noise;      /* [n][A] contiguous, or NULL (= zeros) */
+  uint8_t* mask;           /* [n] out */
+} hz_obs_episode_ticket;
+int hz_obs_pack_episodes(void* stream, int device, const hz_obs_episode_ticket* tickets, int count, int slots, int n,
+                         int num_actions, const hz_obs_layout* layout, int positions, void* x, int32_t* legal,
+                         float* noise);
 
 #ifdef __cplusplus
 }
