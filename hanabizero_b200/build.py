@@ -11,7 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(CSRC, "libhzb200.so")
 SOURCES = ["hz_tree.cu", "hz_env.cu", "hz_nn.cu", "hz_gemm.cu", "hz_rowchain.cu", "hz_selfplay.cu", "hz_traj.cu", "hz_noise.cu", "hz_wave.cu", "hz_obs.cu", "hz_host.cpp"]
-HEADERS = ["hz_common.cuh", "hz_math.cuh", "hz_decode.cuh", "../../include/hzb200.h"]
+HEADERS = ["hz_common.cuh", "hz_math.cuh", "hz_decode.cuh", "hz_detmath.cuh", "../../include/hzb200.h"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -8,9 +8,11 @@
 //   glibc >= 2.27 sysdeps/ieee754/flt-32/e_expf.c + e_exp2f_data.c (N = 32 entry 2^(i/N) table,
 //   cubic polynomial), in the evaluation order of the x86-64 ifunc variant selected on any CPU
 //   with FMA3 (__expf_fma: the range reduction r = InvLn2N*x - kd is one fused multiply-subtract).
-// Verified on the host (oracle/expf_sweep.c) against libm for all 2^32 inputs; on the device the
-// same sequence of IEEE fp64 operations gives the same bits (tests/test_tree_gpu.py checks the
-// kernels' priors bit for bit against the reference).
+// The host restatement (oracle/expf_glibc.h) is verified against libm for all 2^32 inputs
+// (oracle/expf_sweep.c).  Both device copies below are run on the device for all 2^32 inputs and
+// compared with that restatement bit for bit (tests/test_device_math_gpu.py; the warp form with 32
+// consecutive patterns per warp and with 32 patterns 2^27 apart); tests/test_tree_gpu.py checks the
+// kernels' priors bit for bit against the reference.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>

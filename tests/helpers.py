@@ -1,6 +1,9 @@
 """Shared test helpers (test infrastructure)."""
+import ctypes
 import glob
+import math
 import os
+import subprocess
 
 import numpy as np
 
@@ -299,6 +302,92 @@ def unpack_traj_golden(g):
                         r=g["out_r"][s:s + n], o=out_o[so:so + stack + n], la=g["out_la"][sl:sl + n + 1]))
         s, so, sl = s + n, so + stack + n, sl + n + 1
     return obs, eps
+
+
+def build_detmath_harness(out_dir):
+    """tests/detmath_harness.cu -> out_dir/libdetmath_harness.so, compiled with the library's own nvcc flags
+    (hanabizero_b200.build.NVCC_FLAGS) against its headers; loaded with ctypes, argument types set."""
+    from hanabizero_b200.build import CSRC, NVCC_FLAGS
+    so = os.path.join(str(out_dir), "libdetmath_harness.so")
+    nvcc = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
+    cmd = [nvcc] + NVCC_FLAGS + ["-I", CSRC, "-o", so, os.path.join(ROOT, "tests", "detmath_harness.cu")]
+    r = subprocess.run(cmd, capture_output=True, text=True)
+    assert r.returncode == 0, " ".join(cmd) + "\n" + r.stdout + r.stderr
+    lib = ctypes.CDLL(so)
+    p, i64 = ctypes.c_void_p, ctypes.c_int64
+    lib.hzt_expf.argtypes = [p, p, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_int, ctypes.c_int]
+    for name in ("hzt_det_log", "hzt_det_exp"):
+        getattr(lib, name).argtypes = [p, p, p, i64]
+        getattr(lib, "hzt_host_" + name[4:]).argtypes = [p, p, i64]
+        getattr(lib, "hzt_host_" + name[4:]).restype = None
+    return lib
+
+
+def double_neighbours(x, n):
+    """Each finite nonzero double of x with the n adjacent doubles on either side (same sign, so adjacent bit
+    patterns), flattened."""
+    b = np.asarray(x, np.float64).reshape(-1).view(np.int64)[:, None] + np.arange(-n, n + 1)
+    return b.reshape(-1).view(np.float64)
+
+
+SQRT2 = 1.4142135623730951
+_MANT = (1 << 52) - 1
+
+
+def det_log_points(per_binade, exps=range(-1022, 1024), block=128, seed=0):
+    """Normal doubles for det_log (hz_detmath.cuh), yielded per block of binades 2^e, e in exps: per_binade random
+    mantissas, the mantissas 1, 1 + ulp and 2 - ulp, and +-8 ulps around the sqrt(2) split, where det_log halves the
+    mantissa and adds one to the exponent."""
+    rng = np.random.default_rng(seed)
+    exps = np.asarray(list(exps), np.int64)
+    m_sqrt2 = int(np.float64(SQRT2).view(np.int64)) & _MANT
+    fixed = np.concatenate([[0, 1, _MANT], m_sqrt2 + np.arange(-8, 9)]).astype(np.uint64)
+    for i in range(0, exps.size, block):
+        e = exps[i:i + block]
+        top = (e + 1023).astype(np.uint64)[:, None] << np.uint64(52)
+        mant = np.concatenate([rng.integers(0, 1 << 52, (e.size, per_binade), dtype=np.uint64),
+                               np.broadcast_to(fixed, (e.size, fixed.size))], 1)
+        yield (top | mant).reshape(-1).view(np.float64)
+
+
+def det_exp_edges(ks=range(-1010, 1)):
+    """Edges of det_exp (hz_detmath.cuh), x <= 0 save the positive neighbours of +0: +-8 ulps around -700 (below it
+    returns 0) and -580 (the noise's rescale threshold), +0 and -0 with their 8 nearest subnormals, and +-4 ulps
+    around (k - 1/2) ln 2 for each k in ks, where floor(x log2(e) + 1/2) steps from k - 1 to k."""
+    tiny = np.arange(0, 9, dtype=np.uint64)
+    zeros = np.concatenate([tiny, tiny | np.uint64(1 << 63)]).view(np.float64)
+    bounds = (np.asarray(list(ks), np.float64) - 0.5) * math.log(2.0)
+    return np.concatenate([double_neighbours([-700.0, -580.0], 8), zeros, double_neighbours(bounds, 4)])
+
+
+def det_exp_uniform(n, block=1 << 23, seed=0):
+    """n uniform points on [-745, 0] (x < -700 gives 0), yielded in blocks."""
+    rng = np.random.default_rng(seed)
+    for i in range(0, n, block):
+        yield -745.0 * rng.random(min(block, n - i))
+
+
+def build_expf_check(out_dir):
+    """tests/expf_check.c -> out_dir/libexpf_check.so, built the way test_oracle_expf.py builds expf_sweep.c."""
+    so = os.path.join(str(out_dir), "libexpf_check.so")
+    subprocess.run(["gcc", "-O2", "-ffp-contract=off", "-fopenmp", "-shared", "-fPIC", "-I", os.path.join(ROOT, "oracle"),
+                    os.path.join(ROOT, "tests", "expf_check.c"), "-lm", "-o", so], check=True)
+    lib = ctypes.CDLL(so)
+    lib.hz_expf_check.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_int,
+                                  ctypes.c_void_p, ctypes.c_void_p, ctypes.c_int]
+    return lib
+
+
+def expf_check(lib, outs, start, rotate, nfirst=16):
+    """Device outputs `outs` (uint32 arrays of one length, bits at pattern(start + i, rotate)) against the glibc
+    restatement: [(mismatch count, first mismatching patterns)] per output."""
+    outs = [np.ascontiguousarray(o, np.uint32) for o in outs]
+    n = outs[0].size
+    ptrs = (ctypes.c_void_p * len(outs))(*[o.ctypes.data for o in outs])
+    bad = np.zeros(len(outs), np.uint64)
+    first = np.zeros((len(outs), nfirst), np.uint32)
+    assert lib.hz_expf_check(ptrs, len(outs), start, n, rotate, bad.ctypes.data, first.ctypes.data, nfirst) == 0
+    return [(int(b), first[k, :min(int(b), nfirst)].tolist()) for k, b in enumerate(bad)]
 
 
 def rounded_beta_ks(x, a, b):
